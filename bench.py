@@ -48,7 +48,25 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--pageable", action="store_true", help="e2e leg with pageable (malloc) host buffers instead of pinned ones")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (gram: gram, rhs, tau_sq; "
+                         "materialise: a fixed, seeded sample of the columns of regressor and torque of the last launch)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours: the CPU timing loop does not store its outputs")
+    return args
+
+
+DUMP_COLUMNS = 8192   # materialise: sampled columns of Phi / tau written by --dump-outputs (426 rows x 8 B x 8192 = 28 MB for C6)
+
+
+def dump_outputs(path: str, arrays: dict):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), t.detach().cpu().numpy().astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -368,6 +386,14 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t[0])
     value = world * S * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        if gram:
+            dump_outputs(args.dump_outputs, {"gram": G, "rhs": b, "tau_sq": tt})
+        else:   # Phi / tau hold the last launch of the last step; the sampled columns depend only on the launch size
+            import numpy as np
+            cols = np.sort(np.random.default_rng(0).choice(Sl, size=min(Sl, DUMP_COLUMNS), replace=False))
+            cols = torch.from_numpy(cols).to(dev)
+            dump_outputs(args.dump_outputs, {"regressor": phi.index_select(1, cols), "torque": tau.index_select(1, cols)})
 
     # ------------------------------------------------------------------ e2e through the host-buffer C-ABI entry
     e2e = None

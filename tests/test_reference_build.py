@@ -2,8 +2,8 @@
 
 * tests/golden/ref_<chain>.npz were produced by the reference's own rosdyn::Chain (its headers compiled where they lie under
   /root/reference against the stand-in third-party headers of oracle/shim/; generator tests/golden/make_golden_ref.py).
-* when oracle/_ref/librosdyn_ref.so is present (built here by __graft_entry__.build(); it travels to the GPU box) the oracle is also
-  compared live on seeded batches, including permuted / partial input-joint lists and multi-threaded clones (Chain::clone)."""
+* when oracle/_ref/librosdyn_ref.so is present (built by __graft_entry__.build() when the reference sources are available) the oracle is
+  also compared live on seeded batches, including permuted / partial input-joint lists and multi-threaded clones (Chain::clone)."""
 import numpy as np
 import pytest
 
@@ -31,8 +31,18 @@ def test_oracle_matches_reference_outputs(name, fast, golden):
     assert_close(oc.kinematics(g["q"], g["dq"], None, want=("torque",))["torque"], g["torque_nonlin"], f"{name}:torque_nonlin", tol)
     assert_close(oc.inertia(g["q"]), g["inertia"], f"{name}:inertia", tol)
     assert_close(oc.nominal_parameters(), g["nominal"], f"{name}:nominal", tol)
-    # structural zeros (row of chain joint j, column blocks of the links before it) are exact zeros on both sides
+    pt, tt = oc.regressor_torque(g["q"], g["dq"], g["ddq"], nthreads=2)
+    assert_close(pt, g["regressor"], f"{name}:regressor, 2 threads", tol)
+    assert_close(tt, g["torque"], f"{name}:torque, 2 threads", tol)
+    # normal equations: the sums oracle/_ref's oracle_regressor_gram forms from the reference's getRegressor / getJointTorque
     d = fixtures.by_name(name)
+    Y = g["regressor"].reshape(10 * d.n_joints, d.n_inputs, -1)              # [col][row][sample]
+    Gr, br, tr = np.einsum("crs,drs->cd", Y, Y), np.einsum("crs,rs->c", Y, g["torque"]), float(np.sum(g["torque"] ** 2))
+    G, b, t2 = oc.gram(g["q"], g["dq"], g["ddq"])
+    assert_close(G / np.max(np.abs(Gr)), Gr / np.max(np.abs(Gr)), f"{name}:gram", tol)
+    assert_close(b / np.max(np.abs(br)), br / np.max(np.abs(br)), f"{name}:rhs", tol)
+    assert abs(t2 - tr) <= tol * tr
+    # structural zeros (row of chain joint j, column blocks of the links before it) are exact zeros on both sides
     for j, jd in enumerate(d.joints):
         if jd.input_index >= 0:
             rows = [c * d.n_inputs + jd.input_index for c in range(10 * j)]
@@ -86,8 +96,12 @@ def test_reference_input_joint_selection():
     assert_close(o2.kinematics(q, dq, ddq, want=("torque",))["torque"], r2.kinematics(q, dq, ddq, want=("torque",))["torque"], "torque", TOL)
 
 
-@needs_ref
-def test_reference_ur10_known_answer():
-    rc = OracleChain(fixtures.by_name("c6"), fast="ref")
-    T = rc.kinematics(np.zeros((6, 1)), want=("T_tool",))["T_tool"][:, 0].reshape(3, 4)
+def test_reference_ur10_known_answer(golden):
+    """The reference's tool pose of C6 at the zero pose (sample 0 of tests/golden/ref_c6.npz has q = 0; the tool is the last link), and the
+    restatement's at the same pose."""
+    g = golden("ref_c6")
+    assert np.all(g["q"][:, 0] == 0.0)
+    T = g["T_links"][-12:, 0].reshape(3, 4)
+    np.testing.assert_allclose(T[:, 3], [1.1843, 0.256141, 0.0116], atol=1e-12)
+    T = OracleChain(fixtures.by_name("c6")).kinematics(np.zeros((6, 1)), want=("T_tool",))["T_tool"][:, 0].reshape(3, 4)
     np.testing.assert_allclose(T[:, 3], [1.1843, 0.256141, 0.0116], atol=1e-12)
