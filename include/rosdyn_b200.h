@@ -205,6 +205,20 @@ rdb_status rdb_inertia_batch(const rdb_chain* chain, const rdb_samples* in, doub
  * SoA special cases).  Regressor and torque come from one pass over the chain, the inertia from a second launch. */
 rdb_status rdb_dynamics_batch(const rdb_chain* chain, const rdb_samples* in, const rdb_dynamics_out* out, void* stream);
 
+/* Forward dynamics (no reference function; the reference's callers compose getJointInertia PI.h:1357-1379 and
+ * getJointTorqueNonLinearPart PI.h:1285-1293):  ddq = M(q)^-1 (tau - h(q, Dq)),  h = getJointTorque(q, Dq, 0) incl. gravity.
+ * in->q, in->dq (NULL = 0) as everywhere; in->ddq / in->dddq are ignored.  tau[n_inputs][in->ld] (NULL = zero torque, the same
+ * plane stride as q, like tau_meas of rdb_regressor_gram_batch).  ddq[n_inputs][ld_out].  info[n] optional: 0, or 1 when M(q) is not
+ * positive definite (a Cholesky pivot <= 0 or not finite); that sample's ddq is NaN in every component.
+ * Inputs that no chain joint feeds get ddq = 0 and are left out of the solve (their row / column of M is zero).
+ * One pass over the chain per sample: M and h are accumulated in registers, M is factored there (Cholesky) and only ddq leaves the
+ * thread.  Results are per sample: bit-identical across launches and between this entry and its host twin.
+ * Additive joint components (friction, springs) compose by subtraction: copy tau, then
+ * rdb_components_torque_batch(chain, in, -pi_c, tau_copy, ld, accumulate = 1, stream) adds -Phi_c pi_c, and forward dynamics of tau_copy
+ * gives M^-1 (tau - h - Phi_c pi_c). */
+rdb_status rdb_forward_dynamics_batch(const rdb_chain* chain, const rdb_samples* in, const double* tau, double* ddq, int64_t ld_out,
+                                      int32_t* info, void* stream);
+
 /* Fused regressor -> normal equations (no reference code: the consumer rosdyn_identification is external,
  * reference README.md:15).  With P = 10*n_joints and Phi_s the n_inputs x P regressor of sample s:
  *   gram[P*P]  (+)= sum_s Phi_s^T Phi_s   (column-major, full symmetric matrix)
@@ -358,6 +372,8 @@ rdb_status rdb_torque_batch_host(rdb_chain* chain, const rdb_samples* in, double
 rdb_status rdb_regressor_batch_host(rdb_chain* chain, const rdb_samples* in, double* phi, double* torque, int64_t ld_out);
 rdb_status rdb_inertia_batch_host(rdb_chain* chain, const rdb_samples* in, double* inertia, int64_t ld_out);
 rdb_status rdb_dynamics_batch_host(rdb_chain* chain, const rdb_samples* in, const rdb_dynamics_out* out);
+rdb_status rdb_forward_dynamics_batch_host(rdb_chain* chain, const rdb_samples* in, const double* tau, double* ddq, int64_t ld_out,
+                                           int32_t* info);
 rdb_status rdb_regressor_gram_batch_host(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, double* gram, double* rhs,
                                          double* tau_sq, int32_t accumulate);
 

@@ -164,6 +164,15 @@ public:
     check(rdb_torque_batch_host(m_h, &in, tau.data(), 1));
     return tau;
   }
+  // forward dynamics ddq = M(q)^-1 (tau - h(q, Dq)) (rdb_forward_dynamics_batch); all NaN when M(q) is not positive definite
+  VectorXd getJointAcceleration(const VectorXd& q, const VectorXd& Dq, const VectorXd& tau)
+  {
+    sizes(q, &Dq, &tau, nullptr);
+    VectorXd ddq(m_n);
+    rdb_samples in{1, 1, q.data(), Dq.data(), nullptr, nullptr};
+    check(rdb_forward_dynamics_batch_host(m_h, &in, tau.data(), ddq.data(), 1, nullptr));
+    return ddq;
+  }
   // n_act x 10 nJ, column-major (the memory image of the Eigen::MatrixXd the reference returns by value)
   VectorXd getRegressor(const VectorXd& q, const VectorXd& Dq, const VectorXd& DDq)
   {
@@ -192,6 +201,11 @@ public:
     check(rdb_regressor_batch(m_h, &in, phi, torque, ld_out, stream));
   }
   void getJointInertia(const rdb_samples& in, double* inertia, int64_t ld_out, void* stream = nullptr) { check(rdb_inertia_batch(m_h, &in, inertia, ld_out, stream)); }
+  // tau [n_act][in.ld] (nullptr = 0), ddq [n_act][ld_out], info [n] optional (1 = M not positive definite)
+  void getJointAcceleration(const rdb_samples& in, const double* tau, double* ddq, int64_t ld_out, int32_t* info = nullptr, void* stream = nullptr)
+  {
+    check(rdb_forward_dynamics_batch(m_h, &in, tau, ddq, ld_out, info, stream));
+  }
   void getRegressorGram(const rdb_samples& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, bool accumulate, void* stream = nullptr)
   {
     check(rdb_regressor_gram_batch(m_h, &in, tau_meas, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
@@ -277,6 +291,10 @@ public:
   void getJointTorqueHost(const rdb_samples& in, double* torque, int64_t ld_out) { check(rdb_torque_batch_host(m_h, &in, torque, ld_out)); }
   void getRegressorHost(const rdb_samples& in, double* phi, double* torque, int64_t ld_out) { check(rdb_regressor_batch_host(m_h, &in, phi, torque, ld_out)); }
   void getJointInertiaHost(const rdb_samples& in, double* inertia, int64_t ld_out) { check(rdb_inertia_batch_host(m_h, &in, inertia, ld_out)); }
+  void getJointAccelerationHost(const rdb_samples& in, const double* tau, double* ddq, int64_t ld_out, int32_t* info = nullptr)
+  {
+    check(rdb_forward_dynamics_batch_host(m_h, &in, tau, ddq, ld_out, info));
+  }
   void getRegressorGramHost(const rdb_samples& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, bool accumulate)
   {
     check(rdb_regressor_gram_batch_host(m_h, &in, tau_meas, gram, rhs, tau_sq, accumulate ? 1 : 0));
@@ -339,6 +357,10 @@ public:
     return eMat(getRegressor(stdv(q), stdv(Dq), stdv(DDq)), (int)m_n, (int)(10 * m_nj));
   }
   Eigen::MatrixXd getJointInertia(const Eigen::VectorXd& q) { return eMat(getJointInertia(stdv(q)), (int)m_n, (int)m_n); }
+  Eigen::VectorXd getJointAcceleration(const Eigen::VectorXd& q, const Eigen::VectorXd& Dq, const Eigen::VectorXd& tau)
+  {
+    return eVec(getJointAcceleration(stdv(q), stdv(Dq), stdv(tau)));
+  }
   Eigen::VectorXd getNominalParametersEigen() const { return eVec(getNominalParameters()); }
 
   // Batched siblings for Eigen callers: N samples as the COLUMNS of n_act x N matrices (column-major, i.e. one sample = n_act contiguous

@@ -452,6 +452,28 @@ class Chain:
         r = _swap01(M.reshape(self.n_in, self.n_in, n))
         return r[..., 0] if single else r
 
+    def getJointAcceleration(self, q, Dq, tau, with_info: bool = False):
+        """Forward dynamics ddq = M(q)^-1 (tau - h(q, Dq)) with h = getJointTorque(q, Dq, 0) (rdb_forward_dynamics_batch): n_act (x N).
+        Dq / tau may be None (zero).  with_info also returns info, int32 (N,) (or an int for 1-D inputs): 1 where M(q) is not positive
+        definite (that sample's ddq is all NaN), else 0.  Torch CUDA arrays run on the device, host arrays through the host twin."""
+        dev, single, n, arrs = self._prep([q, Dq, None, None])
+        tau_arr = None
+        if tau is not None:
+            arrs, tau_arr = self._with_tau(dev, n, arrs, tau)
+        ddq = self._alloc(dev, self.n_in, n, arrs[0])
+        info = None
+        if with_info:
+            info = torch.empty((max(n, 1),), dtype=torch.int32, device=arrs[0].device)[:n] if dev else np.empty((n,), dtype=np.int32)
+        s = self._samples(n, arrs)
+        if dev:
+            check(self._lib.rdb_forward_dynamics_batch(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(ddq), max(n, 1), _ptr(info), self._stream()))
+        else:
+            check(self._lib.rdb_forward_dynamics_batch_host(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(ddq), max(n, 1), _ptr(info)))
+        if single:
+            ddq = ddq[:, 0]
+            info = int(info[0]) if info is not None else None
+        return (ddq, info) if with_info else ddq
+
     def regressorGram(self, q, Dq, DDq, tau_meas=None, out=None):
         """Fused getRegressor -> normal equations: returns (G[P,P], b[P], tau_sq[1]) with
         G = sum Phi^T Phi, b = sum Phi^T tau, tau_sq = sum tau^T tau; tau = tau_meas or getJointTorque.

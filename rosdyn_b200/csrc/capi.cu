@@ -378,6 +378,25 @@ rdb_status rdb_inertia_batch(const rdb_chain* chain, const rdb_samples* in, doub
   return RDB_OK;
 }
 
+rdb_status rdb_forward_dynamics_batch(const rdb_chain* chain, const rdb_samples* in, const double* tau, double* ddq, int64_t ld_out,
+                                      int32_t* info, void* stream)
+{
+  rdb_status s = check_samples(chain, in, true);
+  if (s != RDB_OK) return s;
+  RDB_ENTER(chain);
+  if (in->n == 0) return RDB_OK;
+  if (!ddq || ld_out < in->n) return fail(RDB_ERR_INVALID_ARG, "ddq: null or ld_out < n");
+  cudaStream_t st = (cudaStream_t)stream;
+  if ((s = prezero(chain, ddq, chain->host.n_in, ld_out, in->n, st)) != RDB_OK) return s;
+  SamplesDev sd = to_dev(in);
+  sd.ddq = sd.dddq = nullptr;  // the walk runs with DDq = 0
+  DynOutDev o = dyn_out_soa(nullptr, ddq, nullptr, ld_out);
+  o.tau_in = tau;
+  o.info = info;
+  RDB_CUDA(launch_dyn(*chain, DYN_FD_, sd, o, st));
+  return RDB_OK;
+}
+
 rdb_status rdb_dynamics_batch(const rdb_chain* chain, const rdb_samples* in, const rdb_dynamics_out* out, void* stream)
 {
   rdb_status s = check_samples(chain, in, true);
@@ -633,9 +652,11 @@ struct Plane
   int64_t planes = 0;
   int64_t ld = 0;  // host plane stride
   bool records = false;  // RDB_LAYOUT_EIGEN output: [sample][planes] dense records on both sides (one contiguous copy per chunk)
+  int64_t es = sizeof(double);  // bytes per element of an output plane (int32 status planes: 4; the device side keeps a double-sized slot)
   double* d[2] = {nullptr, nullptr};
   double* hm = nullptr;  // mapped mode: host alias of d[0]
   double* hp[2] = {nullptr, nullptr};  // bounce mode: pinned mirror of d[slot]
+  void* out_at(int64_t r, int64_t off) const { return reinterpret_cast<char*>(h_out) + (r * ld + off) * es; }  // caller's element (plane r, sample off)
 };
 
 // host threads of the gather / scatter loops: the hardware threads shared out over the visible GPUs (one rank or one handle per GPU is the
@@ -817,7 +838,7 @@ struct HostPipe
         });
       }
       else
-        host_parallel(p.planes, [&](int64_t r) { memcpy(p.h_out + r * p.ld + q.off, src + r * chunk, sizeof(double) * (size_t)q.len); });
+        host_parallel(p.planes, [&](int64_t r) { memcpy(p.out_at(r, q.off), src + r * chunk, p.es * (size_t)q.len); });
     }
     waiting[slot].clear();
   }
@@ -855,7 +876,7 @@ struct HostPipe
       if (p.records)
         RDB_CUDA(cudaMemcpyAsync(p.hp[slot], p.d[slot], sizeof(double) * (size_t)len * p.planes, cudaMemcpyDeviceToHost, st[slot]));
       else
-        RDB_CUDA(cudaMemcpy2DAsync(p.hp[slot], chunk * sizeof(double), p.d[slot], chunk * sizeof(double), len * sizeof(double), p.planes,
+        RDB_CUDA(cudaMemcpy2DAsync(p.hp[slot], chunk * sizeof(double), p.d[slot], chunk * sizeof(double), len * p.es, p.planes,
                                    cudaMemcpyDeviceToHost, st[slot]));
       waiting[slot].push_back({&p, off, len});
       return RDB_OK;
@@ -863,7 +884,7 @@ struct HostPipe
     if (p.records)
       RDB_CUDA(cudaMemcpyAsync(p.h_out + off * p.planes, p.d[slot], sizeof(double) * (size_t)len * p.planes, cudaMemcpyDeviceToHost, st[slot]));
     else
-      RDB_CUDA(cudaMemcpy2DAsync(p.h_out + off, p.ld * sizeof(double), p.d[slot], chunk * sizeof(double), len * sizeof(double), p.planes,
+      RDB_CUDA(cudaMemcpy2DAsync(p.out_at(0, off), p.ld * p.es, p.d[slot], chunk * sizeof(double), len * p.es, p.planes,
                                  cudaMemcpyDeviceToHost, st[slot]));
     return RDB_OK;
   }
@@ -878,7 +899,7 @@ struct HostPipe
       const Plane& p = *q.p;
       if (p.records) memcpy(p.h_out + q.off * p.planes, p.hm, sizeof(double) * (size_t)q.len * p.planes);
       else
-        for (int64_t r = 0; r < p.planes; r++) memcpy(p.h_out + r * p.ld + q.off, p.hm + r * chunk, sizeof(double) * (size_t)q.len);
+        for (int64_t r = 0; r < p.planes; r++) memcpy(p.out_at(r, q.off), p.hm + r * chunk, p.es * (size_t)q.len);
     }
     pending.clear();
     return RDB_OK;
@@ -1018,6 +1039,44 @@ rdb_status rdb_inertia_batch_host(rdb_chain* chain, const rdb_samples* in, doubl
 {
   if (!inertia) return fail(RDB_ERR_INVALID_ARG, "inertia is null");
   return dyn_host(chain, in, nullptr, nullptr, inertia, ld_out, 2);
+}
+
+rdb_status rdb_forward_dynamics_batch_host(rdb_chain* chain, const rdb_samples* in, const double* tau, double* ddq, int64_t ld_out,
+                                           int32_t* info)
+{
+  RDB_TRY(check_samples(chain, in, true));
+  RDB_ENTER(chain);
+  RDB_LOCK(chain);
+  if (in->n == 0) return RDB_OK;
+  if (!ddq || ld_out < in->n) return fail(RDB_ERR_INVALID_ARG, "ddq: null or ld_out < n");
+  const int n_in = chain->host.n_in;
+  HostIn hi;
+  hi.bind(in, n_in);
+  // forward dynamics ignores DDq / DDDq: tau travels in the DDq slot
+  hi.ddq.h_in = tau;
+  hi.ddq.planes = tau ? n_in : 0;
+  hi.dddq.h_in = nullptr;
+  hi.dddq.planes = 0;
+  Plane pdd, pinfo;
+  pdd.h_out = ddq; pdd.planes = n_in; pdd.ld = ld_out;
+  pinfo.h_out = reinterpret_cast<double*>(info); pinfo.planes = info ? 1 : 0; pinfo.ld = in->n; pinfo.es = sizeof(int32_t);
+  HostPipe pipe;
+  RDB_TRY(pipe.init(chain->host_arena, in->n, 1 << 21, {&hi.q, &hi.dq, &hi.ddq, &pdd, &pinfo}));
+  int slot = 0;
+  for (int64_t off = 0; off < in->n; off += pipe.chunk, slot ^= 1)
+  {
+    const int64_t len = std::min<int64_t>(pipe.chunk, in->n - off);
+    RDB_TRY(pipe.begin(slot));
+    RDB_TRY(pipe.h2d(hi.q, slot, off, len));
+    RDB_TRY(pipe.h2d(hi.dq, slot, off, len));
+    RDB_TRY(pipe.h2d(hi.ddq, slot, off, len));
+    const rdb_samples v{len, pipe.chunk, hi.q.d[slot], hi.dq.d[slot], nullptr, nullptr};
+    RDB_TRY(rdb_forward_dynamics_batch(chain, &v, hi.ddq.d[slot], pdd.d[slot], pipe.chunk, info ? reinterpret_cast<int32_t*>(pinfo.d[slot]) : nullptr,
+                                       pipe.st[slot]));
+    RDB_TRY(pipe.d2h(pdd, slot, off, len));
+    RDB_TRY(pipe.d2h(pinfo, slot, off, len));
+  }
+  return pipe.finish();
 }
 
 rdb_status rdb_dynamics_batch_host(rdb_chain* chain, const rdb_samples* in, const rdb_dynamics_out* out)

@@ -75,10 +75,14 @@ struct KinOutDev
 
 // outputs of the link-frame walker.  Element (plane p, sample i) of an array lives at  base + p * ps + i * ss_<array>:
 // SoA planes: ps = ld, ss = 1;  Eigen records: ps = 1, ss = planes of the array (the record is the column-major Eigen matrix)
+// Forward dynamics (DYN_FD) writes ddq into `tau`, reads the applied torques from tau_in [n_in][in.ld] (NULL = 0) and, when info is not
+// NULL, writes info[i] (0, or 1 when M is not positive definite)
 struct DynOutDev
 {
   double *phi, *tau, *M;
   int64_t ps, ss_phi, ss_tau, ss_M;
+  const double* tau_in = nullptr;
+  int32_t* info = nullptr;
 };
 inline DynOutDev dyn_out_soa(double* phi, double* tau, double* M, int64_t ld) { return DynOutDev{phi, tau, M, ld, 1, 1, 1}; }
 

@@ -162,7 +162,8 @@ enum : int
 {
   DYN_REGRESSOR_ = 1,
   DYN_TORQUE_ = 2,
-  DYN_INERTIA_ = 4
+  DYN_INERTIA_ = 4,
+  DYN_FD_ = 8
 };
 
 }  // namespace rdb
