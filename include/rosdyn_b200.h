@@ -312,6 +312,11 @@ rdb_status rdb_multiplicity(int32_t n_inputs, const int32_t* joint_type_of_input
  * the inertia walkers: Phi[:, block B] = Phi[:, block A] T. */
 rdb_status rdb_fold_parameter_map(const double* R, const double* t, double* T);
 
+/* Host-only utility (used by the tests): the rotation Q (row-major, det +1) with Q e_z = axis that turns the frame of a revolute link of the
+ * folded chain, x_old = Q x_new, so that its joint axis is e_z.  An axis along a coordinate axis gets an exact signed permutation matrix.
+ * RDB_ERR_INVALID_ARG when axis is not a unit vector. */
+rdb_status rdb_fold_canonical_frame(const double* axis, double* Q);
+
 /* ---- normal-equation solve (SURVEY.md section 8f N3; HOST arrays, no reference code: the consumer is external) ------
  * Minimum-norm least-squares solution of gram * parameters = rhs through a symmetric eigen-decomposition: the regressor is rank
  * deficient in the standard parameters, so eigenvalues <= rel_tol * lambda_max (rel_tol <= 0: 1e-10) are discarded.

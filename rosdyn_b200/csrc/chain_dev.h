@@ -26,6 +26,10 @@ struct JointDev
   double axp[3];  // axis in the parent frame, R_pj ax  (primitives_impl.h:69)
 };
 
+// the axis of every revolute joint of the folded chain, in the canonical frame of its link (fold.cpp); the REV generators of the fused
+// kernels (gram_common.cuh) are written for it
+constexpr double REV_AXIS[3] = {0.0, 0.0, 1.0};
+
 struct LinkDev
 {
   // the 10 standard inertial parameters about the link origin in link axes (primitives_impl.h:399-417):

@@ -185,9 +185,10 @@ __device__ __forceinline__ void gen_load(const ChainDev<NJ>& C, const SamplesDev
 }
 
 // One sample per lane: all rows of getRegressor (+ getJointTorque) of sample i written to the slot.
-// REV: every joint of the (folded) chain is revolute -- the usual arm.  The joint type is then a compile-time fact: no type selects, the
-// linear half of every joint screw is an exact zero that is never multiplied, and the projection of a link on its own joint (unit twist
-// [0; axis] at birth) loses its linear terms.
+// REV: every joint of the (folded) chain is revolute about e_z of its link frame -- the usual arm, in the canonical frames of fold.cpp.  The
+// joint type and the axis are then compile-time facts: R = A' Rz(q) mixes two columns of A', the rates gain their e_z terms directly, the
+// first transport of a joint's unit twist [0; e_z] is a row of R, and the projection of a link on its own joint has closed forms with two
+// exact zeros (the mass and m c_z columns).
 // Component columns of every joint row (element-wise in q_j, Dq_j; zero padded to one tile), written after the walk by ONE rolled loop over
 // (joint, column): no call (a called function costs the walker its registers through the ABI -- it spilled 280 bytes per thread into an L1
 // that the slots leave at ~20 KB), little code, and the walk stays one basic block.
@@ -253,6 +254,7 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
                                               const double* __restrict__ tau_meas, double* __restrict__ slot, int64_t i, int lane)
 {
   static_assert(!Z || REV, "the zero mass column of a link on its own joint exists for revolute joints only");
+  static_assert(REV_AXIS[0] == 0.0 && REV_AXIS[1] == 0.0 && REV_AXIS[2] == 1.0, "the REV walk below is written for the axis s = e_z");
   using G = GramGeom<NJ, X, Z>;
   constexpr int P = G::P;
 
@@ -266,8 +268,18 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
     const JointDev& J = C.joint[l];
     const double dql = LAZY ? ld_in(in.dq, J.in, in.ld, i) : x.dq[l], ddql = LAZY ? ld_in(in.ddq, J.in, in.ld, i) : x.ddq[l];
     double R[9];
-    V3 t = v3(J.t);
-    if (REV || J.type == RDB_JOINT_REVOLUTE)
+    const V3 t = REV || J.type != RDB_JOINT_PRISMATIC ? v3(J.t) : axpy(v3(J.t), v3(J.axp), x.q[l]);
+    if (REV)
+    {
+#pragma unroll
+      for (int k = 0; k < 3; k++)
+      {
+        R[3 * k] = fma(x.sv[l], J.A[3 * k + 1], x.cv[l] * J.A[3 * k]);
+        R[3 * k + 1] = fma(-x.sv[l], J.A[3 * k], x.cv[l] * J.A[3 * k + 1]);
+        R[3 * k + 2] = J.A[3 * k + 2];
+      }
+    }
+    else if (J.type == RDB_JOINT_REVOLUTE)
     {
       const double c1 = 1.0 - x.cv[l];
 #pragma unroll
@@ -277,11 +289,7 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
     {
 #pragma unroll
       for (int k = 0; k < 9; k++) R[k] = J.A[k];
-      if (J.type == RDB_JOINT_PRISMATIC) t = axpy(t, v3(J.axp), x.q[l]);
     }
-    const V3 axj = v3(J.ax);
-    const V3 su = (!REV && J.type == RDB_JOINT_PRISMATIC) ? axj : v3(0, 0, 0);
-    const V3 ss = (REV || J.type == RDB_JOINT_REVOLUTE) ? axj : v3(0, 0, 0);
     v = rotT(R, cross_add(v, w, t));
     w = rotT(R, w);
     a = rotT(R, cross_add(a, al, t));
@@ -289,55 +297,87 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
     g = rotT(R, g);
     if (REV)
     {
-      w = axpy(w, ss, dql);
-      a = axpy(a, cross(v, ss), dql);
-      al = axpy(axpy(al, cross(w, ss), dql), ss, ddql);
+      // s = e_z:  w += s Dq,  a += (v x s) Dq,  al += (w x s) Dq + s DDq
+      w.z += dql;
+      a.x = fma(v.y, dql, a.x);
+      a.y = fma(-v.x, dql, a.y);
+      al.x = fma(w.y, dql, al.x);
+      al.y = fma(-w.x, dql, al.y);
+      al.z += ddql;
     }
     else
     {
+      const V3 axj = v3(J.ax);
+      const V3 su = J.type == RDB_JOINT_PRISMATIC ? axj : v3(0, 0, 0);
+      const V3 ss = J.type == RDB_JOINT_REVOLUTE ? axj : v3(0, 0, 0);
       v = axpy(v, su, dql);
       w = axpy(w, ss, dql);
       const V3 xl = cross_add(cross(w, su), v, ss);
       const V3 xa = cross(w, ss);
       a = axpy(axpy(a, xl, dql), su, ddql);
       al = axpy(axpy(al, xa, dql), ss, ddql);
+      U[l] = su;
+      S[l] = ss;
     }
 #pragma unroll
     for (int j = 0; j < l; j++)
     {
-      U[j] = rotT(R, cross_add(U[j], S[j], t));
-      S[j] = rotT(R, S[j]);
+      if (REV && j == l - 1)  // [0; e_z] of joint l-1 moved to link l: S = R^T e_z, U = R^T (e_z x t)
+      {
+        S[j] = v3(R[6], R[7], R[8]);
+        U[j] = v3(fma(t.x, R[3], -(t.y * R[0])), fma(t.x, R[4], -(t.y * R[1])), fma(t.x, R[5], -(t.y * R[2])));
+      }
+      else
+      {
+        U[j] = rotT(R, cross_add(U[j], S[j], t));
+        S[j] = rotT(R, S[j]);
+      }
     }
-    U[l] = su;
-    S[l] = ss;
     tau[l] = 0.0;
     const double* Pl = C.link[l].pi;
     const V3 fm = cross_add(a - g, w, v);
 #pragma unroll
     for (int j = 0; j <= l; j++)
     {
-      const V3 u = U[j], s = S[j];
-      const bool own = REV && j == l;  // u == 0 exactly
-      const double e0 = own ? 0.0 : dot(u, fm);
-      const V3 h = own ? cross(fm, s) : cross_add(cross_add(cross(u, al), w, cross(w, u)), fm, s);
-      const V3 rho = cross(s, w);
+      const bool own = REV && j == l;  // unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
       double e[10];
-      e[0] = e0;
-      e[1] = h.x;
-      e[2] = h.y;
-      e[3] = h.z;
-      e[4] = fma(s.x, al.x, rho.x * w.x);
-      e[5] = fma(s.x, al.y, fma(s.y, al.x, fma(rho.x, w.y, rho.y * w.x)));
-      e[6] = fma(s.x, al.z, fma(s.z, al.x, fma(rho.x, w.z, rho.z * w.x)));
-      e[7] = fma(s.y, al.y, rho.y * w.y);
-      e[8] = fma(s.y, al.z, fma(s.z, al.y, fma(rho.y, w.z, rho.z * w.y)));
-      e[9] = fma(s.z, al.z, rho.z * w.z);
-      // tau_j += Phi_{j,l,:} . pi_l in two independent chains
+      if (own)
+      {
+        e[0] = 0.0;
+        e[1] = fm.y;
+        e[2] = -fm.x;
+        e[3] = 0.0;
+        e[7] = w.x * w.y;
+        e[4] = -e[7];
+        e[5] = fma(w.x, w.x, -(w.y * w.y));
+        e[6] = fma(-w.y, w.z, al.x);
+        e[8] = fma(w.x, w.z, al.y);
+        e[9] = al.z;
+      }
+      else
+      {
+        const V3 u = U[j], s = S[j];
+        const V3 h = cross_add(cross_add(cross(u, al), w, cross(w, u)), fm, s);
+        const V3 rho = cross(s, w);
+        e[0] = dot(u, fm);
+        e[1] = h.x;
+        e[2] = h.y;
+        e[3] = h.z;
+        e[4] = fma(s.x, al.x, rho.x * w.x);
+        e[5] = fma(s.x, al.y, fma(s.y, al.x, fma(rho.x, w.y, rho.y * w.x)));
+        e[6] = fma(s.x, al.z, fma(s.z, al.x, fma(rho.x, w.z, rho.z * w.x)));
+        e[7] = fma(s.y, al.y, rho.y * w.y);
+        e[8] = fma(s.y, al.z, fma(s.z, al.y, fma(rho.y, w.z, rho.z * w.y)));
+        e[9] = fma(s.z, al.z, rho.z * w.z);
+      }
+      // tau_j += Phi_{j,l,:} . pi_l in two independent chains (the exact zeros of the own joint are not multiplied)
       double t0 = tau[j], t1 = e[1] * Pl[1];
 #pragma unroll
-      for (int p = 0; p < 10; p += 2) t0 = fma(e[p], Pl[p], t0);
+      for (int p = 0; p < 10; p += 2)
+        if (!(own && p == 0)) t0 = fma(e[p], Pl[p], t0);
 #pragma unroll
-      for (int p = 3; p < 10; p += 2) t1 = fma(e[p], Pl[p], t1);
+      for (int p = 3; p < 10; p += 2)
+        if (!(own && p == 3)) t1 = fma(e[p], Pl[p], t1);
       tau[j] = t0 + t1;
       double* o = slot + G::rowbase(j);
 #pragma unroll

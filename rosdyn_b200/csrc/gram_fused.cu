@@ -19,6 +19,8 @@
 //     phase: the writer of a slot changes from use to use).
 //   * all-revolute chains drop the exact-zero mass column of a link on its own joint (GramGeom Z): the rows are one position shorter,
 //     98 instead of 104 DMMA per 4 samples for 6 joints (143 / 149 for 7).
+//   * all-revolute chains whose folded axes are all e_z (fold.cpp puts every revolute link in such a canonical frame) run the REV generator,
+//     which holds the axis as a compile-time constant: 2 019 instead of 2 412 FP64 instructions per sample for 6 joints (2 658 / 3 119 for 7).
 // Per-CTA partials are summed in a fixed order by gram_fused_reduce_kernel (bit-reproducible for a given n).
 // gram_ext_kernel: the extended model [Phi | Phi_c] (friction / spring columns) in ONE pass -- the same slots, the component columns of
 // every joint in a small side buffer next to each slot, the MMA warps keep the rigid-body tiles and the cross tiles in registers.
@@ -794,8 +796,7 @@ cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double*
                               int accumulate, cudaStream_t st)
 {
   if (in.n <= 0 || ch.gram.fold_version != ch.model_version) return cudaErrorNotSupported;
-  bool rev = true;  // all moving joints revolute: the specialised generator
-  for (int j = 0; j < ch.gram.fold.nj; j++) rev = rev && ch.gram.fold.joint[j].type == RDB_JOINT_REVOLUTE;
+  const bool rev = fold_rev_canonical(ch.gram.fold);  // all moving joints revolute about e_z: the specialised generator
   switch (ch.gram.fold.nj)  // moving joints; every joint of the folded chain is an input
   {
 #define X(N)                                                                                                    \
@@ -969,8 +970,7 @@ cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const dou
       xmap[Pc + c.col + p] = g;
     }
   }
-  bool rev = true;
-  for (int j = 0; j < K; j++) rev = rev && F.joint[j].type == RDB_JOINT_REVOLUTE;
+  const bool rev = fold_rev_canonical(F);
   const int zc = GF_ZCOL && rev ? 1 : 0;  // GramGeom Z of the kernel that will run
   int xcmax = 0;
   for (int j = 0; j < K; j++) xcmax = std::max(xcmax, (int)gc.ncols[j]);

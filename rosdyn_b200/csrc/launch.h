@@ -147,8 +147,18 @@ cudaError_t launch_components_regressor(const ChainHost& ch, const SamplesDev& i
 cudaError_t launch_components_torque(const ChainHost& ch, const SamplesDev& in, const ComponentParams& prm, double* torque, int64_t ld_out,
                                      int accumulate, cudaStream_t st);
 cudaError_t fp64_peak(int kind, int reps, double* tflops);
-// fold.cpp: the chain with its never-moving joints folded away (ch.gram.fold); rebuilt by every model upload
+// fold.cpp: the chain with its never-moving joints folded away and its revolute axes on +z (ch.gram.fold); rebuilt by every model upload
 cudaError_t fold_chain(ChainHost& ch);
+// every joint of the folded chain is revolute about exactly e_z of its link frame: the fused kernels' REV generators (gram_common.cuh) hold
+// the axis as a compile-time constant; any other chain takes the generic generator
+inline bool fold_rev_canonical(const ChainDev<RDB_MAX_JOINTS>& F)
+{
+  bool rev = true;
+  for (int j = 0; j < F.nj; j++)
+    rev = rev && F.joint[j].type == RDB_JOINT_REVOLUTE && F.joint[j].ax[0] == REV_AXIS[0] && F.joint[j].ax[1] == REV_AXIS[1] &&
+          F.joint[j].ax[2] == REV_AXIS[2];
+  return rev;
+}
 // gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                               int accumulate, cudaStream_t st);

@@ -406,8 +406,7 @@ cudaError_t launch_gram_ring(ChainHost& ch, const SamplesDev& in, const double* 
                              int accumulate, cudaStream_t st)
 {
   if (in.n <= 0 || ch.gram.fold_version != ch.model_version) return cudaErrorNotSupported;
-  bool rev = true;  // all moving joints revolute: the specialised generator and the shorter rows
-  for (int j = 0; j < ch.gram.fold.nj; j++) rev = rev && ch.gram.fold.joint[j].type == RDB_JOINT_REVOLUTE;
+  const bool rev = fold_rev_canonical(ch.gram.fold);  // all moving joints revolute about e_z: the specialised generator and the shorter rows
   switch (ch.gram.fold.nj)
   {
 #define X(N)                                                                                              \
