@@ -95,6 +95,8 @@ SYMBOLS = {
     "rdb_regressor_gram_batch_host": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32]),
     "rdb_chain_create_on": (i32, [ctypes.POINTER(CChainDesc), i32, ctypes.POINTER(ctypes.c_void_p)]),
     "rdb_chain_device": (i32, [ctypes.c_void_p]),
+    "rdb_chain_gram_kernel_info": (i32, [ctypes.c_void_p, ctypes.POINTER(i32), ctypes.c_char_p, i32]),
+    "rdb_gram_specialised_cubin": (i32, [ctypes.POINTER(CChainDesc), ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, ctypes.c_char_p, i32]),
     "rdb_regressor_gram_sharded_host": (i32, [ctypes.POINTER(ctypes.c_void_p), i32, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32]),
     "rdb_group_create": (i32, [ctypes.POINTER(CChainDesc), i32, ctypes.POINTER(i32), ctypes.POINTER(ctypes.c_void_p)]),
     "rdb_group_unique_id": (i32, [ctypes.POINTER(ctypes.c_uint8)]),

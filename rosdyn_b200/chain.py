@@ -474,6 +474,14 @@ class Chain:
             info = int(info[0]) if info is not None else None
         return (ddq, info) if with_info else ddq
 
+    def gramKernelInfo(self):
+        """(specialised, reason) of the fused kernel the last regressorGram* call ran: 1 compiled at run time against this chain's
+        constants, 0 precompiled, -1 no call yet (rdb_chain_gram_kernel_info)."""
+        flag = ctypes.c_int32(-1)
+        buf = ctypes.create_string_buffer(4096)
+        check(self._lib.rdb_chain_gram_kernel_info(self._h, ctypes.byref(flag), buf, len(buf)))
+        return flag.value, buf.value.decode(errors="replace")
+
     def regressorGram(self, q, Dq, DDq, tau_meas=None, out=None):
         """Fused getRegressor -> normal equations: returns (G[P,P], b[P], tau_sq[1]) with
         G = sum Phi^T Phi, b = sum Phi^T tau, tau_sq = sum tau^T tau; tau = tau_meas or getJointTorque.

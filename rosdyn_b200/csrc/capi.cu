@@ -8,6 +8,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
 #include <thread>
@@ -596,6 +597,42 @@ rdb_status rdb_chain_create_on(const rdb_chain_desc* desc, int32_t device, rdb_c
 }
 
 int32_t rdb_chain_device(const rdb_chain* chain) { return chain ? chain->device : -1; }
+
+rdb_status rdb_gram_specialised_cubin(const rdb_chain_desc* desc, const char* kernel_args, const char* arch, const char* path, char* reason,
+                                      int32_t reason_len)
+{
+  if (!desc || !kernel_args || !arch || !path) return fail(RDB_ERR_INVALID_ARG, "null argument");
+  if (desc->n_joints < 0 || desc->n_joints > RDB_MAX_JOINTS) return fail(RDB_ERR_INVALID_ARG, "n_joints out of range");
+  if (desc->n_inputs < 0 || desc->n_inputs > RDB_MAX_JOINTS) return fail(RDB_ERR_INVALID_ARG, "n_inputs out of range");
+  if (desc->n_joints > 0 && !desc->joints) return fail(RDB_ERR_INVALID_ARG, "null joints");
+  if (!desc->links) return fail(RDB_ERR_INVALID_ARG, "null links");
+  std::unique_ptr<ChainHost> ch(new (std::nothrow) ChainHost());
+  if (!ch) return fail(RDB_ERR_ALLOC, "out of host memory");
+  rdb_status s = build_model(desc, ch.get());
+  if (s != RDB_OK) return s;
+  if (fold_chain(*ch, false) != cudaSuccess) return fail(RDB_ERR_INVALID_ARG, "fold_chain failed");
+  if (!fold_rev_canonical(ch->gram.fold)) return fail(RDB_ERR_INVALID_ARG, "the folded chain is not all-revolute about e_z: no specialised kernel");
+  std::vector<char> cubin;
+  std::string why;
+  const bool ok = gram_jit_cubin(ch->gram.fold, kernel_args, gram_jit_defines(), arch, cubin, why);
+  if (reason && reason_len > 0) snprintf(reason, (size_t)reason_len, "%s", why.c_str());
+  if (!ok) return fail(RDB_ERR_CUDA, "NVRTC: " + why);
+  FILE* f = fopen(path, "wb");
+  if (!f) return fail(RDB_ERR_INVALID_ARG, std::string("cannot write ") + path);
+  const bool wrote = fwrite(cubin.data(), 1, cubin.size(), f) == cubin.size();
+  if (fclose(f) != 0 || !wrote) return fail(RDB_ERR_INVALID_ARG, std::string("writing ") + path + " failed");
+  return RDB_OK;
+}
+
+rdb_status rdb_chain_gram_kernel_info(const rdb_chain* chain, int32_t* specialised, char* reason, int32_t reason_len)
+{
+  if (!chain) return fail(RDB_ERR_INVALID_ARG, "null chain");
+  rdb_chain* ch = const_cast<rdb_chain*>(chain);
+  RDB_LOCK(ch);
+  if (specialised) *specialised = ch->gram.kernel_specialised;
+  if (reason && reason_len > 0) snprintf(reason, (size_t)reason_len, "%s", ch->gram.kernel_why.c_str());
+  return RDB_OK;
+}
 
 rdb_status rdb_regressor_gram_sharded_host(rdb_chain* const* chains, int32_t n_chains, const rdb_samples* in, const double* tau_meas,
                                            double* gram, double* rhs, double* tau_sq, int32_t accumulate)

@@ -127,7 +127,7 @@ namespace rdb
 {
 
 // (re)builds ch.gram.fold* for the current model (called by every model upload, capi.cu)
-cudaError_t fold_chain(ChainHost& ch)
+cudaError_t fold_chain(ChainHost& ch, bool upload)
 {
   GramWorkspace& w = ch.gram;
   if (w.fold_version == ch.model_version) return cudaSuccess;
@@ -208,7 +208,7 @@ cudaError_t fold_chain(ChainHost& ch)
   }
   F.nj = K;
   w.fold_identity = (K == H.nj) && !rotated;
-  if (!w.fold_identity && K > 0)
+  if (upload && !w.fold_identity && K > 0)
   {
     const size_t need = sizeof(double) * ((size_t)H.nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1)) + sizeof(int32_t) * H.nj;
     if (w.fold_bytes < need)
@@ -226,7 +226,7 @@ cudaError_t fold_chain(ChainHost& ch)
     e = cudaMemcpy(w.fold_dev + (size_t)H.nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1), kof.data(), sizeof(int32_t) * H.nj, cudaMemcpyHostToDevice);
     if (e != cudaSuccess) return e;
   }
-  w.fold_version = ch.model_version;
+  if (upload) w.fold_version = ch.model_version;
   return cudaSuccess;
 }
 

@@ -1,12 +1,13 @@
 // gram_common.cuh -- pieces shared by the fused regressor -> normal-equation kernels (gram_fused.cu: shared-memory slots filled directly by the
 // generator warps; gram_ring.cu: generator warps decoupled from the slots through an L2-resident ring and TMA bulk copies): geometry of the
 // augmented Gram matrix, mbarrier / DMMA wrappers, and the per-sample regressor generator.
+// The header is also compiled at run time by NVRTC (gram_jit.cpp), which has no system headers: it needs chain_dev.h and spatial.cuh only.
 #pragma once
+#ifndef __CUDACC_RTC__
 #include <cuda_runtime.h>
+#endif
 
-#include <type_traits>
-
-#include "launch.h"
+#include "chain_dev.h"
 #include "spatial.cuh"
 
 namespace rdb
@@ -51,14 +52,19 @@ __device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity)
       : "memory");
 }
 
-// compile-time loop: f(std::integral_constant<int, B>) ... f(std::integral_constant<int, E - 1>), so that indices derived from the loop
-// variable are constant expressions (accumulator arrays indexed through constexpr tables must stay in registers)
+template <int V>
+struct ic
+{
+  static constexpr int value = V;
+};
+// compile-time loop: f(ic<B>) ... f(ic<E - 1>), so that indices derived from the loop variable are constant expressions (accumulator arrays
+// indexed through constexpr tables must stay in registers)
 template <int B, int E, class F>
 __device__ __forceinline__ void static_for(F&& f)
 {
   if constexpr (B < E)
   {
-    f(std::integral_constant<int, B>{});
+    f(ic<B>{});
     static_for<B + 1, E>(f);
   }
 }
@@ -166,6 +172,156 @@ struct GramComps
                             // component regressor of components.cu keeps the reference's division)
 };
 
+// ---------------------------------------------------------------------------------------------- model constants and typed arithmetic
+// The walk reads the model (A' and t' of every folded joint, the lumped parameters pi', gravity) through kc<M, ...>.  RtModel: the
+// __grid_constant__ ChainDev of the kernel, values ptxas cannot see (the precompiled kernels).  Any other M is a type generated at run time
+// for one chain (gram_jit.cpp) whose constexpr M::val(field, link, k) holds the exact values: kc then returns Zr for an exact 0, Un<+-1> for
+// an exact +-1 and the value itself otherwise, and the t* operations below drop a product with Zr and turn one with Un into a pass-through or
+// a negation.  Everything else is the same operation in the same order as with RtModel (no reassociation, no snapping of tiny values), so for
+// finite inputs the results are bit-identical up to the sign of exact zeros.  The t* operations use the _rn intrinsics, which are never
+// contracted: a product that loses its addend must not be fused into a later addition that the precompiled kernel rounds separately.
+struct RtModel
+{
+  static constexpr bool RUNTIME = true;
+};
+enum : int
+{
+  MK_A = 0,   // A'[link][0..8]
+  MK_T = 1,   // t'[link][0..2]
+  MK_PI = 2,  // pi'[link][0..9]
+  MK_G = 3    // g[0..2]
+};
+struct Zr
+{
+};
+template <int S>
+struct Un
+{
+};
+template <class T>
+struct tv_unit
+{
+  static constexpr int s = 0;
+};
+template <int S>
+struct tv_unit<Un<S>>
+{
+  static constexpr int s = S;
+};
+template <class T>
+struct tv_zero
+{
+  static constexpr bool v = false;
+};
+template <>
+struct tv_zero<Zr>
+{
+  static constexpr bool v = true;
+};
+
+template <class M, int F, int L, int K, int NJ>
+__device__ __forceinline__ auto kc(const ChainDev<NJ>& C)
+{
+  if constexpr (M::RUNTIME)
+  {
+    if constexpr (F == MK_A) return C.joint[L].A[K];
+    else if constexpr (F == MK_T) return C.joint[L].t[K];
+    else if constexpr (F == MK_PI) return C.link[L].pi[K];
+    else return C.g[K];
+  }
+  else
+  {
+    constexpr double v = M::val(F, L, K);
+    if constexpr (v == 0.0) return Zr{};
+    else if constexpr (v == 1.0) return Un<1>{};
+    else if constexpr (v == -1.0) return Un<-1>{};
+    else return v;
+  }
+}
+
+template <class A>
+__device__ __forceinline__ double tv_d(A a)
+{
+  if constexpr (tv_zero<A>::v) return 0.0;
+  else if constexpr (tv_unit<A>::s != 0) return (double)tv_unit<A>::s;
+  else return a;
+}
+template <class A>
+__device__ __forceinline__ auto tneg(A a)
+{
+  if constexpr (tv_zero<A>::v) return Zr{};
+  else if constexpr (tv_unit<A>::s != 0) return Un<-tv_unit<A>::s>{};
+  else return -a;
+}
+template <class A, class B>
+__device__ __forceinline__ auto tmul(A a, B b)
+{
+  constexpr int ua = tv_unit<A>::s, ub = tv_unit<B>::s;
+  if constexpr (tv_zero<A>::v || tv_zero<B>::v) return Zr{};
+  else if constexpr (ua != 0 && ub != 0) return Un<ua * ub>{};
+  else if constexpr (ua != 0) return ua > 0 ? b : -b;
+  else if constexpr (ub != 0) return ub > 0 ? a : -a;
+  else return __dmul_rn(a, b);
+}
+template <class A, class B>
+__device__ __forceinline__ auto tadd(A a, B b)
+{
+  if constexpr (tv_zero<A>::v) return b;
+  else if constexpr (tv_zero<B>::v) return a;
+  else return __dadd_rn(tv_d(a), tv_d(b));
+}
+// fma(a, b, c): with c == 0 the rounded product, with a or b == +-1 the rounded sum
+template <class A, class B, class C>
+__device__ __forceinline__ auto tfma(A a, B b, C c)
+{
+  using P = decltype(tmul(a, b));
+  if constexpr (tv_zero<P>::v) return c;
+  else if constexpr (tv_zero<C>::v) return tmul(a, b);
+  else if constexpr (tv_unit<A>::s != 0 || tv_unit<B>::s != 0) return tadd(tmul(a, b), c);
+  else return __fma_rn(a, b, tv_d(c));
+}
+
+template <class X, class Y, class W>
+struct T3
+{
+  X x;
+  Y y;
+  W z;
+};
+template <class X, class Y, class W>
+__device__ __forceinline__ T3<X, Y, W> mk3(X x, Y y, W z)
+{
+  return T3<X, Y, W>{x, y, z};
+}
+template <class A>
+__device__ __forceinline__ V3 tod3(const A& a)
+{
+  return V3{tv_d(a.x), tv_d(a.y), tv_d(a.z)};
+}
+// the operations of spatial.cuh, in the same order, on typed vectors (V3 or T3)
+template <class A, class B>
+__device__ __forceinline__ auto tdot(const A& a, const B& b)
+{
+  return tfma(a.x, b.x, tfma(a.y, b.y, tmul(a.z, b.z)));
+}
+template <class A, class B>
+__device__ __forceinline__ auto tcross(const A& a, const B& b)
+{
+  return mk3(tfma(a.y, b.z, tneg(tmul(a.z, b.y))), tfma(a.z, b.x, tneg(tmul(a.x, b.z))), tfma(a.x, b.y, tneg(tmul(a.y, b.x))));
+}
+template <class Cv, class A, class B>
+__device__ __forceinline__ auto tcross_add(const Cv& c, const A& a, const B& b)
+{
+  return mk3(tfma(a.y, b.z, tfma(tneg(a.z), b.y, c.x)), tfma(a.z, b.x, tfma(tneg(a.x), b.z, c.y)), tfma(a.x, b.y, tfma(tneg(a.y), b.x, c.z)));
+}
+// R^T a, R given by its rows R.x, R.y, R.z
+template <class R, class A>
+__device__ __forceinline__ auto trotT(const R& r, const A& a)
+{
+  return mk3(tfma(r.x.x, a.x, tfma(r.y.x, a.y, tmul(r.z.x, a.z))), tfma(r.x.y, a.x, tfma(r.y.y, a.y, tmul(r.z.y, a.z))),
+             tfma(r.x.z, a.x, tfma(r.y.z, a.y, tmul(r.z.z, a.z))));
+}
+
 // ---------------------------------------------------------------------------------------------- generator
 template <int NJ>
 struct GenIn
@@ -184,11 +340,6 @@ __device__ __forceinline__ void gen_load(const ChainDev<NJ>& C, const SamplesDev
   }
 }
 
-// One sample per lane: all rows of getRegressor (+ getJointTorque) of sample i written to the slot.
-// REV: every joint of the (folded) chain is revolute about e_z of its link frame -- the usual arm, in the canonical frames of fold.cpp.  The
-// joint type and the axis are then compile-time facts: R = A' Rz(q) mixes two columns of A', the rates gain their e_z terms directly, the
-// first transport of a joint's unit twist [0; e_z] is a row of R, and the projection of a link on its own joint has closed forms with two
-// exact zeros (the mass and m c_z columns).
 // Component columns of every joint row (element-wise in q_j, Dq_j; zero padded to one tile), written after the walk by ONE rolled loop over
 // (joint, column): no call (a called function costs the walker its registers through the ABI -- it spilled 280 bytes per thread into an L1
 // that the slots leave at ~20 KB), little code, and the walk stays one basic block.
@@ -247,19 +398,116 @@ __device__ __forceinline__ void st_row(double* p, double v)
   else *p = v;
 }
 
-// LAZY: Dq / DDq of a link are loaded inside the walk (the compiler hoists them as far as registers allow) instead of being held in registers
-// from before the wait for the output buffer: with two generator warps per sub-partition the latency hides behind the other warp
-template <int NJ, bool REV, int X, int Z = 0, bool GLOBAL = false, bool LAZY = false>
-__device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramComps* comps, const GenIn<NJ>& x, const SamplesDev& in,
-                                              const double* __restrict__ tau_meas, double* __restrict__ slot, int64_t i, int lane)
+// the projection Phi[j, block of link L] = e of joint j's unit twist (u, s) moved to link L: tau_j += e . pi_L in two independent chains,
+// e stored into the row of joint j.  OWN: the projection of a revolute link on its own joint (e[0] == e[3] == 0, typed Zr, not multiplied).
+template <class M, int NJ, int X, int Z, bool GLOBAL, int L, int J, bool OWN, class E0, class E1, class E2, class E3, class E4, class E5, class E6,
+          class E7, class E8, class E9>
+__device__ __forceinline__ void gram_emit(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, E0 e0, E1 e1, E2 e2, E3 e3,
+                                          E4 e4, E5 e5, E6 e6, E7 e7, E8 e8, E9 e9)
 {
-  static_assert(!Z || REV, "the zero mass column of a link on its own joint exists for revolute joints only");
-  static_assert(REV_AXIS[0] == 0.0 && REV_AXIS[1] == 0.0 && REV_AXIS[2] == 1.0, "the REV walk below is written for the axis s = e_z");
   using G = GramGeom<NJ, X, Z>;
-  constexpr int P = G::P;
+  auto P = [&](auto pc) { return kc<M, MK_PI, L, decltype(pc)::value>(C); };
+  auto t0a = [&] {  // joint L's torque starts here: from +0.0 as the precompiled kernel always did, from nothing with a compile-time model
+    if constexpr (J == L && M::RUNTIME) return 0.0;
+    else if constexpr (J == L) return Zr{};
+    else return tau[J];
+  }();
+  const auto t0 = tfma(e8, P(ic<8>{}), tfma(e6, P(ic<6>{}), tfma(e4, P(ic<4>{}), tfma(e2, P(ic<2>{}), tfma(e0, P(ic<0>{}), t0a)))));
+  const auto t1 = tfma(e9, P(ic<9>{}), tfma(e7, P(ic<7>{}), tfma(e5, P(ic<5>{}), tfma(e3, P(ic<3>{}), tmul(e1, P(ic<1>{}))))));
+  tau[J] = tv_d(tadd(t0, t1));
+  double* o = slot + G::rowbase(J);
+  const double e[10] = {tv_d(e0), tv_d(e1), tv_d(e2), tv_d(e3), tv_d(e4), tv_d(e5), tv_d(e6), tv_d(e7), tv_d(e8), tv_d(e9)};
+#pragma unroll
+  for (int p = 0; p < 10; p++)
+    if (!(Z && OWN && p == 0))  // Z: the exact zero at the end of the row is not stored
+      st_row<GLOBAL>(o + G::pos(L, p) * 32 + (lane ^ (4 * (G::pos(L, p) & 3))), e[p]);
+}
+template <class M, int NJ, int X, int Z, bool GLOBAL, int L, int J, class U, class S>
+__device__ __forceinline__ void gram_project(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, const U& u, const S& s,
+                                             const V3& fm, const V3& w, const V3& al)
+{
+  const auto h = tcross_add(tcross_add(tcross(u, al), w, tcross(w, u)), fm, s);
+  const auto rho = tcross(s, w);
+  gram_emit<M, NJ, X, Z, GLOBAL, L, J, false>(
+      C, tau, slot, lane, tdot(u, fm), h.x, h.y, h.z, tfma(s.x, al.x, tmul(rho.x, w.x)),
+      tfma(s.x, al.y, tfma(s.y, al.x, tfma(rho.x, w.y, tmul(rho.y, w.x)))), tfma(s.x, al.z, tfma(s.z, al.x, tfma(rho.x, w.z, tmul(rho.z, w.x)))),
+      tfma(s.y, al.y, tmul(rho.y, w.y)), tfma(s.y, al.z, tfma(s.z, al.y, tfma(rho.y, w.z, tmul(rho.z, w.y)))), tfma(s.z, al.z, tmul(rho.z, w.z)));
+}
 
+// One sample per lane: all rows of getRegressor (+ getJointTorque) of sample i written to the slot.
+// REV: every joint of the (folded) chain is revolute about e_z of its link frame -- the usual arm, in the canonical frames of fold.cpp.  The
+// joint type and the axis are then compile-time facts: R = A' Rz(q) mixes two columns of A', the rates gain their e_z terms directly, the
+// first transport of a joint's unit twist [0; e_z] is a row of R, and the projection of a link on its own joint has closed forms with two
+// exact zeros (the mass and m c_z columns).  M: where the model constants come from (RtModel, or a run-time generated model type).
+template <int NJ, class M, int X, int Z, bool GLOBAL, bool LAZY>
+__device__ __forceinline__ void gram_walk_rev(const ChainDev<NJ>& C, const GenIn<NJ>& x, const SamplesDev& in, double* __restrict__ slot, int64_t i,
+                                              int lane, double (&tau)[NJ])
+{
+  static_assert(REV_AXIS[0] == 0.0 && REV_AXIS[1] == 0.0 && REV_AXIS[2] == 1.0, "the REV walk below is written for the axis s = e_z");
   V3 U[NJ], S[NJ];
-  double tau[NJ];
+  V3 v = v3(0, 0, 0), w = v3(0, 0, 0), a = v3(0, 0, 0), al = v3(0, 0, 0), g;
+  static_for<0, NJ>([&](auto lc) {
+    constexpr int l = decltype(lc)::value;
+    const JointDev& J = C.joint[l];
+    const double dql = LAZY ? ld_in(in.dq, J.in, in.ld, i) : x.dq[l], ddql = LAZY ? ld_in(in.ddq, J.in, in.ld, i) : x.ddq[l];
+    const double sl = x.sv[l], cl = x.cv[l];
+    const auto t = mk3(kc<M, MK_T, l, 0>(C), kc<M, MK_T, l, 1>(C), kc<M, MK_T, l, 2>(C));
+    // R = A' Rz(q), row k: (fma(s, A'[k][1], c A'[k][0]), fma(-s, A'[k][0], c A'[k][1]), A'[k][2])
+    auto row = [&](auto kc_) {
+      constexpr int k = decltype(kc_)::value;
+      const auto a0 = kc<M, MK_A, l, 3 * k>(C);
+      const auto a1 = kc<M, MK_A, l, 3 * k + 1>(C);
+      return mk3(tfma(sl, a1, tmul(cl, a0)), tfma(-sl, a0, tmul(cl, a1)), kc<M, MK_A, l, 3 * k + 2>(C));
+    };
+    const auto R = mk3(row(ic<0>{}), row(ic<1>{}), row(ic<2>{}));
+    v = tod3(trotT(R, tcross_add(v, w, t)));
+    w = tod3(trotT(R, w));
+    a = tod3(trotT(R, tcross_add(a, al, t)));
+    al = tod3(trotT(R, al));
+    if constexpr (l == 0) g = tod3(trotT(R, mk3(kc<M, MK_G, 0, 0>(C), kc<M, MK_G, 0, 1>(C), kc<M, MK_G, 0, 2>(C))));
+    else g = tod3(trotT(R, g));
+    // s = e_z:  w += s Dq,  a += (v x s) Dq,  al += (w x s) Dq + s DDq
+    w.z += dql;
+    a.x = fma(v.y, dql, a.x);
+    a.y = fma(-v.x, dql, a.y);
+    al.x = fma(w.y, dql, al.x);
+    al.y = fma(-w.x, dql, al.y);
+    al.z += ddql;
+    static_for<0, (l > 0 ? l - 1 : 0)>([&](auto jc) {
+      constexpr int j = decltype(jc)::value;
+      U[j] = tod3(trotT(R, tcross_add(U[j], S[j], t)));
+      S[j] = tod3(trotT(R, S[j]));
+    });
+    // [0; e_z] of joint l-1 moved to link l: S = R^T e_z, U = R^T (e_z x t) -- typed, for the projection of this link
+    const auto S1 = R.z;
+    const auto U1 = mk3(tfma(t.x, R.y.x, tneg(tmul(t.y, R.x.x))), tfma(t.x, R.y.y, tneg(tmul(t.y, R.x.y))), tfma(t.x, R.y.z, tneg(tmul(t.y, R.x.z))));
+    if constexpr (l > 0)
+    {
+      S[l - 1] = tod3(S1);
+      U[l - 1] = tod3(U1);
+    }
+    const V3 fm = cross_add(a - g, w, v);
+    static_for<0, l + 1>([&](auto jc) {
+      constexpr int j = decltype(jc)::value;
+      if constexpr (j == l)  // unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
+      {
+        const double e7 = w.x * w.y;
+        gram_emit<M, NJ, X, Z, GLOBAL, l, j, true>(C, tau, slot, lane, Zr{}, fm.y, -fm.x, Zr{}, -e7, fma(w.x, w.x, -(w.y * w.y)),
+                                                   fma(-w.y, w.z, al.x), e7, fma(w.x, w.z, al.y), al.z);
+      }
+      else if constexpr (j == l - 1) gram_project<M, NJ, X, Z, GLOBAL, l, j>(C, tau, slot, lane, U1, S1, fm, w, al);
+      else gram_project<M, NJ, X, Z, GLOBAL, l, j>(C, tau, slot, lane, U[j], S[j], fm, w, al);
+    });
+  });
+}
+
+// any joint types and axes (the constant-bank model)
+template <int NJ, int X, int Z, bool GLOBAL, bool LAZY>
+__device__ __forceinline__ void gram_walk_gen(const ChainDev<NJ>& C, const GenIn<NJ>& x, const SamplesDev& in, double* __restrict__ slot, int64_t i,
+                                              int lane, double (&tau)[NJ])
+{
+  using G = GramGeom<NJ, X, Z>;
+  V3 U[NJ], S[NJ];
   V3 v = v3(0, 0, 0), w = v3(0, 0, 0), a = v3(0, 0, 0), al = v3(0, 0, 0);
   V3 g = v3(C.g);
 #pragma unroll
@@ -268,18 +516,8 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
     const JointDev& J = C.joint[l];
     const double dql = LAZY ? ld_in(in.dq, J.in, in.ld, i) : x.dq[l], ddql = LAZY ? ld_in(in.ddq, J.in, in.ld, i) : x.ddq[l];
     double R[9];
-    const V3 t = REV || J.type != RDB_JOINT_PRISMATIC ? v3(J.t) : axpy(v3(J.t), v3(J.axp), x.q[l]);
-    if (REV)
-    {
-#pragma unroll
-      for (int k = 0; k < 3; k++)
-      {
-        R[3 * k] = fma(x.sv[l], J.A[3 * k + 1], x.cv[l] * J.A[3 * k]);
-        R[3 * k + 1] = fma(-x.sv[l], J.A[3 * k], x.cv[l] * J.A[3 * k + 1]);
-        R[3 * k + 2] = J.A[3 * k + 2];
-      }
-    }
-    else if (J.type == RDB_JOINT_REVOLUTE)
+    const V3 t = J.type != RDB_JOINT_PRISMATIC ? v3(J.t) : axpy(v3(J.t), v3(J.axp), x.q[l]);
+    if (J.type == RDB_JOINT_REVOLUTE)
     {
       const double c1 = 1.0 - x.cv[l];
 #pragma unroll
@@ -295,43 +533,22 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
     a = rotT(R, cross_add(a, al, t));
     al = rotT(R, al);
     g = rotT(R, g);
-    if (REV)
-    {
-      // s = e_z:  w += s Dq,  a += (v x s) Dq,  al += (w x s) Dq + s DDq
-      w.z += dql;
-      a.x = fma(v.y, dql, a.x);
-      a.y = fma(-v.x, dql, a.y);
-      al.x = fma(w.y, dql, al.x);
-      al.y = fma(-w.x, dql, al.y);
-      al.z += ddql;
-    }
-    else
-    {
-      const V3 axj = v3(J.ax);
-      const V3 su = J.type == RDB_JOINT_PRISMATIC ? axj : v3(0, 0, 0);
-      const V3 ss = J.type == RDB_JOINT_REVOLUTE ? axj : v3(0, 0, 0);
-      v = axpy(v, su, dql);
-      w = axpy(w, ss, dql);
-      const V3 xl = cross_add(cross(w, su), v, ss);
-      const V3 xa = cross(w, ss);
-      a = axpy(axpy(a, xl, dql), su, ddql);
-      al = axpy(axpy(al, xa, dql), ss, ddql);
-      U[l] = su;
-      S[l] = ss;
-    }
+    const V3 axj = v3(J.ax);
+    const V3 su = J.type == RDB_JOINT_PRISMATIC ? axj : v3(0, 0, 0);
+    const V3 ss = J.type == RDB_JOINT_REVOLUTE ? axj : v3(0, 0, 0);
+    v = axpy(v, su, dql);
+    w = axpy(w, ss, dql);
+    const V3 xl = cross_add(cross(w, su), v, ss);
+    const V3 xa = cross(w, ss);
+    a = axpy(axpy(a, xl, dql), su, ddql);
+    al = axpy(axpy(al, xa, dql), ss, ddql);
+    U[l] = su;
+    S[l] = ss;
 #pragma unroll
     for (int j = 0; j < l; j++)
     {
-      if (REV && j == l - 1)  // [0; e_z] of joint l-1 moved to link l: S = R^T e_z, U = R^T (e_z x t)
-      {
-        S[j] = v3(R[6], R[7], R[8]);
-        U[j] = v3(fma(t.x, R[3], -(t.y * R[0])), fma(t.x, R[4], -(t.y * R[1])), fma(t.x, R[5], -(t.y * R[2])));
-      }
-      else
-      {
-        U[j] = rotT(R, cross_add(U[j], S[j], t));
-        S[j] = rotT(R, S[j]);
-      }
+      U[j] = rotT(R, cross_add(U[j], S[j], t));
+      S[j] = rotT(R, S[j]);
     }
     tau[l] = 0.0;
     const double* Pl = C.link[l].pi;
@@ -339,53 +556,46 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
 #pragma unroll
     for (int j = 0; j <= l; j++)
     {
-      const bool own = REV && j == l;  // unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
+      const V3 u = U[j], s = S[j];
+      const V3 h = cross_add(cross_add(cross(u, al), w, cross(w, u)), fm, s);
+      const V3 rho = cross(s, w);
       double e[10];
-      if (own)
-      {
-        e[0] = 0.0;
-        e[1] = fm.y;
-        e[2] = -fm.x;
-        e[3] = 0.0;
-        e[7] = w.x * w.y;
-        e[4] = -e[7];
-        e[5] = fma(w.x, w.x, -(w.y * w.y));
-        e[6] = fma(-w.y, w.z, al.x);
-        e[8] = fma(w.x, w.z, al.y);
-        e[9] = al.z;
-      }
-      else
-      {
-        const V3 u = U[j], s = S[j];
-        const V3 h = cross_add(cross_add(cross(u, al), w, cross(w, u)), fm, s);
-        const V3 rho = cross(s, w);
-        e[0] = dot(u, fm);
-        e[1] = h.x;
-        e[2] = h.y;
-        e[3] = h.z;
-        e[4] = fma(s.x, al.x, rho.x * w.x);
-        e[5] = fma(s.x, al.y, fma(s.y, al.x, fma(rho.x, w.y, rho.y * w.x)));
-        e[6] = fma(s.x, al.z, fma(s.z, al.x, fma(rho.x, w.z, rho.z * w.x)));
-        e[7] = fma(s.y, al.y, rho.y * w.y);
-        e[8] = fma(s.y, al.z, fma(s.z, al.y, fma(rho.y, w.z, rho.z * w.y)));
-        e[9] = fma(s.z, al.z, rho.z * w.z);
-      }
-      // tau_j += Phi_{j,l,:} . pi_l in two independent chains (the exact zeros of the own joint are not multiplied)
+      e[0] = dot(u, fm);
+      e[1] = h.x;
+      e[2] = h.y;
+      e[3] = h.z;
+      e[4] = fma(s.x, al.x, rho.x * w.x);
+      e[5] = fma(s.x, al.y, fma(s.y, al.x, fma(rho.x, w.y, rho.y * w.x)));
+      e[6] = fma(s.x, al.z, fma(s.z, al.x, fma(rho.x, w.z, rho.z * w.x)));
+      e[7] = fma(s.y, al.y, rho.y * w.y);
+      e[8] = fma(s.y, al.z, fma(s.z, al.y, fma(rho.y, w.z, rho.z * w.y)));
+      e[9] = fma(s.z, al.z, rho.z * w.z);
+      // tau_j += Phi_{j,l,:} . pi_l in two independent chains
       double t0 = tau[j], t1 = e[1] * Pl[1];
 #pragma unroll
-      for (int p = 0; p < 10; p += 2)
-        if (!(own && p == 0)) t0 = fma(e[p], Pl[p], t0);
+      for (int p = 0; p < 10; p += 2) t0 = fma(e[p], Pl[p], t0);
 #pragma unroll
-      for (int p = 3; p < 10; p += 2)
-        if (!(own && p == 3)) t1 = fma(e[p], Pl[p], t1);
+      for (int p = 3; p < 10; p += 2) t1 = fma(e[p], Pl[p], t1);
       tau[j] = t0 + t1;
       double* o = slot + G::rowbase(j);
 #pragma unroll
-      for (int p = 0; p < 10; p++)
-        if (!(Z && own && p == 0))  // Z: the exact zero at the end of the row is not stored
-          st_row<GLOBAL>(o + G::pos(l, p) * 32 + (lane ^ (4 * (G::pos(l, p) & 3))), e[p]);
+      for (int p = 0; p < 10; p++) st_row<GLOBAL>(o + G::pos(l, p) * 32 + (lane ^ (4 * (G::pos(l, p) & 3))), e[p]);
     }
   }
+}
+
+// LAZY: Dq / DDq of a link are loaded inside the walk (the compiler hoists them as far as registers allow) instead of being held in registers
+// from before the wait for the output buffer: with two generator warps per sub-partition the latency hides behind the other warp
+template <int NJ, bool REV, int X, int Z = 0, bool GLOBAL = false, bool LAZY = false, class M = RtModel>
+__device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramComps* comps, const GenIn<NJ>& x, const SamplesDev& in,
+                                              const double* __restrict__ tau_meas, double* __restrict__ slot, int64_t i, int lane)
+{
+  static_assert(!Z || REV, "the zero mass column of a link on its own joint exists for revolute joints only");
+  static_assert(REV || M::RUNTIME, "compile-time models are built for the REV walk");
+  using G = GramGeom<NJ, X, Z>;
+  double tau[NJ];
+  if constexpr (REV) gram_walk_rev<NJ, M, X, Z, GLOBAL, LAZY>(C, x, in, slot, i, lane, tau);
+  else gram_walk_gen<NJ, X, Z, GLOBAL, LAZY>(C, x, in, slot, i, lane, tau);
 #pragma unroll
   for (int j = 0; j < NJ; j++)
   {

@@ -4,6 +4,8 @@
 
 #include <atomic>
 #include <mutex>
+#include <string>
+#include <vector>
 
 #include "chain_dev.h"
 
@@ -25,6 +27,9 @@ struct GramWorkspace
   size_t fold_bytes = 0;
   double* ext_dev = nullptr;   // extended model: rigid-body block | cross-tile sums | cross partials | component map
   size_t ext_bytes = 0;
+  // which fused kernel the last Gram call ran (rdb_chain_gram_kernel_info): 1 run-time specialised (gram_jit.cpp), 0 precompiled, -1 none yet
+  int kernel_specialised = -1;
+  std::string kernel_why = "no fused Gram call yet";
 };
 
 // persistent pipeline of rdb_regressor_gram_batch_host (capi.cu)
@@ -148,7 +153,7 @@ cudaError_t launch_components_torque(const ChainHost& ch, const SamplesDev& in, 
                                      int accumulate, cudaStream_t st);
 cudaError_t fp64_peak(int kind, int reps, double* tflops);
 // fold.cpp: the chain with its never-moving joints folded away and its revolute axes on +z (ch.gram.fold); rebuilt by every model upload
-cudaError_t fold_chain(ChainHost& ch);
+cudaError_t fold_chain(ChainHost& ch, bool upload = true);  // upload = false: the host image ch.gram.fold only
 // every joint of the folded chain is revolute about exactly e_z of its link frame: the fused kernels' REV generators (gram_common.cuh) hold
 // the axis as a compile-time constant; any other chain takes the generic generator
 inline bool fold_rev_canonical(const ChainDev<RDB_MAX_JOINTS>& F)
@@ -159,6 +164,15 @@ inline bool fold_rev_canonical(const ChainDev<RDB_MAX_JOINTS>& F)
           F.joint[j].ax[2] == REV_AXIS[2];
   return rev;
 }
+// gram_jit.cpp: the fused kernel `kernel_args` ("gram_fused_kernel<6, 4, true, 0, 4": template arguments without the model) compiled at run
+// time against the constants of ch.gram.fold, or nullptr when the precompiled instantiation has to run; records which one and why in ch.gram.
+// defines: gram_jit_defines() (the launcher's geometry macros), compiled in front of the kernel headers and part of the cache key
+const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args, const std::string& defines);
+// gram_jit.cpp: the same kernel's cubin for `arch` (e.g. "sm_100a") without a device (rdb_gram_specialised_cubin)
+bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const std::string& defines, const char* arch,
+                    std::vector<char>& cubin, std::string& why);
+// gram_fused.cu: "#define GF_TSPLIT ..." lines with the values of the overridable geometry macros the launchers were compiled with
+std::string gram_jit_defines();
 // gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                               int accumulate, cudaStream_t st);

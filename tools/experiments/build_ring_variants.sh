@@ -4,7 +4,7 @@ set -e
 cd "$(dirname "$0")/.."
 NV="/usr/local/cuda/bin/nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo -Xcompiler -fPIC -ccbin /usr/bin/g++ -DRDB_DEV_SWITCHES"
 mkdir -p build/obj_dev
-for src in kernels.cu gram.cu gram_fused.cu gram_ring.cu components.cu aux.cu ik.cu group.cu capi.cu urdf.cpp solve.cpp fold.cpp; do
+for src in kernels.cu gram.cu gram_fused.cu gram_ring.cu gram_jit.cpp gram_jit_headers.cpp components.cu aux.cu ik.cu group.cu capi.cu urdf.cpp solve.cpp fold.cpp; do
   f=${src%.*}
   if [ "$src" = gram.cu ] || [ "$src" = gram_fused.cu ] || [ "$src" = gram_ring.cu ]; then
     $NV -c rosdyn_b200/csrc/$src -o build/obj_dev/$f.o &
@@ -17,7 +17,7 @@ link() { # name, extra objects override
   mkdir -p build/var_$1
   /usr/local/cuda/bin/nvcc -shared -cudart static -ccbin /usr/bin/g++ -gencode arch=compute_100a,code=sm_100a -o build/var_$1/librosdyn_b200.so "${@:2}" -ldl
 }
-objs() { for f in kernels gram gram_fused gram_ring components aux ik group capi urdf solve fold; do echo build/obj_dev/$f.o; done; }
+objs() { for f in kernels gram gram_fused gram_ring gram_jit gram_jit_headers components aux ik group capi urdf solve fold; do echo build/obj_dev/$f.o; done; }
 link dev $(objs)
 for v in "$@"; do
   case $v in

@@ -26,6 +26,7 @@
 #include <cstdint>
 
 #include "gram_common.cuh"
+#include "launch.h"
 
 namespace rdb
 {

@@ -31,7 +31,7 @@ def main():
     out, lines = {}, []
     for f in funcs:
         dem = subprocess.run(["c++filt", f], capture_output=True, text=True).stdout.strip()
-        m = re.search(r"gram_fused_kernel<(\d+), (\d+), (true|false|\(bool\)[01]), (\d+)(?:, (\d+))?>", dem)
+        m = re.search(r"gram_fused_kernel<(\d+), (\d+), (true|false|\(bool\)[01]), (\d+)(?:, (\d+))?(?:, rdb::RtModel)?>", dem)
         if not m:
             continue
         K, slots, rev, X = int(m.group(1)), int(m.group(2)), m.group(3) in ("true", "(bool)1"), int(m.group(4))
@@ -45,7 +45,7 @@ def main():
         dmma = sum(1 for i in ins if "DMMA" in i["text"])
         dp = sum(cnt.values())
         key = f"K{K}_{'rev' if rev else 'gen'}"
-        out[key] = {"kernel": dem.split("(")[0].replace("void rdb::", ""), "slots": slots, "generator_warps": int(m.group(5) or slots),
+        out[key] = {"kernel": dem.split("(")[0].replace("void rdb::", "").replace(", rdb::RtModel>", ">"), "slots": slots, "generator_warps": int(m.group(5) or slots),
                     "gen_dp_instr_per_sample": dp,
                     # flop per sample: every lane of a generator warp instruction works on its own sample
                     "gen_flop_per_sample": float(2 * cnt["DFMA"] + cnt["DMUL"] + cnt["DADD"]),
