@@ -317,6 +317,12 @@ rdb_status rdb_fold_parameter_map(const double* R, const double* t, double* T);
  * RDB_ERR_INVALID_ARG when axis is not a unit vector. */
 rdb_status rdb_fold_canonical_frame(const double* axis, double* Q);
 
+/* Host-only utility (used by the tests): the row layout of the fused normal-equation kernel on all-revolute folded chains of nj (1..7) moving
+ * joints.  pos[j * 10 nj + c]: the position of parameter column c inside the kernel's row of joint j, or -1 where the row stores nothing (the
+ * blocks of the links before j, and the columns the all-revolute regressor makes exact zeros); rowlen[j]: the positions of that row;
+ * *tau_col: 1 when tau is position 0 of every row, 0 when it is accumulated beside the tiles.  RDB_ERR_INVALID_ARG for other nj. */
+rdb_status rdb_gram_row_layout(int32_t nj, int32_t* pos, int32_t* rowlen, int32_t* tau_col);
+
 /* ---- normal-equation solve (SURVEY.md section 8f N3; HOST arrays, no reference code: the consumer is external) ------
  * Minimum-norm least-squares solution of gram * parameters = rhs through a symmetric eigen-decomposition: the regressor is rank
  * deficient in the standard parameters, so eigenvalues <= rel_tol * lambda_max (rel_tol <= 0: 1e-10) are discarded.

@@ -83,6 +83,7 @@ SYMBOLS = {
     "rdb_regressor_gram_ext_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32, ctypes.c_void_p]),
     "rdb_fold_parameter_map": (i32, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
     "rdb_fold_canonical_frame": (i32, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
+    "rdb_gram_row_layout": (i32, [i32, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i32)]),
     "rdb_multiplicity": (i32, [i32, ctypes.POINTER(i32), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),
                                ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), i64, ctypes.POINTER(i64)]),
     "rdb_normal_equations_solve": (i32, [i32, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), ctypes.c_double, ctypes.c_double,

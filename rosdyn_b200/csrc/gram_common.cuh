@@ -72,16 +72,65 @@ __device__ __forceinline__ void static_for(F&& f)
 // geometry of the augmented Gram matrix and of a slot for a (folded) chain of NJ joints, all of them inputs.
 // X = 1 (cross mode, extended model [Phi | Phi_c]): every row carries GX_COLS component columns of its own joint after the tau column.
 constexpr int GX_COLS = 8;  // component columns per joint row (one 8-wide tile)
-// Z = 1 (all-revolute chains, gram_ring.cu): the projection of a link on its OWN revolute joint has no mass term (the unit twist at birth is
-// [0; axis], so Phi[j, 10 j + 0] == 0 exactly).  Inside every link block the mass column therefore comes LAST (p order 1..9, 0): the row of
-// joint j then ends with an exact zero that is neither stored nor multiplied -- rowlen(j) = 10 (NJ - j), and position 10 NJ (the mass of the
-// first moving link, an identically zero column of Phi) is never touched.
+// Z = 1 (all-revolute chains: gram_ext_kernel, gram_ring.cu): the projection of a link on its OWN revolute joint has no mass term (the unit
+// twist at birth is [0; axis], so Phi[j, 10 j + 0] == 0 exactly).  Inside every link block the mass column therefore comes LAST (p order
+// 1..9, 0): the row of joint j then ends with an exact zero that is neither stored nor multiplied -- rowlen(j) = 10 (NJ - j), and position
+// 10 NJ (the mass of the first moving link, an identically zero column of Phi) is never touched.
+// Z = 2 (all-revolute chains: the rigid-body gram_fused_kernel) drops every column that the REV walk (gram_walk_rev) makes an exact zero:
+//   * the own-joint projection [0; e_z] has m c_z == 0 as well as m == 0 (gram_walk_rev, branch j == l);
+//   * the first moving link sits on the fixed base: there v = a = 0, w = (0, 0, Dq_0), alpha = (0, 0, DDq_0), so of its own-joint closed
+//     forms only I_zz = alpha_z, m c_x = fm_y and m c_y = -fm_x are not exact zeros (I_xx, I_xy, I_xz, I_yy, I_yz are -w_x w_y,
+//     w_x^2 - w_y^2, fma(-w_y, w_z, alpha_x), w_x w_y, fma(w_x, w_z, alpha_y) with w_x = w_y = alpha_x = alpha_y = 0).  Link 0 appears in
+//     row 0 only, so these seven are identically zero columns of Phi and have no position at all.
+// Inside every link block the order is I_zz, m c_x, m c_y, I_xx .. I_yz, m c_z, m (inblk): the own block of row j >= 1 is the first 8
+// positions of its block, that of row 0 the first 3.  With GF_TAU_TILE == 0 tau is no column of the tiles either: its row sits behind the
+// regressor rows of the slot and the MMA warps accumulate Phi^T tau and tau^T tau by DFMA on the fragments they load for the DMMAs
+// (gram_tau_step): rowlen(0) = 10 (NJ - 1) + 3, rowlen(j >= 1) = 10 (NJ - j) - 2, C6 81 instead of 98 DMMA per 4 samples.  With
+// GF_TAU_TILE == 1 tau stays the tile column at position 0 (C6 90 DMMA per 4 samples).
+#ifndef GF_TAU_TILE
+#define GF_TAU_TILE 0
+#endif
 template <int NJ, int X = 0, int Z = 0>
 struct GramGeom
 {
   static constexpr int P = 10 * NJ;
-  static constexpr int T = (P + 1 - Z + 7) / 8;   // tile columns of the augmented matrix
+  static constexpr int TC = Z == 2 && !GF_TAU_TILE ? 0 : 1;  // tau positions in front of the link blocks (position 0 when TC == 1)
+  // place of parameter p (m, m c_xyz, I_xx, I_xy, I_xz, I_yy, I_yz, I_zz) inside its link block, and back
+  __host__ __device__ static constexpr int inblk(int p)
+  {
+    constexpr int zord[10] = {9, 1, 2, 8, 3, 4, 5, 6, 7, 0};
+    return Z == 2 ? zord[p] : (Z == 1 ? (p == 0 ? 9 : p - 1) : p);
+  }
+  __host__ __device__ static constexpr int param_at(int q)
+  {
+    constexpr int zinv[10] = {9, 1, 2, 4, 5, 6, 7, 8, 3, 0};
+    return Z == 2 ? zinv[q] : (Z == 1 ? (q == 9 ? 0 : q + 1) : q);
+  }
+  // Column order inside the kernel: tau (TC == 1: POSITION 0), then the link blocks from the LAST link to the first (position of column
+  // 10 l + p: TC + 10 (NJ-1-l) + inblk(p)).  The row of joint j is non-zero in the blocks of the links >= j, i.e. in the positions
+  // [0, rowlen(j)) -- a prefix, aligned with the 8-wide tiles at its start, ragged only at its end: row j needs the tiles I, K < tj(j)
+  // (with the natural order, where a row starts at column 10 j in the middle of a tile, C6 took 109 DMMA per 4 samples).
+  __host__ __device__ static constexpr int pos(int l, int p) { return TC + 10 * (NJ - 1 - l) + inblk(p); }
+  // is column 10 l + p of the row of joint j (l >= j) stored, i.e. not one of the exact zeros the layout drops
+  __host__ __device__ static constexpr bool stored(int j, int l, int p)
+  {
+    if (j != l || Z == 0) return true;
+    if (Z == 1) return p != 0;
+    return l == 0 ? (p == 1 || p == 2 || p == 9) : (p != 0 && p != 3);
+  }
+  __host__ __device__ static constexpr int rowlen(int j)
+  {
+    return Z == 2 ? TC + 10 * (NJ - 1 - j) + (j == 0 ? 3 : 8) : 1 + 10 * (NJ - j) - Z;
+  }
+  static constexpr int NPOS = rowlen(0);  // positions that exist
+  // parameter column at a position (P: tau), and whether a parameter column has a position (else it is identically zero in Phi)
+  __host__ __device__ static constexpr int col_of(int q) { return q < TC ? P : 10 * (NJ - 1 - (q - TC) / 10) + param_at((q - TC) % 10); }
+  __host__ __device__ static constexpr bool has_pos(int c) { return c / 10 > 0 || stored(0, 0, c % 10); }
+  static constexpr int T = (NPOS + 7) / 8;    // tile columns of the augmented matrix
   static constexpr int NT = T * (T + 1) / 2;  // upper-triangular tiles
+  static constexpr int NF = T + 1 - TC;       // values a lane loads per k-step: one per tile column, then (TC == 0) the tau of its sample
+  // per-CTA partial: the NT tiles (64 doubles each), then with TC == 0 b by position (8 T) and tau^T tau
+  static constexpr int PARTIAL = NT * 64 + (TC ? 0 : 8 * T + 1);
   static constexpr int KPW = 8 / GF_KSPLIT;   // k-steps (4 samples) of one MMA warp per joint row and slot
   static constexpr int NSTEPS = NJ * KPW;     // k-steps of one MMA warp per slot
   __host__ __device__ static constexpr int threads(int slots) { return 32 * (GF_MMA_WARPS + slots); }
@@ -89,19 +138,21 @@ struct GramGeom
   __host__ __device__ static constexpr int rowbase(int j)
   {
     int o = 0;
-    for (int i = 0; i < j; i++) o += (P + 1 - Z - 10 * i + (X ? GX_COLS : 0)) * 32;
+    for (int i = 0; i < j; i++) o += (rowlen(i) + (X ? GX_COLS : 0)) * 32;
     return o;
   }
-  static constexpr int SLOT_DOUBLES = rowbase(NJ);
+  // offset of the tau row of joint j: position 0 of its row, or (TC == 0) behind all rows, [joint][sample]
+  __host__ __device__ static constexpr int taubase(int j) { return TC ? rowbase(j) : rowbase(NJ) + 32 * j; }
+  static constexpr int SLOT_DOUBLES = rowbase(NJ) + (TC ? 0 : 32 * NJ);
   __host__ __device__ static constexpr int tile(int I, int J) { return I * T - I * (I - 1) / 2 + (J - I); }
   // tile rows owned by an MMA warp: all (TS == 1) or the rows of parity `par` (TS == 2)
   __host__ __device__ static constexpr bool owns(int I, int ts, int par) { return ts == 1 || (I & 1) == par; }
-  __host__ __device__ static constexpr int ntiles(int ts, int par)
+  __host__ __device__ static constexpr int ntiles(int ts, int par)  // at least 1: a warp may own no tile row (T == 1), arrays need a size
   {
     int n = 0;
     for (int I = 0; I < T; I++)
       if (owns(I, ts, par)) n += T - I;
-    return n;
+    return n > 0 ? n : 1;
   }
   __host__ __device__ static constexpr int local(int I, int J, int ts, int par)
   {
@@ -110,12 +161,16 @@ struct GramGeom
       if (owns(K, ts, par)) n += T - K;
     return n + (J - I);
   }
-  // Column order inside the kernel: POSITION 0 is tau, then the link blocks from the LAST link to the first (position of column 10 l + p:
-  // 1 + 10 (NJ-1-l) + p).  The row of joint j is non-zero in the blocks of the links >= j, i.e. in the positions [0, rowlen(j)) -- a prefix,
-  // aligned with the 8-wide tiles at its start, ragged only at its end: row j needs the tiles I, K < tj(j) (C6: 104 DMMA per 4 samples;
-  // with the natural order, where a row starts at column 10 j in the middle of a tile, it was 109).
-  __host__ __device__ static constexpr int pos(int l, int p) { return 1 + 10 * (NJ - 1 - l) + (Z ? (p == 0 ? 9 : p - 1) : p); }
-  __host__ __device__ static constexpr int rowlen(int j) { return 1 + 10 * (NJ - j) - Z; }
+  // TC == 0: DFMA accumulators of an MMA warp -- b at position 8 I + g for each tile row I it owns (lane (g, t): the samples t mod 4), then
+  // in the par 0 warps tau^T tau; bown(I): the accumulator of tile row I
+  __host__ __device__ static constexpr int bown(int I, int ts, int par)
+  {
+    int n = 0;
+    for (int K = 0; K < I; K++)
+      if (owns(K, ts, par)) n++;
+    return n;
+  }
+  __host__ __device__ static constexpr int nbacc(int ts, int par) { return TC || (par != 0 && bown(T, ts, par) == 0) ? 1 : bown(T, ts, par) + (par == 0 ? 1 : 0); }
   __host__ __device__ static constexpr int tj(int j) { return (rowlen(j) + 7) / 8; }
   // cross mode: per joint row j the tiles (regular tile I, component tile of joint j), I = 0 .. tj(j)-1, then (component, component)
   __host__ __device__ static constexpr int xtile(int j, int I)  // I == tj(j): the (component, component) tile
@@ -419,7 +474,7 @@ __device__ __forceinline__ void gram_emit(const ChainDev<NJ>& C, double (&tau)[N
   const double e[10] = {tv_d(e0), tv_d(e1), tv_d(e2), tv_d(e3), tv_d(e4), tv_d(e5), tv_d(e6), tv_d(e7), tv_d(e8), tv_d(e9)};
 #pragma unroll
   for (int p = 0; p < 10; p++)
-    if (!(Z && OWN && p == 0))  // Z: the exact zero at the end of the row is not stored
+    if (G::stored(J, L, p))  // the exact zeros the layout drops are not stored
       st_row<GLOBAL>(o + G::pos(L, p) * 32 + (lane ^ (4 * (G::pos(L, p) & 3))), e[p]);
 }
 template <class M, int NJ, int X, int Z, bool GLOBAL, int L, int J, class U, class S>
@@ -600,7 +655,7 @@ __device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramC
   for (int j = 0; j < NJ; j++)
   {
     const double tv = tau_meas ? __ldcs(tau_meas + (int64_t)C.joint[j].in * in.ld + i) : tau[j];
-    st_row<GLOBAL>(slot + G::rowbase(j) + lane, tv);  // position 0
+    st_row<GLOBAL>(slot + G::taubase(j) + lane, tv);
   }
   if (X) gram_component_columns<NJ>(C, *comps, in, i, slot, lane);
 }
@@ -613,6 +668,7 @@ __device__ __noinline__ void gram_zero_lane(double* __restrict__ slot, int lane)
   for (int j = 0; j < NJ; j++)
   {
     for (int c = 0; c < G::rowlen(j); c++) st_row<GLOBAL>(slot + G::rowbase(j) + c * 32 + (lane ^ (4 * (c & 3))), 0.0);
+    if (!G::TC) st_row<GLOBAL>(slot + G::taubase(j) + lane, 0.0);
     if (X)
       for (int c = 0; c < GX_COLS; c++) st_row<GLOBAL>(slot + G::rowbase(j) + (G::rowlen(j) + c) * 32 + (lane ^ (4 * (c & 3))), 0.0);
   }

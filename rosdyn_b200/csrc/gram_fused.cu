@@ -14,44 +14,57 @@
 namespace rdb
 {
 
-// fixed-order sum of the per-CTA partials -> gram (full symmetric, column-major), rhs, tau_sq
-// zcol: GramGeom Z = 1 position order (the mass column last in every link block; position P does not exist and the row / column of the first
-// moving link's mass, an identically zero column of Phi, is written as exact zeros)
-__global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int nparts, int T, int P, double* __restrict__ gram,
-                                         double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate, int zcol, int pstride)
+// fixed-order sum of the per-CTA partials (GramGeom<NJ, 0, Z>::PARTIAL doubles each, pstride apart) -> gram (full symmetric,
+// column-major), rhs, tau_sq.  One thread per partial entry, and per entry of the P x (P + 1) output: the parameter columns without a position
+// (identically zero columns of Phi, GramGeom::has_pos) get exact zeros in their row, column and rhs.
+template <int NJ, int Z>
+__global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int nparts, int pstride, double* __restrict__ gram,
+                                         double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
 {
-  const int NT = T * (T + 1) / 2;
+  using G = GramGeom<NJ, 0, Z>;
+  constexpr int P = G::P;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= NT * 64) return;
-  double s = 0.0;
-  for (int p = 0; p < nparts; p++) s += partial[(size_t)p * pstride + e];  // pstride: doubles between the partials of two CTAs
-  int k = e >> 6, I = 0;
-  while (k >= T - I)
+  if (!accumulate && e < P * (P + 1))
   {
-    k -= T - I;
+    const int c = e / (P + 1), r = e % (P + 1);  // r == P: rhs
+    if (!G::has_pos(c))
+    {
+      if (r == P) rhs[c] = 0.0;
+      else
+      {
+        gram[(size_t)c * P + r] = 0.0;
+        gram[(size_t)r * P + c] = 0.0;
+      }
+    }
+  }
+  if (e >= G::PARTIAL) return;
+  double s = 0.0;
+  for (int p = 0; p < nparts; p++) s += partial[(size_t)p * pstride + e];
+  if (e >= G::NT * 64)  // TC == 0: b by position, then tau^T tau
+  {
+    const int q = e - G::NT * 64;
+    if (q == 8 * G::T)
+    {
+      if (tau_sq) *tau_sq = accumulate ? *tau_sq + s : s;
+    }
+    else if (q < G::NPOS)
+    {
+      const int a = G::col_of(q);
+      rhs[a] = accumulate ? rhs[a] + s : s;
+    }
+    return;
+  }
+  int k = e >> 6, I = 0;
+  while (k >= G::T - I)
+  {
+    k -= G::T - I;
     I++;
   }
   const int J = I + k;
   const int rp = 8 * I + ((e >> 3) & 7), cp = 8 * J + (e & 7);  // positions inside the kernel (GramGeom::pos)
-  if (zcol && e <= P && !accumulate)  // the untouched mass column of the first moving link (parameter 0): exact zeros
-  {
-    if (e == P) rhs[0] = 0.0;
-    else
-    {
-      gram[(size_t)e * P] = 0.0;
-      gram[e] = 0.0;
-    }
-  }
-  if (rp > P - zcol || cp > P - zcol) return;
+  if (rp >= G::NPOS || cp >= G::NPOS) return;
   if (I == J && rp > cp) return;  // diagonal tiles hold both halves; keep the upper one
-  // position -> column of the (folded) parameter vector, P = tau
-  const int nj = P / 10;
-  auto col_of = [&](int pos) {
-    if (pos == 0) return P;
-    const int q = (pos - 1) % 10;
-    return 10 * (nj - 1 - (pos - 1) / 10) + (zcol ? (q == 9 ? 0 : q + 1) : q);
-  };
-  const int row = col_of(rp), col = col_of(cp);
+  const int row = G::col_of(rp), col = G::col_of(cp);  // P: tau
   if (row < P && col < P)
   {
     const double v = accumulate ? gram[(size_t)col * P + row] + s : s;
@@ -65,6 +78,15 @@ __global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int
   }
   else if (tau_sq)
     *tau_sq = accumulate ? *tau_sq + s : s;
+}
+template <int NJ, int Z>
+static void launch_fused_reduce(const double* partial, int nparts, int pstride, double* gram, double* rhs, double* tau_sq, int accumulate,
+                                cudaStream_t st)
+{
+  using G = GramGeom<NJ, 0, Z>;
+  const int n = std::max(G::PARTIAL, G::P * (G::P + 1));
+  gram_fused_reduce_kernel<NJ, Z><<<(n + 255) / 256, 256, 0, st>>>(partial, nparts, pstride, gram, rhs, tau_sq, accumulate);
+  count_launch();
 }
 
 // G = E^T G' E, b = E^T b' (upper triangle computed, mirrored): one thread per entry of the full matrix, 100 products each
@@ -132,7 +154,8 @@ cudaError_t launch_fold_expand(ChainHost& ch, double* gram, double* rhs, double*
 std::string gram_jit_defines()
 {
   char b[160];
-  snprintf(b, sizeof b, "#define GF_TSPLIT %d\n#define GF_ZCOL %d\n#define GF_SPIN_NS %d\n", (int)GF_TSPLIT, (int)GF_ZCOL, (int)GF_SPIN_NS);
+  snprintf(b, sizeof b, "#define GF_TSPLIT %d\n#define GF_ZCOL %d\n#define GF_TAU_TILE %d\n#define GF_SPIN_NS %d\n", (int)GF_TSPLIT, (int)GF_ZCOL,
+           (int)GF_TAU_TILE, (int)GF_SPIN_NS);
   return b;
 }
 
@@ -193,9 +216,9 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
                                    int accumulate, cudaStream_t st)
 {
   constexpr int GENS = gf_gens<SLOTS>();
-  constexpr int Z = GF_ZCOL && REV ? 1 : 0;  // as in the kernel
+  constexpr int Z = GF_ZCOL && REV ? 2 : 0;  // as in the kernel
   using G = GramGeom<NJ, 0, Z>;
-  const size_t smem = sizeof(double) * (size_t)std::max(G::SLOT_DOUBLES * SLOTS, G::NT * 64);
+  const size_t smem = sizeof(double) * (size_t)std::max(G::SLOT_DOUBLES * SLOTS, G::PARTIAL);
   const void* kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, 0, GENS>);
   {
     const void* jk = gram_kernel_for<REV>(ch, "gram_fused_kernel<%d, %d, true, 0, %d", NJ, SLOTS, GENS);
@@ -207,7 +230,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
   const int64_t ngroups = (in.n + 31) / 32;
   const int grid = (int)std::min<int64_t>(ch.sm_count, GENS != SLOTS ? ngroups : (ngroups + SLOTS - 1) / SLOTS);
   {
-    cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::NT * 64);
+    cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL);
     if (e != cudaSuccess) return e;
   }
   {
@@ -224,8 +247,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
   count_launch();
   if (ch.gram.fold_identity)
   {
-    gram_fused_reduce_kernel<<<(G::NT * 64 + 255) / 256, 256, 0, st>>>(ch.gram.fused_partials, grid, G::T, G::P, gram, rhs, tau_sq, accumulate, Z, G::NT * 64);
-    count_launch();
+    launch_fused_reduce<NJ, Z>(ch.gram.fused_partials, grid, G::PARTIAL, gram, rhs, tau_sq, accumulate, st);
     return cudaGetLastError();
   }
   // folded chain: reduce into G', b', then expand to the reference's full parameter vector
@@ -234,8 +256,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
   double* Gr = Tm + (size_t)nj * 100;
   double* br = Gr + (size_t)Pr * Pr;
   double* tsr = br + Pr;
-  gram_fused_reduce_kernel<<<(G::NT * 64 + 255) / 256, 256, 0, st>>>(ch.gram.fused_partials, grid, G::T, G::P, Gr, br, tsr, 0, Z, G::NT * 64);
-  count_launch();
+  launch_fused_reduce<NJ, Z>(ch.gram.fused_partials, grid, G::PARTIAL, Gr, br, tsr, 0, st);
   return launch_fold_expand(ch, gram, rhs, tau_sq, accumulate, st);
 }
 
@@ -382,19 +403,13 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const Sampl
     if (e != cudaSuccess) return e;
   }
   count_launch();
-  const int nred = (G0::NT * 64 + 255) / 256;
-  if (ch.gram.fold_identity)
-  {
-    gram_fused_reduce_kernel<<<nred, 256, 0, st>>>(xpart, grid, G0::T, G0::P, Gt, bt, tst, 0, Z, PSTRIDE);
-    count_launch();
-  }
+  if (ch.gram.fold_identity) launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gt, bt, tst, 0, st);
   else
   {
     const int nj = ch.host.nj, Pr = G0::P;
     double* Gr = ch.gram.fold_dev + (size_t)nj * 100;
     double* br = Gr + (size_t)Pr * Pr;
-    gram_fused_reduce_kernel<<<nred, 256, 0, st>>>(xpart, grid, G0::T, G0::P, Gr, br, br + Pr, 0, Z, PSTRIDE);
-    count_launch();
+    launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gr, br, br + Pr, 0, st);
     e = launch_fold_expand(ch, Gt, bt, tst, 0, st);
     if (e != cudaSuccess) return e;
   }
@@ -481,4 +496,32 @@ cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const dou
   return cudaGetLastError();
 }
 
+// the row layout of gram_fused_kernel on all-revolute chains (host entry for tests, rdb_gram_row_layout)
+template <int NJ>
+static void gram_row_layout_nj(int32_t* pos, int32_t* rowlen, int32_t* tau_col)
+{
+  using G = GramGeom<NJ, 0, GF_ZCOL ? 2 : 0>;
+  for (int j = 0; j < NJ; j++)
+  {
+    rowlen[j] = G::rowlen(j);
+    for (int c = 0; c < G::P; c++) pos[j * G::P + c] = c / 10 >= j && G::stored(j, c / 10, c % 10) ? G::pos(c / 10, c % 10) : -1;
+  }
+  *tau_col = G::TC;
+}
+
 }  // namespace rdb
+
+extern "C" rdb_status rdb_gram_row_layout(int32_t nj, int32_t* pos, int32_t* rowlen, int32_t* tau_col)
+{
+  if (!pos || !rowlen || !tau_col) return RDB_ERR_INVALID_ARG;
+  switch (nj)
+  {
+#define X(N)                                                \
+  case N:                                                   \
+    rdb::gram_row_layout_nj<N>(pos, rowlen, tau_col);       \
+    return RDB_OK;
+    X(1) X(2) X(3) X(4) X(5) X(6) X(7)
+#undef X
+  }
+  return RDB_ERR_INVALID_ARG;
+}

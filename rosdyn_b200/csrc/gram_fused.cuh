@@ -17,13 +17,15 @@
 //   * slots cycle through shared-memory mbarriers (full / empty per slot); as many slots as fit the 227 KB (3 for 7 joints, 4 below).  Chains
 //     with only 3 slots still run 4 generator warps, one per SM sub-partition, over them (monotone counters instead of the one-bit mbarrier
 //     phase: the writer of a slot changes from use to use).
-//   * all-revolute chains drop the exact-zero mass column of a link on its own joint (GramGeom Z): the rows are one position shorter,
-//     98 instead of 104 DMMA per 4 samples for 6 joints (143 / 149 for 7).
+//   * all-revolute chains drop the columns their walk makes exact zeros (GramGeom Z = 2): m and m c_z of a link on its own joint, and all
+//     but I_zz, m c_x, m c_y of the first moving link; tau is no tile column but is accumulated by DFMA on the fragments the MMA warps load
+//     anyway (b = Phi^T tau for the tile rows a warp owns, tau^T tau in one warp per k-split): 81 instead of 104 DMMA per 4 samples for 6
+//     joints (125 / 149 for 7), plus 32 (42) DFMA.  The extended model keeps Z = 1 (only the own-joint mass dropped, tau in the tiles).
 //   * all-revolute chains whose folded axes are all e_z (fold.cpp puts every revolute link in such a canonical frame) run the REV generator,
 //     which holds the axis as a compile-time constant: 2 019 instead of 2 412 FP64 instructions per sample for 6 joints (2 658 / 3 119 for 7).
 //   * on such chains the launchers run the same kernel compiled at run time against the chain's own constants (gram_jit.cpp, model type M):
 //     the products with exact zeros and ones are not issued, 1 347 FP64 instructions per sample for C6 (1 851 for C7), same results.
-// Per-CTA partials are summed in a fixed order by gram_fused_reduce_kernel (bit-reproducible for a given n).
+// Per-CTA partials (tiles, then b and tau^T tau) are summed in a fixed order by gram_fused_reduce_kernel (bit-reproducible for a given n).
 // gram_ext_kernel: the extended model [Phi | Phi_c] (friction / spring columns) in ONE pass -- the same slots, the component columns of
 // every joint in a small side buffer next to each slot, the MMA warps keep the rigid-body tiles and the cross tiles in registers.
 //
@@ -47,9 +49,10 @@ namespace rdb
 {
 
 // ---------------------------------------------------------------------------------------------- MMA side
-// B fragments of one k-step (4 samples of joint row J, k-step kk of the slot): lane (g, t) holds column 8 I + g of sample 4 kk + t
+// B fragments of one k-step (4 samples of joint row J, k-step kk of the slot): lane (g, t) holds column 8 I + g of sample 4 kk + t in b[I],
+// and (GramGeom::TC == 0) the tau of joint J for that sample in b[T]
 template <int NJ, int J, int X = 0, int Z = 0>
-__device__ __forceinline__ void gram_load_frags(const double* __restrict__ slot, int kk, int lane, double (&b)[GramGeom<NJ, 0, Z>::T])
+__device__ __forceinline__ void gram_load_frags(const double* __restrict__ slot, int kk, int lane, double (&b)[GramGeom<NJ, 0, Z>::NF])
 {
   using G = GramGeom<NJ, X, Z>;
   constexpr int T = G::T, L = G::rowlen(J), TJ = G::tj(J);
@@ -63,9 +66,10 @@ __device__ __forceinline__ void gram_load_frags(const double* __restrict__ slot,
     if (8 * I + 7 < L || col < L) b[I] = rowp[col * 32];  // only the last tile of the row can be ragged
     else b[I] = 0.0;
   }
+  if constexpr (!G::TC) b[T] = slot[G::taubase(J) + 4 * kk + t];
 }
 template <int NJ, int PAR, int J, int Z>
-__device__ __forceinline__ void gram_mma_step(const double (&b)[GramGeom<NJ, 0, Z>::T], double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2])
+__device__ __forceinline__ void gram_mma_step(const double (&b)[GramGeom<NJ, 0, Z>::NF], double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2])
 {
   using G = GramGeom<NJ, 0, Z>;
   constexpr int T = G::T, TJ = G::tj(J);
@@ -78,33 +82,53 @@ __device__ __forceinline__ void gram_mma_step(const double (&b)[GramGeom<NJ, 0, 
       if (K < TJ) dmma884f(acc[G::local(I, K, GF_TS, PAR)][0], acc[G::local(I, K, GF_TS, PAR)][1], b[I], b[K]);
   }
 }
+// TC == 0: Phi^T tau on the tile rows this warp owns and (par 0) tau^T tau, by DFMA on the fragments of the step's DMMAs
+template <int NJ, int PAR, int J, int Z>
+__device__ __forceinline__ void gram_tau_step(const double (&b)[GramGeom<NJ, 0, Z>::NF], double (&bacc)[GramGeom<NJ, 0, Z>::nbacc(GF_TS, PAR)])
+{
+  using G = GramGeom<NJ, 0, Z>;
+  if constexpr (!G::TC)
+  {
+    static_for<0, G::tj(J)>([&](auto Ic) {
+      constexpr int I = decltype(Ic)::value;
+      if constexpr (G::owns(I, GF_TS, PAR)) bacc[G::bown(I, GF_TS, PAR)] = fma(b[I], b[G::T], bacc[G::bown(I, GF_TS, PAR)]);
+    });
+    if constexpr (PAR == 0) bacc[G::nbacc(GF_TS, PAR) - 1] = fma(b[G::T], b[G::T], bacc[G::nbacc(GF_TS, PAR) - 1]);
+  }
+}
 // k-steps STEP.. of this warp in one slot; step = (joint row, k-step of the warp); the fragments of the next step are in flight while the
 // DMMAs of the current one issue
 template <int NJ, int PAR, int STEP, int Z>
-__device__ __forceinline__ void gram_consume_steps(const double* __restrict__ slot, int ks, int lane, const double (&bcur)[GramGeom<NJ, 0, Z>::T],
-                                                   double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2])
+__device__ __forceinline__ void gram_consume_steps(const double* __restrict__ slot, int ks, int lane, const double (&bcur)[GramGeom<NJ, 0, Z>::NF],
+                                                   double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2],
+                                                   double (&bacc)[GramGeom<NJ, 0, Z>::nbacc(GF_TS, PAR)])
 {
   using G = GramGeom<NJ, 0, Z>;
   constexpr int J = STEP / G::KPW;
   if constexpr (STEP + 1 < G::NSTEPS)
   {
-    double bnext[G::T];
+    double bnext[G::NF];
     gram_load_frags<NJ, (STEP + 1) / G::KPW, 0, Z>(slot, ks * G::KPW + (STEP + 1) % G::KPW, lane, bnext);
     gram_mma_step<NJ, PAR, J, Z>(bcur, acc);
-    gram_consume_steps<NJ, PAR, STEP + 1, Z>(slot, ks, lane, bnext, acc);
+    gram_tau_step<NJ, PAR, J, Z>(bcur, bacc);
+    gram_consume_steps<NJ, PAR, STEP + 1, Z>(slot, ks, lane, bnext, acc, bacc);
   }
   else
+  {
     gram_mma_step<NJ, PAR, J, Z>(bcur, acc);
+    gram_tau_step<NJ, PAR, J, Z>(bcur, bacc);
+  }
 }
 // the k-steps of one slot for this warp
 template <int NJ, int PAR, int Z>
 __device__ __forceinline__ void gram_consume_slot(const double* __restrict__ slot, int ks, int lane,
-                                                  double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2])
+                                                  double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2],
+                                                  double (&bacc)[GramGeom<NJ, 0, Z>::nbacc(GF_TS, PAR)])
 {
   using G = GramGeom<NJ, 0, Z>;
-  double b0[G::T];
+  double b0[G::NF];
   gram_load_frags<NJ, 0, 0, Z>(slot, ks * G::KPW, lane, b0);
-  gram_consume_steps<NJ, PAR, 0, Z>(slot, ks, lane, b0, acc);
+  gram_consume_steps<NJ, PAR, 0, Z>(slot, ks, lane, b0, acc, bacc);
 }
 
 #ifndef GF_SPIN_NS
@@ -173,15 +197,51 @@ __device__ __forceinline__ void gram_mma_reduce(double (&acc)[GramGeom<NJ, 0, Z>
     bar_sync(GF_BAR_REDUCE, 32 * GF_MMA_WARPS);
   }
 }
+// TC == 0: b (8 T doubles by position) and tau^T tau behind the tiles in shared memory, in a fixed order: the four lanes t of a position
+// first, then the k-split warps
+template <int NJ, int PAR, int Z>
+__device__ __forceinline__ void gram_tau_reduce(double (&bacc)[GramGeom<NJ, 0, Z>::nbacc(GF_TS, PAR)], double* smem, int ks, int lane)
+{
+  using G = GramGeom<NJ, 0, Z>;
+  if constexpr (!G::TC)
+  {
+    constexpr int NB = G::nbacc(GF_TS, PAR);
+#pragma unroll
+    for (int k = 0; k < NB; k++)
+    {
+      bacc[k] += __shfl_xor_sync(0xffffffffu, bacc[k], 1);
+      bacc[k] += __shfl_xor_sync(0xffffffffu, bacc[k], 2);
+    }
+    const int g = lane >> 2, t = lane & 3;
+    double* ob = smem + G::NT * 64;
+    for (int w = 0; w < GF_KSPLIT; w++)
+    {
+      if (ks == w && t == 0)
+      {
+#pragma unroll
+        for (int I = 0; I < G::T; I++)
+        {
+          if (!G::owns(I, GF_TS, PAR)) continue;
+          double& o = ob[8 * I + g];
+          o = w == 0 ? bacc[G::bown(I, GF_TS, PAR)] : o + bacc[G::bown(I, GF_TS, PAR)];
+        }
+        if (PAR == 0 && g == 0) ob[8 * G::T] = w == 0 ? bacc[NB - 1] : ob[8 * G::T] + bacc[NB - 1];
+      }
+      bar_sync(GF_BAR_REDUCE, 32 * GF_MMA_WARPS);
+    }
+  }
+}
 
 template <int NJ, int SLOTS, int PAR, int Z>
 __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem, GramBars* bars, int ks, int lane, int dbg)
 {
   using G = GramGeom<NJ, 0, Z>;
   constexpr int NTP = G::ntiles(GF_TS, PAR);
-  double acc[NTP][2];
+  double acc[NTP][2], bacc[G::nbacc(GF_TS, PAR)];
 #pragma unroll
   for (int k = 0; k < NTP; k++) acc[k][0] = acc[k][1] = 0.0;
+#pragma unroll
+  for (int k = 0; k < G::nbacc(GF_TS, PAR); k++) bacc[k] = 0.0;
   const int64_t ngroups = (in.n + 31) / 32;
   const int64_t stride = (int64_t)gridDim.x * SLOTS;
   uint32_t parity = 0;
@@ -195,7 +255,7 @@ __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem
       mbar_wait(&bars->full[s], parity);
       if (!(dbg & 2))
       {
-        gram_consume_slot<NJ, PAR, Z>(slot, ks, lane, acc);
+        gram_consume_slot<NJ, PAR, Z>(slot, ks, lane, acc, bacc);
       }
       if (base + s + stride < ngroups)  // the generator will come back for this slot
       {
@@ -205,6 +265,7 @@ __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem
     }
   }
   gram_mma_reduce<NJ, PAR, Z>(acc, smem, ks, lane);
+  gram_tau_reduce<NJ, PAR, Z>(bacc, smem, ks, lane);
 }
 
 // ---------------------------------------------------------------------------------------------- MMA side, cross mode
@@ -220,7 +281,7 @@ __device__ __forceinline__ double gram_load_xfrag(const double* __restrict__ slo
   return slot[G::rowbase(J) + (G::rowlen(J) + g) * 32 + ((4 * kk + t) ^ (4 * (g & 3)))];
 }
 template <int NJ, int PAR, int J, int Z = 0>
-__device__ __forceinline__ void gram_cross_step(const double (&b)[GramGeom<NJ, 0, Z>::T], double bx,
+__device__ __forceinline__ void gram_cross_step(const double (&b)[GramGeom<NJ, 0, Z>::NF], double bx,
                                                 double (&acc)[GramGeom<NJ, 1, Z>::nxtiles(GF_TS, PAR)][2])
 {
   using G = GramGeom<NJ, 1, Z>;
@@ -335,9 +396,11 @@ __device__ __forceinline__ void gram_mma_role_c(const SamplesDev& in, double* sm
 {
   using G = GramGeom<NJ, 0, Z>;
   constexpr int NTP = G::ntiles(GF_TS, PAR);
-  double acc[NTP][2];
+  double acc[NTP][2], bacc[G::nbacc(GF_TS, PAR)];
 #pragma unroll
   for (int k = 0; k < NTP; k++) acc[k][0] = acc[k][1] = 0.0;
+#pragma unroll
+  for (int k = 0; k < G::nbacc(GF_TS, PAR); k++) bacc[k] = 0.0;
   const int64_t ngroups = (in.n + 31) / 32;
   const int64_t nk = ngroups > blockIdx.x ? (ngroups - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
 #pragma unroll 1
@@ -349,12 +412,13 @@ __device__ __forceinline__ void gram_mma_role_c(const SamplesDev& in, double* sm
     wait_counter_ge(&bars->filled[s], u + 1);
     if (!(dbg & 2))
     {
-      gram_consume_slot<NJ, PAR, Z>(slot, ks, lane, acc);
+      gram_consume_slot<NJ, PAR, Z>(slot, ks, lane, acc, bacc);
     }
     __syncwarp();
     if (lane == 0) red_release_inc(&bars->drained[s]);
   }
   gram_mma_reduce<NJ, PAR, Z>(acc, smem, ks, lane);
+  gram_tau_reduce<NJ, PAR, Z>(bacc, smem, ks, lane);
 }
 
 // ---------------------------------------------------------------------------------------------- extended model [Phi | Phi_c] in ONE pass
@@ -430,7 +494,7 @@ __device__ __forceinline__ double gram_load_xside(const double* __restrict__ sid
 }
 template <int NJ, int PAR, int STEP, int Z, int XC>
 __device__ __forceinline__ void gram_ext_steps(const double* __restrict__ slot, const double* __restrict__ side, int ks, int lane,
-                                               const double (&bcur)[GramGeom<NJ, 0, Z>::T], double bxcur,
+                                               const double (&bcur)[GramGeom<NJ, 0, Z>::NF], double bxcur,
                                                double (&acc)[GramGeom<NJ, 0, Z>::ntiles(GF_TS, PAR)][2],
                                                double (&xacc)[GramGeom<NJ, 1, Z>::nxtiles(GF_TS, PAR)][2])
 {
@@ -438,7 +502,7 @@ __device__ __forceinline__ void gram_ext_steps(const double* __restrict__ slot, 
   constexpr int J = STEP / G::KPW;
   if constexpr (STEP + 1 < G::NSTEPS)
   {
-    double bnext[G::T];
+    double bnext[G::NF];
     constexpr int JN = (STEP + 1) / G::KPW;
     const int kn = ks * G::KPW + (STEP + 1) % G::KPW;
     gram_load_frags<NJ, JN, 0, Z>(slot, kn, lane, bnext);
@@ -474,7 +538,7 @@ __device__ __forceinline__ void gram_ext_mma_role(const SamplesDev& in, double* 
     const double* slot = smem + (size_t)s * G0::SLOT_DOUBLES;
     const double* side = side0 + (size_t)s * gram_ext_side_doubles<NJ, XC>();
     wait_counter_ge(&bars->filled[s], u + 1);
-    double b0[G0::T];
+    double b0[G0::NF];
     gram_load_frags<NJ, 0, 0, Z>(slot, ks * G0::KPW, lane, b0);
     const double bx0 = gram_load_xside<0, XC>(side, ks * G0::KPW, lane);
     gram_ext_steps<NJ, PAR, 0, Z, XC>(slot, side, ks, lane, b0, bx0, acc, xacc);
@@ -548,9 +612,9 @@ __global__ void __launch_bounds__(GramGeom<NJ>::threads(GENS), 1)
     gram_fused_kernel(const __grid_constant__ ChainDev<NJ> C, const __grid_constant__ GramComps comps, const SamplesDev in,
                       const double* __restrict__ tau_meas, double* __restrict__ partial, const int dbg)
 {
-  // Z (gram_common.cuh): on all-revolute chains the mass column of a link on its own joint is an exact zero; it is put last in its block and
-  // neither stored nor multiplied (rigid-body mode only: 98 instead of 104 DMMA per 4 samples for 6 joints, 143 instead of 149 for 7)
-  constexpr int Z = GF_ZCOL && REV && X == 0 ? 1 : 0;
+  // Z = 2 (gram_common.cuh): on all-revolute chains the exact-zero columns of the REV walk are neither stored nor multiplied, and (TC == 0)
+  // tau is accumulated by DFMA beside the tiles: 81 instead of 104 DMMA per 4 samples for 6 joints, 125 instead of 149 for 7
+  constexpr int Z = GF_ZCOL && REV && X == 0 ? 2 : 0;
   using G = GramGeom<NJ, X, Z>;
   extern __shared__ __align__(16) double smem[];
   __shared__ GramBars bars;
@@ -577,7 +641,7 @@ __global__ void __launch_bounds__(GramGeom<NJ>::threads(GENS), 1)
   // ------------------------------------------------ MMA warps: k-split index = warp % 4 (its SM sub-partition), tile-row parity = warp / 4
   const int mma_id = warp;
   const int ks = mma_id % GF_KSPLIT;
-  constexpr int NOUT = (X ? G::NXT : G::NT) * 64;
+  constexpr int NOUT = X ? G::NXT * 64 : G::PARTIAL;
   static_assert(X == 0, "the extended model runs through gram_ext_kernel");
   {
     if constexpr (GENS != SLOTS)

@@ -33,10 +33,11 @@ def count(cubin: str):
     gen = ins[:first_dmma]
     cnt = {op: sum(1 for i in gen if re.match(r"(@!?U?P\d+\s+)?" + op + r"\b", i["text"])) for op in ("DFMA", "DMUL", "DADD")}
     dmma = sum(1 for i in ins if "DMMA" in i["text"])
+    mma_dfma = sum(1 for i in ins[first_dmma:] if re.match(r"(@!?U?P\d+\s+)?DFMA\b", i["text"]))
     res = subprocess.run(["cuobjdump", "-res-usage", cubin], capture_output=True, text=True, check=True).stdout
     m = re.search(r"REG:(\d+) STACK:(\d+)", res)
     return {"gen_dp_instr_per_sample": sum(cnt.values()), "gen_flop_per_sample": float(2 * cnt["DFMA"] + cnt["DMUL"] + cnt["DADD"]),
-            "gen_ops": cnt, "dmma_total": dmma, "dmma_per_4_samples": dmma / KPW,
+            "gen_ops": cnt, "dmma_total": dmma, "dmma_per_4_samples": dmma / KPW, "mma_dfma_per_4_samples": mma_dfma / KPW,
             "registers": int(m.group(1)) if m else None, "stack_bytes": int(m.group(2)) if m else None}
 
 

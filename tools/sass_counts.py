@@ -10,6 +10,8 @@ For every instantiation gram_fused_kernel<K, ..., REV, X = 0>:
   * gen_flop_per_sample     : DFMA = 2 flop, DMUL / DADD = 1 flop.
   * dmma_per_4_samples      : DMMA.8x8x4 of the MMA roles for one k-step (4 samples) of every joint row = all DMMAs of the kernel / k-steps per
     warp and joint row (GramGeom::KPW = 2: the two tile-parity roles each unroll KPW k-steps of every row).
+  * mma_dfma_per_4_samples  : DFMA of the MMA roles (behind the first DMMA) for the same 4 samples: Phi^T tau and tau^T tau accumulated beside
+    the tiles (GramGeom TC == 0).
 bench.py reads the JSON for roofline.executed."""
 import json
 import os
@@ -43,13 +45,15 @@ def main():
         gen = ins[:first_dmma]
         cnt = {op: sum(1 for i in gen if re.match(r"(@!?U?P\d+\s+)?" + op + r"\b", i["text"])) for op in ("DFMA", "DMUL", "DADD")}
         dmma = sum(1 for i in ins if "DMMA" in i["text"])
+        mma_dfma = sum(1 for i in ins[first_dmma:] if re.match(r"(@!?U?P\d+\s+)?DFMA\b", i["text"]))
         dp = sum(cnt.values())
         key = f"K{K}_{'rev' if rev else 'gen'}"
         out[key] = {"kernel": dem.split("(")[0].replace("void rdb::", "").replace(", rdb::RtModel>", ">"), "slots": slots, "generator_warps": int(m.group(5) or slots),
                     "gen_dp_instr_per_sample": dp,
                     # flop per sample: every lane of a generator warp instruction works on its own sample
                     "gen_flop_per_sample": float(2 * cnt["DFMA"] + cnt["DMUL"] + cnt["DADD"]),
-                    "gen_ops": cnt, "dmma_total": dmma, "dmma_per_4_samples": dmma / KPW}
+                    "gen_ops": cnt, "dmma_total": dmma, "dmma_per_4_samples": dmma / KPW,
+                    "mma_dfma_per_4_samples": mma_dfma / KPW}
         lines.append(f"{out[key]['kernel']:48s} generator FP64 instr / sample {dp:5d} (DFMA {cnt['DFMA']}, DMUL {cnt['DMUL']}, DADD {cnt['DADD']}) = "
                      f"{out[key]['gen_flop_per_sample']:.0f} flop;  DMMA.8x8x4 in the kernel {dmma} = {dmma / KPW:.0f} per 4 samples "
                      f"({dmma / KPW * 128:.0f} flop / sample)")
