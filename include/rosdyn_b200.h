@@ -339,9 +339,11 @@ rdb_status rdb_normal_equations_solve(int32_t P, const double* gram, const doubl
  * library needed.  The handles must describe the same chain (same joints / inputs); several handles may share a device. */
 rdb_status rdb_chain_create_on(const rdb_chain_desc* desc, int32_t device, rdb_chain** out);
 int32_t rdb_chain_device(const rdb_chain* chain);
-/* Which fused normal-equation kernel the chain's last rdb_regressor_gram* call ran: *specialised = 1 for the kernel compiled at run time
- * (NVRTC) against the chain's own constants, 0 for the precompiled kernel (chains that are not all-revolute, NVRTC missing or failing,
- * RDB_GRAM_JIT=0), -1 before the first call.  reason (optional, reason_len bytes, NUL-terminated) says why, or how long the compile took. */
+/* Which normal-equation kernel the chain's last rdb_regressor_gram* call ran: *specialised = 1 for the fused kernel compiled at run time
+ * (NVRTC) against the chain's own constants, 0 for the precompiled fused kernel (chains that are not all-revolute, NVRTC missing or failing,
+ * RDB_GRAM_JIT=0), 2 for the general pipeline (materialised regressor and tiled contraction: more than 7 moving joints, no moving joint, or
+ * a component set the one-pass kernel refuses), -1 before the first call.  reason (optional, reason_len bytes, NUL-terminated) says why, or
+ * how long the compile took; for the general pipeline it starts with "general pipeline:". */
 rdb_status rdb_chain_gram_kernel_info(const rdb_chain* chain, int32_t* specialised, char* reason, int32_t reason_len);
 /* Host only, no device needed (inspection tools): the cubin of the run-time specialised kernel of an all-revolute chain, written to `path`.
  * kernel_args: the kernel and its template arguments without the model, e.g. "gram_fused_kernel<6, 4, true, 0, 4"; arch e.g. "sm_100a". */

@@ -475,8 +475,9 @@ class Chain:
         return (ddq, info) if with_info else ddq
 
     def gramKernelInfo(self):
-        """(specialised, reason) of the fused kernel the last regressorGram* call ran: 1 compiled at run time against this chain's
-        constants, 0 precompiled, -1 no call yet (rdb_chain_gram_kernel_info)."""
+        """(specialised, reason) of the kernel the last regressorGram* call ran: 1 fused kernel compiled at run time against this chain's
+        constants, 0 precompiled fused kernel, 2 general pipeline (more than 7 moving joints, no moving joint, or a component set the
+        one-pass kernel refuses; reason starts with "general pipeline:"), -1 no call yet (rdb_chain_gram_kernel_info)."""
         flag = ctypes.c_int32(-1)
         buf = ctypes.create_string_buffer(4096)
         check(self._lib.rdb_chain_gram_kernel_info(self._h, ctypes.byref(flag), buf, len(buf)))

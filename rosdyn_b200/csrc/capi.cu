@@ -250,6 +250,7 @@ void rdb_chain_destroy(rdb_chain* chain)
   if (chain->gram.fused_partials) cudaFree(chain->gram.fused_partials);
   if (chain->gram.fold_dev) cudaFree(chain->gram.fold_dev);
   if (chain->gram.ext_dev) cudaFree(chain->gram.ext_dev);
+  if (chain->gram.tau_sq_part) cudaFree(chain->gram.tau_sq_part);
   if (chain->host_arena.base) cudaFree(chain->host_arena.base);
   if (chain->host_arena.map_h) cudaFreeHost(chain->host_arena.map_h);
   if (chain->host_arena.pin) cudaFreeHost(chain->host_arena.pin);

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <vector>
 
 #include "launch.h"
 
@@ -160,6 +161,38 @@ __global__ void gram_reduce_kernel(const double* __restrict__ partial, int npart
   }
 }
 
+// tau_sq = (accumulate ? tau_sq : 0) + (part + the measured torques of the inputs no chain joint feeds, squared and summed).  The fused
+// kernels walk the folded chain, whose rows are the fed inputs only; such an input has a zero regressor row (nothing to add to G or b) but
+// its torque is part of the residual |tau - Phi pi|^2.  part: the fused kernels' tau^T tau of this call.  One block, fixed order: reproducible.
+struct UnfedRows
+{
+  int32_t n, row[RDB_MAX_JOINTS];
+};
+__global__ void __launch_bounds__(256) gram_unfed_tau_sq_kernel(const double* __restrict__ tau, int64_t ld, int64_t n, UnfedRows u,
+                                                                const double* __restrict__ part, double* __restrict__ tau_sq, int accumulate)
+{
+  __shared__ double red[256];
+  double s = 0.0;
+  for (int r = 0; r < u.n; r++)
+    for (int64_t i = threadIdx.x; i < n; i += blockDim.x)
+    {
+      const double t = tau[(int64_t)u.row[r] * ld + i];
+      s = fma(t, t, s);
+    }
+  red[threadIdx.x] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1)
+  {
+    if ((int)threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0)
+  {
+    const double v = *part + red[0];
+    *tau_sq = accumulate ? *tau_sq + v : v;
+  }
+}
+
 cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
                         cudaStream_t st, bool with_components)
 {
@@ -186,12 +219,43 @@ cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_m
     if (!force_v0)
     {
       cudaError_t e = cudaErrorNotSupported;
+      // measured torques on inputs no chain joint feeds: the fused kernels' tau^T tau goes to a zeroed scratch word first
+      const bool unfed = tau_meas && tau_sq && !ch.inputs_cover_all;
+      if (unfed && !ch.gram.tau_sq_part)
+      {
+        e = cudaMalloc(&ch.gram.tau_sq_part, sizeof(double));
+        if (e != cudaSuccess) return e;
+      }
+      if (unfed) cudaMemsetAsync(ch.gram.tau_sq_part, 0, sizeof(double), st);
+      double* ts = unfed ? ch.gram.tau_sq_part : tau_sq;
       if (P == Pr)
-        e = launch_gram_fused(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
+        e = launch_gram_fused(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
       else
-        e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
+        e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
+      if (e == cudaSuccess && unfed)
+      {
+        UnfedRows u{};
+        std::vector<char> fed(n_in, 0);
+        for (int j = 0; j < ch.host.nj; j++)
+          if (ch.host.joint[j].in >= 0) fed[ch.host.joint[j].in] = 1;
+        for (int i = 0; i < n_in; i++)
+          if (!fed[i]) u.row[u.n++] = i;
+        gram_unfed_tau_sq_kernel<<<1, 256, 0, st>>>(tau_meas, in.ld, in.n, u, ts, tau_sq, accumulate);
+        count_launch();
+        e = cudaGetLastError();
+      }
       if (e != cudaErrorNotSupported) return e;
     }
+    // rdb_chain_gram_kernel_info describes the last Gram call: say that this one ran the general pipeline, and why
+    const int K = ch.gram.fold.nj;
+    ch.gram.kernel_specialised = 2;
+    if (force_v0) ch.gram.kernel_why = "general pipeline: RDB_GRAM_IMPL=v0";
+    else if (K > 7) ch.gram.kernel_why = "general pipeline: more than 7 moving joints (" + std::to_string(K) + ")";
+    else if (K < 1) ch.gram.kernel_why = "general pipeline: no moving joint";
+    else if (P != Pr)
+      ch.gram.kernel_why = "general pipeline: a component set the one-pass kernel refuses (a component on an input no chain joint feeds, "
+                           "or more than 8 component columns on one joint)";
+    else ch.gram.kernel_why = "general pipeline: the fused kernel does not take this chain";
   }
   const int nblk = (P + 1 + BLK - 1) / BLK;
   const int npairs = nblk * (nblk + 1) / 2;

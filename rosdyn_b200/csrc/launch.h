@@ -27,7 +27,9 @@ struct GramWorkspace
   size_t fold_bytes = 0;
   double* ext_dev = nullptr;   // extended model: rigid-body block | cross-tile sums | cross partials | component map
   size_t ext_bytes = 0;
-  // which fused kernel the last Gram call ran (rdb_chain_gram_kernel_info): 1 run-time specialised (gram_jit.cpp), 0 precompiled, -1 none yet
+  double* tau_sq_part = nullptr;  // gram.cu: the fused kernels' tau^T tau when measured torques also sit on inputs no chain joint feeds
+  // which kernel the last Gram call ran (rdb_chain_gram_kernel_info): 1 run-time specialised (gram_jit.cpp), 0 precompiled, 2 general
+  // pipeline (gram.cu), -1 none yet
   int kernel_specialised = -1;
   std::string kernel_why = "no fused Gram call yet";
 };
