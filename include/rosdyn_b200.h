@@ -346,7 +346,7 @@ int32_t rdb_chain_device(const rdb_chain* chain);
  * how long the compile took; for the general pipeline it starts with "general pipeline:". */
 rdb_status rdb_chain_gram_kernel_info(const rdb_chain* chain, int32_t* specialised, char* reason, int32_t reason_len);
 /* Host only, no device needed (inspection tools): the cubin of the run-time specialised kernel of an all-revolute chain, written to `path`.
- * kernel_args: the kernel and its template arguments without the model, e.g. "gram_fused_kernel<6, 4, true, 0, 4"; arch e.g. "sm_100a". */
+ * kernel_args: the kernel and its template arguments without the model, e.g. "gram_fused_kernel<6, 4, true, 0"; arch e.g. "sm_100a". */
 rdb_status rdb_gram_specialised_cubin(const rdb_chain_desc* desc, const char* kernel_args, const char* arch, const char* path, char* reason,
                                       int32_t reason_len);
 rdb_status rdb_regressor_gram_sharded_host(rdb_chain* const* chains, int32_t n_chains, const rdb_samples* in, const double* tau_meas,

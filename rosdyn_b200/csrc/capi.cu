@@ -615,7 +615,7 @@ rdb_status rdb_gram_specialised_cubin(const rdb_chain_desc* desc, const char* ke
   if (!fold_rev_canonical(ch->gram.fold)) return fail(RDB_ERR_INVALID_ARG, "the folded chain is not all-revolute about e_z: no specialised kernel");
   std::vector<char> cubin;
   std::string why;
-  const bool ok = gram_jit_cubin(ch->gram.fold, kernel_args, gram_jit_defines(), arch, cubin, why);
+  const bool ok = gram_jit_cubin(ch->gram.fold, kernel_args, arch, cubin, why);
   if (reason && reason_len > 0) snprintf(reason, (size_t)reason_len, "%s", why.c_str());
   if (!ok) return fail(RDB_ERR_CUDA, "NVRTC: " + why);
   FILE* f = fopen(path, "wb");

@@ -1,6 +1,5 @@
-// gram_common.cuh -- pieces shared by the fused regressor -> normal-equation kernels (gram_fused.cu: shared-memory slots filled directly by the
-// generator warps; gram_ring.cu: generator warps decoupled from the slots through an L2-resident ring and TMA bulk copies): geometry of the
-// augmented Gram matrix, mbarrier / DMMA wrappers, and the per-sample regressor generator.
+// gram_common.cuh -- pieces shared by the fused regressor -> normal-equation kernels (gram_fused.cuh): geometry of the augmented Gram
+// matrix and of a slot, the DMMA wrapper, and the per-sample regressor generator.
 // The header is also compiled at run time by NVRTC (gram_jit.cpp), which has no system headers: it needs chain_dev.h and spatial.cuh only.
 #pragma once
 #ifndef __CUDACC_RTC__
@@ -13,15 +12,10 @@
 namespace rdb
 {
 
-#ifndef GF_TSPLIT
-#define GF_TSPLIT 2
-#endif
-#ifndef GF_ZCOL
-#define GF_ZCOL 1  // all-revolute chains: drop the exact-zero mass column of a link on its own joint (GramGeom Z)
-#endif
-constexpr int GF_KSPLIT = 4;      // MMA warps that share the k-steps of a slot (one per SM sub-partition)
-constexpr int GF_TS = GF_TSPLIT;  // 1: each MMA warp owns all tiles; 2: two warps per sub-partition split the tile rows by parity
-constexpr int GF_MMA_WARPS = GF_KSPLIT * GF_TS;
+constexpr int GF_KSPLIT = 4;                   // MMA warps that share the k-steps of a slot (one per SM sub-partition)
+constexpr int GF_MMA_WARPS = 2 * GF_KSPLIT;    // two per sub-partition: they split the tile rows by parity
+constexpr int GF_GENS = GF_KSPLIT;             // generator warps: one per sub-partition, whatever the number of slots
+constexpr int GF_THREADS = 32 * (GF_MMA_WARPS + GF_GENS);
 constexpr int GF_MAX_SLOTS = 4;   // 32-sample slots in shared memory: as many as fit the 227 KB (3 for a 7-joint chain, 4 from 6 joints down);
                                   // 8 MMA + 4 generator warps = 3 warps per SM sub-partition is also what the 168-register budget allows
 constexpr int GF_BAR_REDUCE = 1;  // named barrier of the final k-split reduction (0 is __syncthreads)
@@ -31,26 +25,7 @@ __device__ __forceinline__ void dmma884f(double& d0, double& d1, double a, doubl
 {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
 }
-// mbarriers in shared memory (one full / one empty per slot); arrive = release.cta, wait = acquire.cta
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* b, int count)
-{
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* b)
-{
-  asm volatile("{\n .reg .b64 st;\n mbarrier.arrive.shared::cta.b64 st, [%0];\n}" ::"r"(smem_u32(b)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* b, uint32_t parity)
-{
-  asm volatile(
-      "{\n .reg .pred p;\n"
-      "W: mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      " @p bra D;\n bra W;\n"
-      "D:\n}" ::"r"(smem_u32(b)),
-      "r"(parity)
-      : "memory");
-}
 
 template <int V>
 struct ic
@@ -70,31 +45,26 @@ __device__ __forceinline__ void static_for(F&& f)
 }
 
 // geometry of the augmented Gram matrix and of a slot for a (folded) chain of NJ joints, all of them inputs.
-// X = 1 (cross mode, extended model [Phi | Phi_c]): every row carries GX_COLS component columns of its own joint after the tau column.
-constexpr int GX_COLS = 8;  // component columns per joint row (one 8-wide tile)
-// Z = 1 (all-revolute chains: gram_ext_kernel, gram_ring.cu): the projection of a link on its OWN revolute joint has no mass term (the unit
+constexpr int GX_COLS = 8;  // component columns per joint row (extended model: one 8-wide cross tile)
+// Z = 1 (all-revolute chains, extended model): the projection of a link on its OWN revolute joint has no mass term (the unit
 // twist at birth is [0; axis], so Phi[j, 10 j + 0] == 0 exactly).  Inside every link block the mass column therefore comes LAST (p order
 // 1..9, 0): the row of joint j then ends with an exact zero that is neither stored nor multiplied -- rowlen(j) = 10 (NJ - j), and position
 // 10 NJ (the mass of the first moving link, an identically zero column of Phi) is never touched.
-// Z = 2 (all-revolute chains: the rigid-body gram_fused_kernel) drops every column that the REV walk (gram_walk_rev) makes an exact zero:
+// Z = 2 (all-revolute chains, rigid-body model) drops every column that the REV walk (gram_walk_rev) makes an exact zero:
 //   * the own-joint projection [0; e_z] has m c_z == 0 as well as m == 0 (gram_walk_rev, branch j == l);
 //   * the first moving link sits on the fixed base: there v = a = 0, w = (0, 0, Dq_0), alpha = (0, 0, DDq_0), so of its own-joint closed
 //     forms only I_zz = alpha_z, m c_x = fm_y and m c_y = -fm_x are not exact zeros (I_xx, I_xy, I_xz, I_yy, I_yz are -w_x w_y,
 //     w_x^2 - w_y^2, fma(-w_y, w_z, alpha_x), w_x w_y, fma(w_x, w_z, alpha_y) with w_x = w_y = alpha_x = alpha_y = 0).  Link 0 appears in
 //     row 0 only, so these seven are identically zero columns of Phi and have no position at all.
 // Inside every link block the order is I_zz, m c_x, m c_y, I_xx .. I_yz, m c_z, m (inblk): the own block of row j >= 1 is the first 8
-// positions of its block, that of row 0 the first 3.  With GF_TAU_TILE == 0 tau is no column of the tiles either: its row sits behind the
-// regressor rows of the slot and the MMA warps accumulate Phi^T tau and tau^T tau by DFMA on the fragments they load for the DMMAs
-// (gram_tau_step): rowlen(0) = 10 (NJ - 1) + 3, rowlen(j >= 1) = 10 (NJ - j) - 2, C6 81 instead of 98 DMMA per 4 samples.  With
-// GF_TAU_TILE == 1 tau stays the tile column at position 0 (C6 90 DMMA per 4 samples).
-#ifndef GF_TAU_TILE
-#define GF_TAU_TILE 0
-#endif
-template <int NJ, int X = 0, int Z = 0>
+// positions of its block, that of row 0 the first 3.  tau is no column of the tiles either (TC == 0): its row sits behind the regressor rows
+// of the slot and the MMA warps accumulate Phi^T tau and tau^T tau by DFMA on the fragments they load for the DMMAs (gram_tau_step):
+// rowlen(0) = 10 (NJ - 1) + 3, rowlen(j >= 1) = 10 (NJ - j) - 2, C6 81 instead of 98 DMMA per 4 samples (90 with tau as tile column 0).
+template <int NJ, int Z = 0>
 struct GramGeom
 {
   static constexpr int P = 10 * NJ;
-  static constexpr int TC = Z == 2 && !GF_TAU_TILE ? 0 : 1;  // tau positions in front of the link blocks (position 0 when TC == 1)
+  static constexpr int TC = Z == 2 ? 0 : 1;  // tau positions in front of the link blocks (position 0 when TC == 1)
   // place of parameter p (m, m c_xyz, I_xx, I_xy, I_xz, I_yy, I_yz, I_zz) inside its link block, and back
   __host__ __device__ static constexpr int inblk(int p)
   {
@@ -133,46 +103,45 @@ struct GramGeom
   static constexpr int PARTIAL = NT * 64 + (TC ? 0 : 8 * T + 1);
   static constexpr int KPW = 8 / GF_KSPLIT;   // k-steps (4 samples) of one MMA warp per joint row and slot
   static constexpr int NSTEPS = NJ * KPW;     // k-steps of one MMA warp per slot
-  __host__ __device__ static constexpr int threads(int slots) { return 32 * (GF_MMA_WARPS + slots); }
   // offset (doubles) of the row of joint j inside a slot: [position][sample], only the positions 0 .. rowlen(j)-1 are stored
   __host__ __device__ static constexpr int rowbase(int j)
   {
     int o = 0;
-    for (int i = 0; i < j; i++) o += (rowlen(i) + (X ? GX_COLS : 0)) * 32;
+    for (int i = 0; i < j; i++) o += rowlen(i) * 32;
     return o;
   }
   // offset of the tau row of joint j: position 0 of its row, or (TC == 0) behind all rows, [joint][sample]
   __host__ __device__ static constexpr int taubase(int j) { return TC ? rowbase(j) : rowbase(NJ) + 32 * j; }
   static constexpr int SLOT_DOUBLES = rowbase(NJ) + (TC ? 0 : 32 * NJ);
   __host__ __device__ static constexpr int tile(int I, int J) { return I * T - I * (I - 1) / 2 + (J - I); }
-  // tile rows owned by an MMA warp: all (TS == 1) or the rows of parity `par` (TS == 2)
-  __host__ __device__ static constexpr bool owns(int I, int ts, int par) { return ts == 1 || (I & 1) == par; }
-  __host__ __device__ static constexpr int ntiles(int ts, int par)  // at least 1: a warp may own no tile row (T == 1), arrays need a size
+  // tile rows owned by an MMA warp: the rows of parity `par`
+  __host__ __device__ static constexpr bool owns(int I, int par) { return (I & 1) == par; }
+  __host__ __device__ static constexpr int ntiles(int par)  // at least 1: a warp may own no tile row (T == 1), arrays need a size
   {
     int n = 0;
     for (int I = 0; I < T; I++)
-      if (owns(I, ts, par)) n += T - I;
+      if (owns(I, par)) n += T - I;
     return n > 0 ? n : 1;
   }
-  __host__ __device__ static constexpr int local(int I, int J, int ts, int par)
+  __host__ __device__ static constexpr int local(int I, int J, int par)
   {
     int n = 0;
     for (int K = 0; K < I; K++)
-      if (owns(K, ts, par)) n += T - K;
+      if (owns(K, par)) n += T - K;
     return n + (J - I);
   }
   // TC == 0: DFMA accumulators of an MMA warp -- b at position 8 I + g for each tile row I it owns (lane (g, t): the samples t mod 4), then
   // in the par 0 warps tau^T tau; bown(I): the accumulator of tile row I
-  __host__ __device__ static constexpr int bown(int I, int ts, int par)
+  __host__ __device__ static constexpr int bown(int I, int par)
   {
     int n = 0;
     for (int K = 0; K < I; K++)
-      if (owns(K, ts, par)) n++;
+      if (owns(K, par)) n++;
     return n;
   }
-  __host__ __device__ static constexpr int nbacc(int ts, int par) { return TC || (par != 0 && bown(T, ts, par) == 0) ? 1 : bown(T, ts, par) + (par == 0 ? 1 : 0); }
+  __host__ __device__ static constexpr int nbacc(int par) { return TC || (par != 0 && bown(T, par) == 0) ? 1 : bown(T, par) + (par == 0 ? 1 : 0); }
   __host__ __device__ static constexpr int tj(int j) { return (rowlen(j) + 7) / 8; }
-  // cross mode: per joint row j the tiles (regular tile I, component tile of joint j), I = 0 .. tj(j)-1, then (component, component)
+  // extended model: per joint row j the cross tiles (regular tile I, component tile of joint j), I = 0 .. tj(j)-1, then (component, component)
   __host__ __device__ static constexpr int xtile(int j, int I)  // I == tj(j): the (component, component) tile
   {
     int n = 0;
@@ -186,29 +155,29 @@ struct GramGeom
     return n;
   }
   static constexpr int NXT = nxt();
-  __host__ __device__ static constexpr bool xowns(int j, int I, int ts, int par) { return ts == 1 || ((I == tj(j) ? j : I) & 1) == par; }
-  __host__ __device__ static constexpr int xlocal(int j, int I, int ts, int par)
+  __host__ __device__ static constexpr bool xowns(int j, int I, int par) { return ((I == tj(j) ? j : I) & 1) == par; }
+  __host__ __device__ static constexpr int xlocal(int j, int I, int par)
   {
     int n = 0;
     for (int k = 0; k <= j; k++)
       for (int K = 0; K <= tj(k); K++)
       {
         if (k == j && K == I) return n;
-        if (xowns(k, K, ts, par)) n++;
+        if (xowns(k, K, par)) n++;
       }
     return n;
   }
-  __host__ __device__ static constexpr int nxtiles(int ts, int par)
+  __host__ __device__ static constexpr int nxtiles(int par)
   {
     int n = 0;
     for (int k = 0; k < NJ; k++)
       for (int K = 0; K <= tj(k); K++)
-        if (xowns(k, K, ts, par)) n++;
+        if (xowns(k, K, par)) n++;
     return n;
   }
 };
 
-// components of the joints of the folded chain (cross mode): the columns they contribute to the row of their joint, one entry per column
+// components of the joints of the folded chain (extended model): the columns they contribute to the row of their joint, one entry per column
 enum : int
 {
   GXK_SAT = 1,    // FirstOrderPolynomialFriction column 0: clamp(omega / thr, -1, 1)           (friction_polynomial1.h:47-50)
@@ -395,72 +364,14 @@ __device__ __forceinline__ void gen_load(const ChainDev<NJ>& C, const SamplesDev
   }
 }
 
-// Component columns of every joint row (element-wise in q_j, Dq_j; zero padded to one tile), written after the walk by ONE rolled loop over
-// (joint, column): no call (a called function costs the walker its registers through the ABI -- it spilled 280 bytes per thread into an L1
-// that the slots leave at ~20 KB), little code, and the walk stays one basic block.
-template <int NJ>
-__device__ __forceinline__ void gram_component_columns(const ChainDev<NJ>& C, const GramComps& comps, const SamplesDev& in, int64_t i,
-                                                       double* __restrict__ slot, int lane)
-{
-  using G = GramGeom<NJ, 1>;
-  // q_j / Dq_j are read again (L2 hits; keeping them in registers through the walk spills), ALL joints at once so that the loads overlap;
-  // joint loop unrolled, column loop rolled: little code, no call
-  double qv[NJ], dqv[NJ];
-#pragma unroll
-  for (int j = 0; j < NJ; j++)
-  {
-    qv[j] = ld_in(in.q, C.joint[j].in, in.ld, i);
-    dqv[j] = ld_in(in.dq, C.joint[j].in, in.ld, i);
-  }
-  static_for<0, NJ>([&](auto jc) {
-    constexpr int j = decltype(jc)::value;
-    const double q = qv[j], dq = dqv[j];
-    const int nc = comps.ncols[j];
-    double* o = slot + G::rowbase(j) + G::rowlen(j) * 32;
-#pragma unroll 1
-    for (int c = 0; c < GX_COLS; c++)
-    {
-      double val = 0.0;
-      if (c < nc)
-      {
-        const int kd = comps.kind[j][c];
-        const double th = comps.thr[j][c], vm = comps.vmax[j][c];
-        const double omega = fmin(fmax(dq, -vm), vm);
-        if (kd == GXK_OMEGA) val = omega;
-        else if (kd == GXK_Q) val = q;
-        else if (kd == GXK_ONE) val = 1.0;
-        else
-        {
-          const double r = omega * comps.ithr[j][c];
-          if (kd == GXK_SAT) val = fmin(fmax(r, -1.0), 1.0);
-          else
-          {
-            const double sg = omega == 0.0 ? 0.0 : (omega > th ? 1.0 : (omega < -th ? -1.0 : r));
-            val = kd == GXK_SGN ? sg : omega * omega * sg;
-          }
-        }
-      }
-      o[c * 32 + (lane ^ (4 * (c & 3)))] = val;
-    }
-  });
-}
-
-// GLOBAL: the rows go to an L2-resident ring entry in global memory (st.global.cg: no L1 allocation) instead of a shared-memory slot
-template <bool GLOBAL>
-__device__ __forceinline__ void st_row(double* p, double v)
-{
-  if (GLOBAL) __stcg(p, v);
-  else *p = v;
-}
-
 // the projection Phi[j, block of link L] = e of joint j's unit twist (u, s) moved to link L: tau_j += e . pi_L in two independent chains,
 // e stored into the row of joint j.  OWN: the projection of a revolute link on its own joint (e[0] == e[3] == 0, typed Zr, not multiplied).
-template <class M, int NJ, int X, int Z, bool GLOBAL, int L, int J, bool OWN, class E0, class E1, class E2, class E3, class E4, class E5, class E6,
+template <class M, int NJ, int Z, int L, int J, bool OWN, class E0, class E1, class E2, class E3, class E4, class E5, class E6,
           class E7, class E8, class E9>
 __device__ __forceinline__ void gram_emit(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, E0 e0, E1 e1, E2 e2, E3 e3,
                                           E4 e4, E5 e5, E6 e6, E7 e7, E8 e8, E9 e9)
 {
-  using G = GramGeom<NJ, X, Z>;
+  using G = GramGeom<NJ, Z>;
   auto P = [&](auto pc) { return kc<M, MK_PI, L, decltype(pc)::value>(C); };
   auto t0a = [&] {  // joint L's torque starts here: from +0.0 as the precompiled kernel always did, from nothing with a compile-time model
     if constexpr (J == L && M::RUNTIME) return 0.0;
@@ -475,15 +386,15 @@ __device__ __forceinline__ void gram_emit(const ChainDev<NJ>& C, double (&tau)[N
 #pragma unroll
   for (int p = 0; p < 10; p++)
     if (G::stored(J, L, p))  // the exact zeros the layout drops are not stored
-      st_row<GLOBAL>(o + G::pos(L, p) * 32 + (lane ^ (4 * (G::pos(L, p) & 3))), e[p]);
+      o[G::pos(L, p) * 32 + (lane ^ (4 * (G::pos(L, p) & 3)))] = e[p];
 }
-template <class M, int NJ, int X, int Z, bool GLOBAL, int L, int J, class U, class S>
+template <class M, int NJ, int Z, int L, int J, class U, class S>
 __device__ __forceinline__ void gram_project(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, const U& u, const S& s,
                                              const V3& fm, const V3& w, const V3& al)
 {
   const auto h = tcross_add(tcross_add(tcross(u, al), w, tcross(w, u)), fm, s);
   const auto rho = tcross(s, w);
-  gram_emit<M, NJ, X, Z, GLOBAL, L, J, false>(
+  gram_emit<M, NJ, Z, L, J, false>(
       C, tau, slot, lane, tdot(u, fm), h.x, h.y, h.z, tfma(s.x, al.x, tmul(rho.x, w.x)),
       tfma(s.x, al.y, tfma(s.y, al.x, tfma(rho.x, w.y, tmul(rho.y, w.x)))), tfma(s.x, al.z, tfma(s.z, al.x, tfma(rho.x, w.z, tmul(rho.z, w.x)))),
       tfma(s.y, al.y, tmul(rho.y, w.y)), tfma(s.y, al.z, tfma(s.z, al.y, tfma(rho.y, w.z, tmul(rho.z, w.y)))), tfma(s.z, al.z, tmul(rho.z, w.z)));
@@ -494,17 +405,15 @@ __device__ __forceinline__ void gram_project(const ChainDev<NJ>& C, double (&tau
 // joint type and the axis are then compile-time facts: R = A' Rz(q) mixes two columns of A', the rates gain their e_z terms directly, the
 // first transport of a joint's unit twist [0; e_z] is a row of R, and the projection of a link on its own joint has closed forms with two
 // exact zeros (the mass and m c_z columns).  M: where the model constants come from (RtModel, or a run-time generated model type).
-template <int NJ, class M, int X, int Z, bool GLOBAL, bool LAZY>
-__device__ __forceinline__ void gram_walk_rev(const ChainDev<NJ>& C, const GenIn<NJ>& x, const SamplesDev& in, double* __restrict__ slot, int64_t i,
-                                              int lane, double (&tau)[NJ])
+template <int NJ, class M, int Z>
+__device__ __forceinline__ void gram_walk_rev(const ChainDev<NJ>& C, const GenIn<NJ>& x, double* __restrict__ slot, int lane, double (&tau)[NJ])
 {
   static_assert(REV_AXIS[0] == 0.0 && REV_AXIS[1] == 0.0 && REV_AXIS[2] == 1.0, "the REV walk below is written for the axis s = e_z");
   V3 U[NJ], S[NJ];
   V3 v = v3(0, 0, 0), w = v3(0, 0, 0), a = v3(0, 0, 0), al = v3(0, 0, 0), g;
   static_for<0, NJ>([&](auto lc) {
     constexpr int l = decltype(lc)::value;
-    const JointDev& J = C.joint[l];
-    const double dql = LAZY ? ld_in(in.dq, J.in, in.ld, i) : x.dq[l], ddql = LAZY ? ld_in(in.ddq, J.in, in.ld, i) : x.ddq[l];
+    const double dql = x.dq[l], ddql = x.ddq[l];
     const double sl = x.sv[l], cl = x.cv[l];
     const auto t = mk3(kc<M, MK_T, l, 0>(C), kc<M, MK_T, l, 1>(C), kc<M, MK_T, l, 2>(C));
     // R = A' Rz(q), row k: (fma(s, A'[k][1], c A'[k][0]), fma(-s, A'[k][0], c A'[k][1]), A'[k][2])
@@ -547,21 +456,20 @@ __device__ __forceinline__ void gram_walk_rev(const ChainDev<NJ>& C, const GenIn
       if constexpr (j == l)  // unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
       {
         const double e7 = w.x * w.y;
-        gram_emit<M, NJ, X, Z, GLOBAL, l, j, true>(C, tau, slot, lane, Zr{}, fm.y, -fm.x, Zr{}, -e7, fma(w.x, w.x, -(w.y * w.y)),
-                                                   fma(-w.y, w.z, al.x), e7, fma(w.x, w.z, al.y), al.z);
+        gram_emit<M, NJ, Z, l, j, true>(C, tau, slot, lane, Zr{}, fm.y, -fm.x, Zr{}, -e7, fma(w.x, w.x, -(w.y * w.y)), fma(-w.y, w.z, al.x),
+                                        e7, fma(w.x, w.z, al.y), al.z);
       }
-      else if constexpr (j == l - 1) gram_project<M, NJ, X, Z, GLOBAL, l, j>(C, tau, slot, lane, U1, S1, fm, w, al);
-      else gram_project<M, NJ, X, Z, GLOBAL, l, j>(C, tau, slot, lane, U[j], S[j], fm, w, al);
+      else if constexpr (j == l - 1) gram_project<M, NJ, Z, l, j>(C, tau, slot, lane, U1, S1, fm, w, al);
+      else gram_project<M, NJ, Z, l, j>(C, tau, slot, lane, U[j], S[j], fm, w, al);
     });
   });
 }
 
 // any joint types and axes (the constant-bank model)
-template <int NJ, int X, int Z, bool GLOBAL, bool LAZY>
-__device__ __forceinline__ void gram_walk_gen(const ChainDev<NJ>& C, const GenIn<NJ>& x, const SamplesDev& in, double* __restrict__ slot, int64_t i,
-                                              int lane, double (&tau)[NJ])
+template <int NJ, int Z>
+__device__ __forceinline__ void gram_walk_gen(const ChainDev<NJ>& C, const GenIn<NJ>& x, double* __restrict__ slot, int lane, double (&tau)[NJ])
 {
-  using G = GramGeom<NJ, X, Z>;
+  using G = GramGeom<NJ, Z>;
   V3 U[NJ], S[NJ];
   V3 v = v3(0, 0, 0), w = v3(0, 0, 0), a = v3(0, 0, 0), al = v3(0, 0, 0);
   V3 g = v3(C.g);
@@ -569,7 +477,7 @@ __device__ __forceinline__ void gram_walk_gen(const ChainDev<NJ>& C, const GenIn
   for (int l = 0; l < NJ; l++)
   {
     const JointDev& J = C.joint[l];
-    const double dql = LAZY ? ld_in(in.dq, J.in, in.ld, i) : x.dq[l], ddql = LAZY ? ld_in(in.ddq, J.in, in.ld, i) : x.ddq[l];
+    const double dql = x.dq[l], ddql = x.ddq[l];
     double R[9];
     const V3 t = J.type != RDB_JOINT_PRISMATIC ? v3(J.t) : axpy(v3(J.t), v3(J.axp), x.q[l]);
     if (J.type == RDB_JOINT_REVOLUTE)
@@ -634,43 +542,38 @@ __device__ __forceinline__ void gram_walk_gen(const ChainDev<NJ>& C, const GenIn
       tau[j] = t0 + t1;
       double* o = slot + G::rowbase(j);
 #pragma unroll
-      for (int p = 0; p < 10; p++) st_row<GLOBAL>(o + G::pos(l, p) * 32 + (lane ^ (4 * (G::pos(l, p) & 3))), e[p]);
+      for (int p = 0; p < 10; p++) o[G::pos(l, p) * 32 + (lane ^ (4 * (G::pos(l, p) & 3)))] = e[p];
     }
   }
 }
 
-// LAZY: Dq / DDq of a link are loaded inside the walk (the compiler hoists them as far as registers allow) instead of being held in registers
-// from before the wait for the output buffer: with two generator warps per sub-partition the latency hides behind the other warp
-template <int NJ, bool REV, int X, int Z = 0, bool GLOBAL = false, bool LAZY = false, class M = RtModel>
-__device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GramComps* comps, const GenIn<NJ>& x, const SamplesDev& in,
-                                              const double* __restrict__ tau_meas, double* __restrict__ slot, int64_t i, int lane)
+template <int NJ, bool REV, int Z, class M>
+__device__ __forceinline__ void gram_generate(const ChainDev<NJ>& C, const GenIn<NJ>& x, const SamplesDev& in, const double* __restrict__ tau_meas,
+                                              double* __restrict__ slot, int64_t i, int lane)
 {
   static_assert(!Z || REV, "the zero mass column of a link on its own joint exists for revolute joints only");
   static_assert(REV || M::RUNTIME, "compile-time models are built for the REV walk");
-  using G = GramGeom<NJ, X, Z>;
+  using G = GramGeom<NJ, Z>;
   double tau[NJ];
-  if constexpr (REV) gram_walk_rev<NJ, M, X, Z, GLOBAL, LAZY>(C, x, in, slot, i, lane, tau);
-  else gram_walk_gen<NJ, X, Z, GLOBAL, LAZY>(C, x, in, slot, i, lane, tau);
+  if constexpr (REV) gram_walk_rev<NJ, M, Z>(C, x, slot, lane, tau);
+  else gram_walk_gen<NJ, Z>(C, x, slot, lane, tau);
 #pragma unroll
   for (int j = 0; j < NJ; j++)
   {
     const double tv = tau_meas ? __ldcs(tau_meas + (int64_t)C.joint[j].in * in.ld + i) : tau[j];
-    st_row<GLOBAL>(slot + G::taubase(j) + lane, tv);
+    slot[G::taubase(j) + lane] = tv;
   }
-  if (X) gram_component_columns<NJ>(C, *comps, in, i, slot, lane);
 }
 
 // lanes past the end of the batch (last group only): their rows become exact zeros
-template <int NJ, int X, int Z = 0, bool GLOBAL = false>
+template <int NJ, int Z>
 __device__ __noinline__ void gram_zero_lane(double* __restrict__ slot, int lane)
 {
-  using G = GramGeom<NJ, X, Z>;
+  using G = GramGeom<NJ, Z>;
   for (int j = 0; j < NJ; j++)
   {
-    for (int c = 0; c < G::rowlen(j); c++) st_row<GLOBAL>(slot + G::rowbase(j) + c * 32 + (lane ^ (4 * (c & 3))), 0.0);
-    if (!G::TC) st_row<GLOBAL>(slot + G::taubase(j) + lane, 0.0);
-    if (X)
-      for (int c = 0; c < GX_COLS; c++) st_row<GLOBAL>(slot + G::rowbase(j) + (G::rowlen(j) + c) * 32 + (lane ^ (4 * (c & 3))), 0.0);
+    for (int c = 0; c < G::rowlen(j); c++) slot[G::rowbase(j) + c * 32 + (lane ^ (4 * (c & 3)))] = 0.0;
+    if (!G::TC) slot[G::taubase(j) + lane] = 0.0;
   }
 }
 

@@ -14,14 +14,14 @@
 namespace rdb
 {
 
-// fixed-order sum of the per-CTA partials (GramGeom<NJ, 0, Z>::PARTIAL doubles each, pstride apart) -> gram (full symmetric,
+// fixed-order sum of the per-CTA partials (GramGeom<NJ, Z>::PARTIAL doubles each, pstride apart) -> gram (full symmetric,
 // column-major), rhs, tau_sq.  One thread per partial entry, and per entry of the P x (P + 1) output: the parameter columns without a position
 // (identically zero columns of Phi, GramGeom::has_pos) get exact zeros in their row, column and rhs.
 template <int NJ, int Z>
 __global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int nparts, int pstride, double* __restrict__ gram,
                                          double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
 {
-  using G = GramGeom<NJ, 0, Z>;
+  using G = GramGeom<NJ, Z>;
   constexpr int P = G::P;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (!accumulate && e < P * (P + 1))
@@ -83,7 +83,7 @@ template <int NJ, int Z>
 static void launch_fused_reduce(const double* partial, int nparts, int pstride, double* gram, double* rhs, double* tau_sq, int accumulate,
                                 cudaStream_t st)
 {
-  using G = GramGeom<NJ, 0, Z>;
+  using G = GramGeom<NJ, Z>;
   const int n = std::max(G::PARTIAL, G::P * (G::P + 1));
   gram_fused_reduce_kernel<NJ, Z><<<(n + 255) / 256, 256, 0, st>>>(partial, nparts, pstride, gram, rhs, tau_sq, accumulate);
   count_launch();
@@ -149,32 +149,6 @@ cudaError_t launch_fold_expand(ChainHost& ch, double* gram, double* rhs, double*
   return cudaGetLastError();
 }
 
-// the overridable geometry macros of gram_common.cuh / gram_fused.cuh as this launcher was compiled with them: the run-time compiled kernel
-// must lay out the slots, tiles and partials exactly as the launcher sizes them
-std::string gram_jit_defines()
-{
-  char b[160];
-  snprintf(b, sizeof b, "#define GF_TSPLIT %d\n#define GF_ZCOL %d\n#define GF_TAU_TILE %d\n#define GF_SPIN_NS %d\n", (int)GF_TSPLIT, (int)GF_ZCOL,
-           (int)GF_TAU_TILE, (int)GF_SPIN_NS);
-  return b;
-}
-
-// REV chains: the kernel specialised at run time to the chain's constants when it can be built (gram_jit.cpp), else nullptr: the precompiled
-// instantiation runs.  Other chains always run the precompiled generic kernel.
-template <bool REV, class... A>
-static const void* gram_kernel_for(ChainHost& ch, const char* fmt, A... a)
-{
-  if (!REV)
-  {
-    ch.gram.kernel_specialised = 0;
-    ch.gram.kernel_why = "precompiled kernel: not every folded joint is revolute about e_z (generic generator)";
-    return nullptr;
-  }
-  char args[96];
-  snprintf(args, sizeof args, fmt, a...);
-  return gram_jit_kernel(ch, args, gram_jit_defines());
-}
-
 template <int NJ>
 static ChainDev<NJ> narrow_g(const ChainDev<RDB_MAX_JOINTS>& h)
 {
@@ -201,50 +175,66 @@ static cudaError_t grow(double*& p, size_t& have, size_t need)
   return e;
 }
 
-// generator warps of the rigid-body kernel: one per SM sub-partition even when fewer slots fit (GF_GENS4 = 0: one per slot, as before)
-#ifndef GF_GENS4
-#define GF_GENS4 1
-#endif
-template <int SLOTS>
-constexpr int gf_gens()
+// slots that fit the shared memory of an SM (227 KB minus 1 KB of barriers / static data): the rows, and XC component columns per joint
+template <int NJ, int Z, int XC>
+constexpr int gf_slots()
 {
-  return (GF_GENS4 && GF_TS == 2 && SLOTS < 4) ? 4 : SLOTS;
+  return std::min<int>(GF_MAX_SLOTS,
+                       (int)((227 * 1024 - 1024) / (sizeof(double) * (GramGeom<NJ, Z>::SLOT_DOUBLES + gram_ext_side_doubles<NJ, XC>()))));
 }
 
-template <int NJ, int SLOTS, bool REV>
+// gram_fused_kernel on the folded chain, one per-CTA partial (gram_partial_doubles) each into `partials`: *grid CTAs.  On REV chains the
+// kernel is the one specialised at run time to the chain's constants when it can be built (gram_jit.cpp), else the precompiled
+// instantiation; other chains always run the precompiled generic kernel.
+template <int NJ, bool REV, int XC>
+static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const SamplesDev& in, const double* tau_meas, double* partials,
+                                       int* grid, cudaStream_t st)
+{
+  constexpr int Z = REV ? (XC ? 1 : 2) : 0;  // as in the kernel
+  constexpr int SLOTS = gf_slots<NJ, Z, XC>();
+  static_assert(SLOTS >= 2, "the fused kernel needs two slots");
+  const void* kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, XC>);
+  if (REV)
+  {
+    char args[64];
+    snprintf(args, sizeof args, "gram_fused_kernel<%d, %d, true, %d", NJ, SLOTS, XC);
+    if (const void* jk = gram_jit_kernel(ch, args)) kfn = jk;
+  }
+  else
+  {
+    ch.gram.kernel_specialised = 0;
+    ch.gram.kernel_why = "precompiled kernel: not every folded joint is revolute about e_z (generic generator)";
+  }
+  const size_t smem = sizeof(double) * (size_t)gram_smem_doubles<NJ, Z, SLOTS, XC>();
+  cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  const int64_t ngroups = (in.n + 31) / 32;
+  constexpr int B = gram_group_block<SLOTS, XC>();
+  *grid = (int)std::min<int64_t>(ch.sm_count, (ngroups + B - 1) / B);
+  ChainDev<NJ> C = narrow_g<NJ>(ch.gram.fold);
+  GramComps comps = gc;
+  SamplesDev ins = in;
+  const double* tm = tau_meas;
+  double* part = partials;
+  int dbg = gram_dev_switch();
+  void* args[] = {&C, &comps, &ins, &tm, &part, &dbg};
+  e = cudaLaunchKernel(kfn, dim3(*grid), dim3(GF_THREADS), args, smem, st);
+  if (e != cudaSuccess) return e;
+  count_launch();
+  return cudaSuccess;
+}
+
+template <int NJ, bool REV>
 static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                                    int accumulate, cudaStream_t st)
 {
-  constexpr int GENS = gf_gens<SLOTS>();
-  constexpr int Z = GF_ZCOL && REV ? 2 : 0;  // as in the kernel
-  using G = GramGeom<NJ, 0, Z>;
-  const size_t smem = sizeof(double) * (size_t)std::max(G::SLOT_DOUBLES * SLOTS, G::PARTIAL);
-  const void* kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, 0, GENS>);
-  {
-    const void* jk = gram_kernel_for<REV>(ch, "gram_fused_kernel<%d, %d, true, 0, %d", NJ, SLOTS, GENS);
-    if (jk) kfn = jk;
-    cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-  }
-  const int dbg = gram_dev_switch();
-  const int64_t ngroups = (in.n + 31) / 32;
-  const int grid = (int)std::min<int64_t>(ch.sm_count, GENS != SLOTS ? ngroups : (ngroups + SLOTS - 1) / SLOTS);
-  {
-    cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL);
-    if (e != cudaSuccess) return e;
-  }
-  {
-    ChainDev<NJ> C = narrow_g<NJ>(ch.gram.fold);
-    GramComps comps{};
-    SamplesDev ins = in;
-    const double* tm = tau_meas;
-    double* part = ch.gram.fused_partials;
-    int dbgv = dbg;
-    void* args[] = {&C, &comps, &ins, &tm, &part, &dbgv};
-    cudaError_t e = cudaLaunchKernel(kfn, dim3(grid), dim3(G::threads(GENS)), args, smem, st);
-    if (e != cudaSuccess) return e;
-  }
-  count_launch();
+  constexpr int Z = REV ? 2 : 0;  // as in the kernel
+  using G = GramGeom<NJ, Z>;
+  cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL);
+  if (e != cudaSuccess) return e;
+  int grid = 0;
+  e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, ch.gram.fused_partials, &grid, st);
+  if (e != cudaSuccess) return e;
   if (ch.gram.fold_identity)
   {
     launch_fused_reduce<NJ, Z>(ch.gram.fused_partials, grid, G::PARTIAL, gram, rhs, tau_sq, accumulate, st);
@@ -260,13 +250,6 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
   return launch_fold_expand(ch, gram, rhs, tau_sq, accumulate, st);
 }
 
-// slots that fit the shared memory of an SM (227 KB minus 1 KB of barriers / static data)
-template <int NJ, int X = 0>
-constexpr int gf_slots()
-{
-  return std::min<int>(GF_MAX_SLOTS, (int)((227 * 1024 - 1024) / (sizeof(double) * GramGeom<NJ, X>::SLOT_DOUBLES)));
-}
-
 // returns cudaErrorNotSupported when the chain does not fit the fused kernel (caller falls back to the general pipeline)
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                               int accumulate, cudaStream_t st)
@@ -275,10 +258,10 @@ cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double*
   const bool rev = fold_rev_canonical(ch.gram.fold);  // all moving joints revolute about e_z: the specialised generator
   switch (ch.gram.fold.nj)  // moving joints; every joint of the folded chain is an input
   {
-#define X(N)                                                                                                    \
-  case N:                                                                                                       \
-    return rev ? launch_fused_nj<N, gf_slots<N>(), true>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st)  \
-               : launch_fused_nj<N, gf_slots<N>(), false>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
+#define X(N)                                                                                  \
+  case N:                                                                                     \
+    return rev ? launch_fused_nj<N, true>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st) \
+               : launch_fused_nj<N, false>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
     X(1) X(2) X(3) X(4) X(5) X(6) X(7)
 #undef X
   }
@@ -313,29 +296,27 @@ __global__ void gram_ext_scatter_kernel(const double* __restrict__ G, const doub
   gram[(size_t)c * Pt + a] = accumulate ? gram[(size_t)c * Pt + a] + v : v;
 }
 
-// cross blocks of the extended normal equations from the reduced cross tiles:
+// cross blocks of the extended normal equations from the reduced cross tiles X of the folded chain (NJ joints, layout GramGeom<NJ, Z>):
 //   gram[a][P + cc] (and its mirror) = sum_c T[la][c][pa] X(10 ka + c ; joint, slot of cc)     a < P   (fold expansion of the rigid column)
 //   rhs[P + cc] = X(P' ; joint, slot)                                                          (tau column of the last regular tile)
 //   gram[P + c2][P + cc] = XX(joint)[slot2][slot] when both components act on the same joint, else 0
 // xj / xs: reduced joint and slot of every component column.  One thread per (a in 0 .. P + Pc, cc).
+template <int NJ, int Z>
 __global__ void gram_cross_finish_kernel(const double* __restrict__ X, const double* __restrict__ Tm, const int32_t* __restrict__ kof,
-                                         const int32_t* __restrict__ xj, const int32_t* __restrict__ xs, int nj, int njr, int Pc,
-                                         double* __restrict__ gram, double* __restrict__ rhs, int accumulate, int zcol)
+                                         const int32_t* __restrict__ xj, const int32_t* __restrict__ xs, int nj, int Pc, double* __restrict__ gram,
+                                         double* __restrict__ rhs, int accumulate)
 {
-  const int P = 10 * nj, Pr = 10 * njr, Pt = P + Pc;
+  using G = GramGeom<NJ, Z>;
+  static_assert(G::TC == 1, "tau is the tile column at position 0");
+  const int P = 10 * nj, Pt = P + Pc;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= (P + 1 + Pc) * Pc) return;
   const int a = e / Pc, cc = e % Pc;
   const int j = xj[cc], g = xs[cc];
-  auto tjf = [&](int k) { return (1 + 10 * (njr - k) - zcol + 7) / 8; };  // GramGeom::tj
-  int tb = 0;  // first cross tile of joint j
-  for (int k = 0; k < j; k++) tb += tjf(k) + 1;
-  const int tjj = tjf(j);
-  auto xval = [&](int col) -> double {  // reduced regular column `col` (Pr = tau) against (j, g)
-    const int p = col % 10;
-    const int pos = col == Pr ? 0 : 1 + 10 * (njr - 1 - col / 10) + (zcol ? (p == 0 ? 9 : p - 1) : p);  // GramGeom::pos
-    const int I = pos >> 3;
-    return (pos >= 1 + 10 * (njr - j) - zcol) ? 0.0 : X[(size_t)(tb + I) * 64 + (pos & 7) * 8 + g];  // behind rowlen(j): an exact zero of Phi
+  const int tb = G::xtile(j, 0);  // first cross tile of joint j
+  auto xval = [&](int col) -> double {  // reduced regular column `col` (G::P = tau) against (j, g)
+    const int pos = col == G::P ? 0 : G::pos(col / 10, col % 10);
+    return pos >= G::rowlen(j) ? 0.0 : X[(size_t)(tb + (pos >> 3)) * 64 + (pos & 7) * 8 + g];  // behind rowlen(j): an exact zero of Phi
   };
   if (a < P)
   {
@@ -355,71 +336,65 @@ __global__ void gram_cross_finish_kernel(const double* __restrict__ X, const dou
   }
   else if (a == P)
   {
-    const double s = xval(Pr);
+    const double s = xval(G::P);
     rhs[P + cc] = accumulate ? rhs[P + cc] + s : s;
   }
   else
   {
     const int c2 = a - P - 1;
-    const double s = (xj[c2] == j) ? X[(size_t)(tb + tjj) * 64 + xs[c2] * 8 + g] : 0.0;
+    const double s = (xj[c2] == j) ? X[(size_t)(tb + G::tj(j)) * 64 + xs[c2] * 8 + g] : 0.0;
     double* o = gram + (size_t)(P + cc) * Pt + P + c2;
     *o = accumulate ? *o + s : s;
   }
 }
 
-// slots of the extended-model kernel: rigid-body rows + XC component columns per joint
-template <int NJ, int Z, int XC>
-constexpr int gf_slots_ext()
-{
-  return std::min<int>(GF_MAX_SLOTS, (int)((227 * 1024 - 256) / (sizeof(double) * (GramGeom<NJ, 0, Z>::SLOT_DOUBLES + gram_ext_side_doubles<NJ, XC>()))));
-}
-// single pass (gram_ext_kernel): rigid-body tiles -> Gt | bt | tst (full parameter vector), cross tiles -> xsum
+// one pass of gram_fused_kernel<.., XC> over the samples: rigid-body tiles -> Gt | bt | tst (full parameter vector) -> the rigid block of the
+// extended normal equations; cross tiles -> xsum -> the cross blocks.  xmap: reduced joint, then slot, of every component column.
 template <int NJ, bool REV, int XC>
-static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const SamplesDev& in, const double* tau_meas, double* Gt, double* bt, double* tst,
-                                 double* xpart, double* xsum, cudaStream_t st)
+static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::vector<int32_t>& xmap, const SamplesDev& in, const double* tau_meas,
+                                 double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
 {
-  constexpr int Z = GF_ZCOL && REV ? 1 : 0;  // as in the kernel
-  using G0 = GramGeom<NJ, 0, Z>;
-  using GX = GramGeom<NJ, 1, Z>;
-  constexpr int SLOTS = gf_slots_ext<NJ, Z, XC>();
-  static_assert(SLOTS >= 2, "the extended-model kernel needs two slots");
-  constexpr int GENS = GF_TS == 2 ? 4 : SLOTS;  // 8 MMA + 4 generator warps (one per SM sub-partition) whatever the number of slots
-  constexpr int PSTRIDE = (G0::NT + GX::NXT) * 64;
-  const size_t smem = sizeof(double) * ((size_t)std::max(G0::SLOT_DOUBLES * SLOTS, PSTRIDE) + (size_t)SLOTS * gram_ext_side_doubles<NJ, XC>());
-  const void* kfn = reinterpret_cast<const void*>(gram_ext_kernel<NJ, SLOTS, GENS, REV, XC>);
-  if (const void* jk = gram_kernel_for<REV>(ch, "gram_ext_kernel<%d, %d, %d, true, %d", NJ, SLOTS, GENS, XC)) kfn = jk;
-  cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  constexpr int Z = REV ? 1 : 0;  // as in the kernel
+  using G = GramGeom<NJ, Z>;
+  constexpr int PSTRIDE = gram_partial_doubles<NJ, Z, XC>();
+  const int nj = ch.host.nj, P = 10 * nj, Pc = ch.comps.cols, Pt = P + Pc;
+  // workspace: rigid block (P*P + P + 1) | cross sums (NXT*64) | per-CTA partials (sm_count*PSTRIDE) | component map (2 Pc ints)
+  const size_t n_rigid = (size_t)P * P + P + 1, n_sum = (size_t)G::NXT * 64, n_part = (size_t)ch.sm_count * PSTRIDE;
+  cudaError_t e = grow(ch.gram.ext_dev, ch.gram.ext_bytes, sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc);
   if (e != cudaSuccess) return e;
-  const int64_t ngroups = (in.n + 31) / 32;
-  const int grid = (int)std::min<int64_t>(ch.sm_count, ngroups);
-  {
-    ChainDev<NJ> C = narrow_g<NJ>(ch.gram.fold);
-    GramComps comps = gc;
-    SamplesDev ins = in;
-    const double* tm = tau_meas;
-    double* part = xpart;
-    void* args[] = {&C, &comps, &ins, &tm, &part};
-    e = cudaLaunchKernel(kfn, dim3(grid), dim3(G0::threads(GENS)), args, smem, st);
-    if (e != cudaSuccess) return e;
-  }
-  count_launch();
+  double* Gt = ch.gram.ext_dev;
+  double* bt = Gt + (size_t)P * P;
+  double* tst = bt + P;
+  double* xsum = tst + 1;
+  double* xpart = xsum + n_sum;
+  int32_t* dmap = reinterpret_cast<int32_t*>(xpart + n_part);
+  e = cudaMemcpyAsync(dmap, xmap.data(), sizeof(int32_t) * xmap.size(), cudaMemcpyHostToDevice, st);  // pageable source: staged before return
+  if (e != cudaSuccess) return e;
+  int grid = 0;
+  e = launch_fused_kernel<NJ, REV, XC>(ch, gc, in, tau_meas, xpart, &grid, st);
+  if (e != cudaSuccess) return e;
   if (ch.gram.fold_identity) launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gt, bt, tst, 0, st);
   else
   {
-    const int nj = ch.host.nj, Pr = G0::P;
     double* Gr = ch.gram.fold_dev + (size_t)nj * 100;
-    double* br = Gr + (size_t)Pr * Pr;
-    launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gr, br, br + Pr, 0, st);
+    double* br = Gr + (size_t)G::P * G::P;
+    launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gr, br, br + G::P, 0, st);
     e = launch_fold_expand(ch, Gt, bt, tst, 0, st);
     if (e != cudaSuccess) return e;
   }
-  gram_cross_reduce_kernel<<<(GX::NXT * 64 + 255) / 256, 256, 0, st>>>(xpart + G0::NT * 64, grid, GX::NXT * 64, PSTRIDE, xsum);
+  gram_cross_reduce_kernel<<<(G::NXT * 64 + 255) / 256, 256, 0, st>>>(xpart + G::NT * 64, grid, G::NXT * 64, PSTRIDE, xsum);
+  count_launch();
+  gram_ext_scatter_kernel<<<(P * (P + 1) + 255) / 256, 256, 0, st>>>(Gt, bt, tst, P, Pt, gram, rhs, tau_sq, accumulate);
+  count_launch();
+  const double* Tm1 = ch.gram.fold_identity ? nullptr : ch.gram.fold_dev;
+  const int32_t* kof1 =
+      ch.gram.fold_identity ? nullptr : reinterpret_cast<const int32_t*>(ch.gram.fold_dev + (size_t)nj * 100 + (size_t)(G::P + 1) * (G::P + 1));
+  gram_cross_finish_kernel<NJ, Z><<<((P + 1 + Pc) * Pc + 127) / 128, 128, 0, st>>>(xsum, Tm1, kof1, dmap, dmap + Pc, nj, Pc, gram, rhs, accumulate);
   count_launch();
   return cudaGetLastError();
 }
 
-// Normal equations of the extended model in one pass over the samples (gram_ext_kernel); the two-pass scheme (rigid-body kernel, then the cross
-// mode of gram_fused_kernel) is kept for development builds (RDB_GRAM_EXT=2).
+// Normal equations of the extended model in one pass over the samples.
 // cudaErrorNotSupported: more than 7 moving joints, a component on an input no chain joint feeds, or more than GX_COLS component columns
 // on one joint (caller falls back to the general pipeline).
 cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
@@ -427,7 +402,7 @@ cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const dou
 {
   if (in.n <= 0 || ch.gram.fold_version != ch.model_version) return cudaErrorNotSupported;
   const ChainDev<RDB_MAX_JOINTS>& F = ch.gram.fold;
-  const int K = F.nj, nj = ch.host.nj, P = 10 * nj, Pc = ch.comps.cols, Pt = P + Pc;
+  const int K = F.nj, Pc = ch.comps.cols;
   if (K < 1 || K > 7 || Pc <= 0) return cudaErrorNotSupported;
   GramComps gc{};
   std::vector<int32_t> xmap(2 * (size_t)Pc, 0);
@@ -452,55 +427,29 @@ cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const dou
     }
   }
   const bool rev = fold_rev_canonical(F);
-  const int zc = GF_ZCOL && rev ? 1 : 0;  // GramGeom Z of the kernel that will run
   int xcmax = 0;
   for (int j = 0; j < K; j++) xcmax = std::max(xcmax, (int)gc.ncols[j]);
-  int nxt = 0;
-  for (int j = 0; j < K; j++) nxt += (1 + 10 * (K - j) - zc + 7) / 8 + 1;  // GramGeom::nxt
-  const int Tt = (10 * K + 1 - zc + 7) / 8, ntt = Tt * (Tt + 1) / 2;      // GramGeom::T, NT
-  // workspace: rigid block (P*P + P + 1) | cross sums (nxt*64) | per-CTA partials (sm_count*(ntt+nxt)*64) | component map (2 Pc ints)
-  const size_t n_rigid = (size_t)P * P + P + 1, n_sum = (size_t)nxt * 64, n_part = (size_t)ch.sm_count * (ntt + nxt) * 64;
-  cudaError_t e = grow(ch.gram.ext_dev, ch.gram.ext_bytes, sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc);
-  if (e != cudaSuccess) return e;
-  double* Gt = ch.gram.ext_dev;
-  double* bt = Gt + (size_t)P * P;
-  double* tst = bt + P;
-  double* xsum = tst + 1;
-  double* xpart = xsum + n_sum;
-  int32_t* dmap = reinterpret_cast<int32_t*>(xpart + n_part);
-  e = cudaMemcpyAsync(dmap, xmap.data(), sizeof(int32_t) * xmap.size(), cudaMemcpyHostToDevice, st);  // pageable source: staged before return
-  if (e != cudaSuccess) return e;
   switch (K)
   {
 #define XL(N, R)                                                                                                  \
-  (xcmax <= 2 ? launch_ext_nj<N, R, 2>(ch, gc, in, tau_meas, Gt, bt, tst, xpart, xsum, st)                         \
-              : (xcmax <= 4 ? launch_ext_nj<N, R, 4>(ch, gc, in, tau_meas, Gt, bt, tst, xpart, xsum, st)           \
-                            : launch_ext_nj<N, R, 8>(ch, gc, in, tau_meas, Gt, bt, tst, xpart, xsum, st)))
-#define X(N)                                \
-  case N:                                   \
-  e = rev ? XL(N, true) : XL(N, false);     \
-  break;
+  (xcmax <= 2 ? launch_ext_nj<N, R, 2>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st)               \
+              : (xcmax <= 4 ? launch_ext_nj<N, R, 4>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st) \
+                            : launch_ext_nj<N, R, 8>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st)))
+#define X(N) \
+  case N:    \
+    return rev ? XL(N, true) : XL(N, false);
     X(1) X(2) X(3) X(4) X(5) X(6) X(7)
 #undef X
 #undef XL
   }
-  if (e != cudaSuccess) return e;
-  gram_ext_scatter_kernel<<<(P * (P + 1) + 255) / 256, 256, 0, st>>>(Gt, bt, tst, P, Pt, gram, rhs, tau_sq, accumulate);
-  count_launch();
-  const double* Tm1 = ch.gram.fold_identity ? nullptr : ch.gram.fold_dev;
-  const int32_t* kof1 = ch.gram.fold_identity
-                            ? nullptr
-                            : reinterpret_cast<const int32_t*>(ch.gram.fold_dev + (size_t)nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1));
-  gram_cross_finish_kernel<<<((P + 1 + Pc) * Pc + 127) / 128, 128, 0, st>>>(xsum, Tm1, kof1, dmap, dmap + Pc, nj, K, Pc, gram, rhs, accumulate, zc);
-  count_launch();
-  return cudaGetLastError();
+  return cudaErrorNotSupported;
 }
 
 // the row layout of gram_fused_kernel on all-revolute chains (host entry for tests, rdb_gram_row_layout)
 template <int NJ>
 static void gram_row_layout_nj(int32_t* pos, int32_t* rowlen, int32_t* tau_col)
 {
-  using G = GramGeom<NJ, 0, GF_ZCOL ? 2 : 0>;
+  using G = GramGeom<NJ, 2>;
   for (int j = 0; j < NJ; j++)
   {
     rowlen[j] = G::rowlen(j);

@@ -233,7 +233,7 @@ std::string kernel_expr(const char* kernel_args) { return std::string("&rdb::") 
 
 }  // namespace
 
-const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args, const std::string& defines)
+const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args)
 {
   std::string& why = ch.gram.kernel_why;
   ch.gram.kernel_specialised = 0;
@@ -243,13 +243,12 @@ const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args, const std::s
     why = "precompiled kernel: run-time specialisation disabled (RDB_GRAM_JIT=0)";
     return nullptr;
   }
-  const std::string model = model_source(ch.gram.fold);
-  if (model.empty())
+  const std::string src = model_source(ch.gram.fold);
+  if (src.empty())
   {
     why = "precompiled kernel: the model has non-finite constants";
     return nullptr;
   }
-  const std::string src = defines + model;
   const std::string expr = kernel_expr(kernel_args);
   int major = 0, minor = 0;
   cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, ch.device);
@@ -270,8 +269,7 @@ const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args, const std::s
   return reinterpret_cast<const void*>(it->second.kernel);
 }
 
-bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const std::string& defines, const char* arch,
-                    std::vector<char>& cubin, std::string& why)
+bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const char* arch, std::vector<char>& cubin, std::string& why)
 {
   const std::string model = model_source(F);
   if (model.empty())
@@ -280,7 +278,7 @@ bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, 
     return false;
   }
   std::string kname;
-  return compile_cubin(defines + model, kernel_expr(kernel_args), arch, cubin, kname, why);
+  return compile_cubin(model, kernel_expr(kernel_args), arch, cubin, kname, why);
 }
 
 }  // namespace rdb

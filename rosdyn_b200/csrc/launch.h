@@ -166,15 +166,11 @@ inline bool fold_rev_canonical(const ChainDev<RDB_MAX_JOINTS>& F)
           F.joint[j].ax[2] == REV_AXIS[2];
   return rev;
 }
-// gram_jit.cpp: the fused kernel `kernel_args` ("gram_fused_kernel<6, 4, true, 0, 4": template arguments without the model) compiled at run
+// gram_jit.cpp: the fused kernel `kernel_args` ("gram_fused_kernel<6, 4, true, 0": template arguments without the model) compiled at run
 // time against the constants of ch.gram.fold, or nullptr when the precompiled instantiation has to run; records which one and why in ch.gram.
-// defines: gram_jit_defines() (the launcher's geometry macros), compiled in front of the kernel headers and part of the cache key
-const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args, const std::string& defines);
+const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args);
 // gram_jit.cpp: the same kernel's cubin for `arch` (e.g. "sm_100a") without a device (rdb_gram_specialised_cubin)
-bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const std::string& defines, const char* arch,
-                    std::vector<char>& cubin, std::string& why);
-// gram_fused.cu: "#define GF_TSPLIT ..." lines with the values of the overridable geometry macros the launchers were compiled with
-std::string gram_jit_defines();
+bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const char* arch, std::vector<char>& cubin, std::string& why);
 // gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                               int accumulate, cudaStream_t st);

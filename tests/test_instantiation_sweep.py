@@ -9,8 +9,8 @@ every dispatch key of the launchers is reached:
 * regressor walker ``dyn_kernel<NJ, REGRESSOR, false, REC>`` on the unfolded chain, SoA and Eigen-record layouts;
 * torque / inertia / forward-dynamics walkers on the folded chain, K = 1..8 moving inputs x all-revolute or not, generic above 8;
 * wrench / link Jacobian (``aux_kernel``), fast and generic;
-* fused Gram ``gram_fused_kernel<K, .., REV>``, K = 1..7, run-time specialised (NVRTC) and precompiled twins;
-* extended Gram ``gram_ext_kernel<K, .., REV, XC>``, K = 1..7, XC = 2, 4, 8 component columns on the widest joint;
+* fused Gram ``gram_fused_kernel<K, .., REV, 0>``, K = 1..7, run-time specialised (NVRTC) and precompiled twins;
+* extended Gram ``gram_fused_kernel<K, .., REV, XC>``, K = 1..7, XC = 2, 4, 8 component columns on the widest joint;
 * the general Gram pipeline (gram.cu): K >= 8, no moving joint, and the component sets the one-pass kernel refuses.
 
 The CPU test recomputes each case's dispatch key from its descriptor with the launchers' rules and fails when the family stops covering

@@ -290,8 +290,8 @@ def test_input_selection_drops_components_and_tau_shape_is_checked(torch):
 
 @pytest.mark.parametrize("name", ["c6", "c7", "random_a"])
 def test_gram_is_bit_reproducible(name, torch):
-    """The producer / consumer handshake of the fused kernels (mbarriers; compute-sanitizer's racecheck does not model them and reports the
-    slot stores against the fragment loads) leaves no timing dependence: repeated runs on the same inputs are bit-identical, for batches
+    """The producer / consumer handshake of the fused kernels (release / acquire counters; compute-sanitizer's racecheck does not model them
+    and reports the slot stores against the fragment loads) leaves no timing dependence: repeated runs on the same inputs are bit-identical, for batches
     that end inside a group, a k-step and a slot."""
     from rosdyn_b200.chain import Chain, fill_uniform
     d = fixtures.by_name(name)

@@ -3,7 +3,7 @@
 
   python tools/gram_jit_sass_counts.py      -> profiles/gram_jit_sass.json
 
-For C6 and C7 (rosdyn_b200.fixtures), rdb_gram_specialised_cubin compiles gram_fused_kernel<K, SLOTS, true, 0, 4> against the chain's folded
+For C6 and C7 (rosdyn_b200.fixtures), rdb_gram_specialised_cubin compiles gram_fused_kernel<K, SLOTS, true, 0> against the chain's folded
 constants for sm_100a, as a Gram call on a B200 does.  The counts are taken as in tools/sass_counts.py (generator = the code in front of the
 first DMMA), next to the precompiled kernel's from profiles/gram_fused_sass.json; registers and spills come from cuobjdump -res-usage."""
 import ctypes
@@ -23,7 +23,7 @@ from rosdyn_b200 import _lib, fixtures  # noqa: E402
 from rosdyn_b200.descriptor import to_ctypes  # noqa: E402
 
 KPW = 2
-CHAINS = {"c6": "gram_fused_kernel<6, 4, true, 0, 4", "c7": "gram_fused_kernel<7, 3, true, 0, 4"}
+CHAINS = {"c6": "gram_fused_kernel<6, 4, true, 0", "c7": "gram_fused_kernel<7, 3, true, 0"}
 
 
 def count(cubin: str):

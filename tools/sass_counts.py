@@ -3,7 +3,7 @@
 
   python tools/sass_counts.py            -> profiles/gram_fused_sass.json  (+ profiles/r02_gram_fused_sass_summary.txt)
 
-For every instantiation gram_fused_kernel<K, ..., REV, X = 0>:
+For every rigid-body instantiation gram_fused_kernel<K, SLOTS, REV, XC = 0>:
   * gen_dp_instr_per_sample : FP64 instructions (DFMA / DMUL / DADD) one generator LANE executes for its sample (a warp instruction serves 32
     samples).  The generator's code is the straight-line region in front of the first DMMA of the kernel (the MMA roles follow it); the
     rarely taken library sincos for |q| > 1e5 is a CALL outside it.
@@ -24,6 +24,7 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 import sass_stalls  # noqa: E402
 
 KPW = 2
+GENS = 4  # generator warps of every instantiation (GF_GENS)
 
 
 def main():
@@ -33,11 +34,11 @@ def main():
     out, lines = {}, []
     for f in funcs:
         dem = subprocess.run(["c++filt", f], capture_output=True, text=True).stdout.strip()
-        m = re.search(r"gram_fused_kernel<(\d+), (\d+), (true|false|\(bool\)[01]), (\d+)(?:, (\d+))?(?:, rdb::RtModel)?>", dem)
+        m = re.search(r"gram_fused_kernel<(\d+), (\d+), (true|false|\(bool\)[01]), (\d+)(?:, rdb::RtModel)?>", dem)
         if not m:
             continue
-        K, slots, rev, X = int(m.group(1)), int(m.group(2)), m.group(3) in ("true", "(bool)1"), int(m.group(4))
-        if X != 0:
+        K, slots, rev, XC = int(m.group(1)), int(m.group(2)), m.group(3) in ("true", "(bool)1"), int(m.group(4))
+        if XC != 0:
             continue
         sass = subprocess.run(["cuobjdump", "-sass", "-fun", f, obj], capture_output=True, text=True).stdout.splitlines()
         ins = sass_stalls.parse(sass)
@@ -48,7 +49,7 @@ def main():
         mma_dfma = sum(1 for i in ins[first_dmma:] if re.match(r"(@!?U?P\d+\s+)?DFMA\b", i["text"]))
         dp = sum(cnt.values())
         key = f"K{K}_{'rev' if rev else 'gen'}"
-        out[key] = {"kernel": dem.split("(")[0].replace("void rdb::", "").replace(", rdb::RtModel>", ">"), "slots": slots, "generator_warps": int(m.group(5) or slots),
+        out[key] = {"kernel": dem.split("(")[0].replace("void rdb::", "").replace(", rdb::RtModel>", ">"), "slots": slots, "generator_warps": GENS,
                     "gen_dp_instr_per_sample": dp,
                     # flop per sample: every lane of a generator warp instruction works on its own sample
                     "gen_flop_per_sample": float(2 * cnt["DFMA"] + cnt["DMUL"] + cnt["DADD"]),
