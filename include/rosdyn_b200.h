@@ -23,7 +23,14 @@
  *   - a handle lives on ONE device (the current device at rdb_chain_create, or the one given to rdb_chain_create_on); every entry point
  *     makes that device current for the call and restores the caller's device, so handles of several devices can be driven from one thread;
  *   - entries that take `const rdb_chain*` only read the handle and may run concurrently on one handle (distinct streams); entries that take
- *     `rdb_chain*` use per-handle workspaces and are serialised by a per-handle lock.
+ *     `rdb_chain*` use per-handle workspaces and are serialised by a per-handle lock;
+ *   - the Gram entries of one handle (rdb_regressor_gram_batch, rdb_regressor_gram_ext_batch, rdb_regressor_gram_batch_host, and
+ *     rdb_regressor_gram_sharded on each device) run their device work in call order whatever the streams: each call's stream waits for the
+ *     device work of the previous call before it touches the shared workspace (free on the same stream).  They never overlap on one handle;
+ *     for concurrent Gram work use one handle per stream;
+ *   - a model change (rdb_chain_set_input_joints, and the creation of the handle) synchronises the handle's device before and after it
+ *     rewrites the device constants: calls queued before it, on any stream, complete on the old model, calls issued after it see the new one.
+ *     It is a set-up-time call.
  *
  * There is no CPU fallback: every compute entry fails with RDB_ERR_NO_DEVICE when no CUDA device exists.
  */
@@ -383,6 +390,7 @@ rdb_status rdb_group_synchronize(rdb_group* group);
 /* ---- host-buffer convenience wrappers (pointers are HOST pointers; copies + sync inside) ----------
  * The handle is NOT const here: the staging buffers, streams and events of these pipelines live in the handle (grown on demand, freed with
  * it).  Calls on one handle from several host threads are serialised by a per-handle lock (they do not race, they do not overlap either);
+ * rdb_regressor_gram_batch_host also waits for the device work of a Gram call still in flight on the handle (any stream) before it starts;
  * for concurrency use one handle per thread, as the reference does with Chain::clone() (P.h:554).  Pinned (cudaHostAlloc /
  * cudaHostRegister) buffers overlap the copies with the kernels at the link's rate; pageable buffers work: the entries gather / scatter them
  * through pinned bounce buffers of the handle with a few host threads (0.5 - 0.6 of the link's rate; the driver's own staging reaches 0.2 - 0.3).

@@ -7,6 +7,9 @@ Same method names and argument meaning as the reference; every method is ALSO it
 
 torch CUDA tensors go through the device entry points on torch's current stream (asynchronous, results are
 torch CUDA tensors); numpy arrays go through the ``*_host`` entry points (copies + sync inside, results numpy).
+Calls that only read the handle may overlap on distinct streams; the regressorGram* calls of one Chain run one after the other on the device
+whatever the streams (they share the handle's workspace: one Chain per stream for concurrent Gram work), and setInputJointsName waits
+for every call already queued.
 torch is used for device memory and streams only.  There is no CPU fallback: constructing a Chain without the
 built library or without a CUDA device raises.
 """

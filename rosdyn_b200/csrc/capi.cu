@@ -128,14 +128,19 @@ static rdb_status build_model(const rdb_chain_desc* d, ChainHost* ch)
   return RDB_OK;
 }
 
-// the handle's device (fixed at creation) must be current: every caller holds a DeviceScope
+// the handle's device (fixed at creation) must be current: every caller holds a DeviceScope.
+// Kernels read the model constants (ch->dev) and the fold maps (ch->gram.fold_dev) from device memory while they run, and the const entries
+// may have queued them on any stream without a trace in the handle: the device is synchronised before the constants are rewritten, and
+// again after, so that no stream can start on a copy still in flight.  A set-up-time call.
 static rdb_status upload_model(ChainHost* ch)
 {
+  RDB_CUDA(cudaDeviceSynchronize());
   if (!ch->dev) RDB_CUDA(cudaMalloc(&ch->dev, sizeof(ch->host)));
   RDB_CUDA(cudaMemcpy(ch->dev, &ch->host, sizeof(ch->host), cudaMemcpyHostToDevice));
   cudaDeviceGetAttribute(&ch->sm_count, cudaDevAttrMultiProcessorCount, ch->device);
   ch->model_version++;
   RDB_CUDA(fold_chain(*ch));
+  RDB_CUDA(cudaDeviceSynchronize());
   return RDB_OK;
 }
 
@@ -245,6 +250,8 @@ void rdb_chain_destroy(rdb_chain* chain)
 {
   if (!chain) return;
   DeviceScope dev__(chain->device);
+  cudaDeviceSynchronize();  // work queued on the caller's streams may still read the model and the workspaces freed below
+  if (chain->gram.done) cudaEventDestroy(chain->gram.done);
   if (chain->dev) cudaFree(chain->dev);
   if (chain->gram.partials) cudaFree(chain->gram.partials);
   if (chain->gram.fused_partials) cudaFree(chain->gram.fused_partials);
@@ -428,7 +435,7 @@ rdb_status rdb_regressor_gram_batch(rdb_chain* chain, const rdb_samples* in, con
   rdb_status s = check_samples(chain, in, true);
   if (s != RDB_OK) return s;
   RDB_ENTER(chain);
-  RDB_LOCK(chain);  // the per-CTA partials live in the handle
+  RDB_LOCK(chain);  // host-side state of the Gram workspace; launch_gram orders the device work of successive calls across streams
   if (in->n > 0 && (!in->dq || !in->ddq)) return fail(RDB_ERR_DIM_MISMATCH, "Input data dimensions mismatch");
   if (!gram || !rhs) return fail(RDB_ERR_INVALID_ARG, "gram / rhs must not be null");
   RDB_CUDA(launch_gram(*chain, to_dev(in), tau_meas, gram, rhs, tau_sq, accumulate, (cudaStream_t)stream));

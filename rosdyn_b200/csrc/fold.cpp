@@ -210,6 +210,7 @@ cudaError_t fold_chain(ChainHost& ch, bool upload)
   w.fold_identity = (K == H.nj) && !rotated;
   if (upload && !w.fold_identity && K > 0)
   {
+    // the caller (upload_model) has synchronised the device: no kernel still reads fold_dev, so it may be freed and rewritten here
     const size_t need = sizeof(double) * ((size_t)H.nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1)) + sizeof(int32_t) * H.nj;
     if (w.fold_bytes < need)
     {

@@ -193,8 +193,8 @@ __global__ void __launch_bounds__(256) gram_unfed_tau_sq_kernel(const double* __
   }
 }
 
-cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
-                        cudaStream_t st, bool with_components)
+static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
+                                 int accumulate, cudaStream_t st, bool with_components)
 {
   const int n_in = ch.host.n_in, Pr = 10 * ch.host.nj;     // rigid-body columns
   const int P = Pr + (with_components ? ch.comps.cols : 0);  // + component columns (extended model)
@@ -267,7 +267,12 @@ cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_m
   const size_t need = sizeof(double) * ((size_t)chunk * (P * n_in + n_in) + (size_t)gx * npairs * TILE_ELEMS);
   if (ch.gram.bytes < need)
   {
-    if (ch.gram.partials) cudaFree(ch.gram.partials);
+    if (ch.gram.partials)
+    {
+      cudaError_t e = cudaEventSynchronize(ch.gram.done);  // the previous Gram call may still read the old buffer
+      if (e != cudaSuccess) return e;
+      cudaFree(ch.gram.partials);
+    }
     ch.gram.partials = nullptr;
     ch.gram.bytes = 0;
     cudaError_t e = cudaMalloc(&ch.gram.partials, need);
@@ -307,6 +312,21 @@ cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_m
     if (e != cudaSuccess) return e;
   }
   return cudaSuccess;
+}
+
+// Every Gram call of a handle (device entries, the host entry's chunks, the group's shards) goes through here.  The workspace of
+// ch.gram is shared by all of them, and callers may pass any stream: each call's stream first waits for the device work of the previous
+// call (free on the same stream), and the call's own work is recorded for the next one.
+cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
+                        cudaStream_t st, bool with_components)
+{
+  cudaError_t e = ch.gram.done ? cudaSuccess : cudaEventCreateWithFlags(&ch.gram.done, cudaEventDisableTiming);
+  if (e != cudaSuccess) return e;
+  e = cudaStreamWaitEvent(st, ch.gram.done, 0);
+  if (e != cudaSuccess) return e;
+  e = gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components);
+  const cudaError_t r = cudaEventRecord(ch.gram.done, st);  // also after a failed launch: whatever was queued stays ordered
+  return e != cudaSuccess ? e : r;
 }
 
 // ---------------------------------------------------------------------------------------------------------

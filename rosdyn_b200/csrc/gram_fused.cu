@@ -164,10 +164,16 @@ static ChainDev<NJ> narrow_g(const ChainDev<RDB_MAX_JOINTS>& h)
   return c;
 }
 
-static cudaError_t grow(double*& p, size_t& have, size_t need)
+// done: the handle's Gram event (launch_gram); the previous Gram call, possibly on another stream, may still use the old buffer
+static cudaError_t grow(double*& p, size_t& have, size_t need, cudaEvent_t done)
 {
   if (have >= need) return cudaSuccess;
-  if (p) cudaFree(p);
+  if (p)
+  {
+    const cudaError_t e = cudaEventSynchronize(done);
+    if (e != cudaSuccess) return e;
+    cudaFree(p);
+  }
   p = nullptr;
   have = 0;
   cudaError_t e = cudaMalloc(&p, need);
@@ -230,7 +236,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
 {
   constexpr int Z = REV ? 2 : 0;  // as in the kernel
   using G = GramGeom<NJ, Z>;
-  cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL);
+  cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL, ch.gram.done);
   if (e != cudaSuccess) return e;
   int grid = 0;
   e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, ch.gram.fused_partials, &grid, st);
@@ -360,7 +366,8 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   const int nj = ch.host.nj, P = 10 * nj, Pc = ch.comps.cols, Pt = P + Pc;
   // workspace: rigid block (P*P + P + 1) | cross sums (NXT*64) | per-CTA partials (sm_count*PSTRIDE) | component map (2 Pc ints)
   const size_t n_rigid = (size_t)P * P + P + 1, n_sum = (size_t)G::NXT * 64, n_part = (size_t)ch.sm_count * PSTRIDE;
-  cudaError_t e = grow(ch.gram.ext_dev, ch.gram.ext_bytes, sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc);
+  cudaError_t e = grow(ch.gram.ext_dev, ch.gram.ext_bytes, sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc,
+                       ch.gram.done);
   if (e != cudaSuccess) return e;
   double* Gt = ch.gram.ext_dev;
   double* bt = Gt + (size_t)P * P;

@@ -104,6 +104,7 @@ struct rdb_group
   std::vector<ncclComm_t> comms;     // one communicator per local device
   std::vector<double*> packed;       // [G | b | tau_sq] on each local device
   std::vector<cudaStream_t> streams; // default streams of the group (used when the caller passes none)
+  std::vector<cudaEvent_t> done;     // recorded after the last use of packed[k] by a call; the next call on device k waits for it
   int nranks = 0;                    // ranks in the communicator (local devices for rdb_group_create, all processes for rdb_group_create_rank)
   int P = 0;
   std::mutex mu;
@@ -136,6 +137,10 @@ static rdb_status group_alloc(rdb_group* g, const rdb_chain_desc* desc, int ndev
     e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
     if (e != cudaSuccess) return cuda_fail_g(e, "cudaStreamCreate");
     g->streams.push_back(st);
+    cudaEvent_t ev = nullptr;
+    e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e != cudaSuccess) return cuda_fail_g(e, "cudaEventCreate");
+    g->done.push_back(ev);
   }
   return RDB_OK;
 }
@@ -152,6 +157,7 @@ void rdb_group_destroy(rdb_group* g)
     if (k < g->comms.size() && g->comms[k] && a.CommDestroy) a.CommDestroy(g->comms[k]);
     if (k < g->packed.size() && g->packed[k]) cudaFree(g->packed[k]);
     if (k < g->streams.size() && g->streams[k]) cudaStreamDestroy(g->streams[k]);
+    if (k < g->done.size() && g->done[k]) cudaEventDestroy(g->done[k]);
   }
   for (rdb_chain* ch : g->chains) rdb_chain_destroy(ch);
   delete g;
@@ -256,11 +262,17 @@ rdb_status rdb_regressor_gram_sharded(rdb_group* g, const rdb_samples* shards, c
   const int nd = (int)g->chains.size(), P = g->P;
   const size_t n_out = (size_t)P * P + P + 1;
   NcclApi& a = nccl();
-  // 1. every local device: fused regressor -> normal equations of its shard, written straight into the packed buffer
+  // 1. every local device: fused regressor -> normal equations of its shard, written straight into the packed buffer once the previous
+  //    call, whatever its stream, has unpacked it
   for (int k = 0; k < nd; k++)
   {
     cudaStream_t st = streams ? (cudaStream_t)streams[k] : g->streams[(size_t)k];  // an entry of `streams` may be 0 = the default stream
     double* pk = g->packed[(size_t)k];
+    {
+      DeviceScope dev(rdb_chain_device(g->chains[(size_t)k]));
+      const cudaError_t e = cudaStreamWaitEvent(st, g->done[(size_t)k], 0);
+      if (e != cudaSuccess) return cuda_fail_g(e, "cudaStreamWaitEvent");
+    }
     const rdb_status s = rdb_regressor_gram_batch(g->chains[(size_t)k], &shards[k], tau_meas ? tau_meas[k] : nullptr, pk, pk + (size_t)P * P,
                                                   pk + (size_t)P * P + P, 0, st);
     if (s != RDB_OK) return s;
@@ -281,19 +293,23 @@ rdb_status rdb_regressor_gram_sharded(rdb_group* g, const rdb_samples* shards, c
     if (r != kNcclSuccess) return nccl_fail(r, "ncclAllReduce");
     if (r2 != kNcclSuccess) return nccl_fail(r2, "ncclGroupEnd");
   }
-  // 3. into the caller's arrays
+  // 3. into the caller's arrays; packed[k] is free for the next call after this
   for (int k = 0; k < nd; k++)
   {
     double* G = gram ? gram[k] : nullptr;
     double* b = rhs ? rhs[k] : nullptr;
     double* t = tau_sq ? tau_sq[k] : nullptr;
-    if (!G && !b && !t) continue;
     cudaStream_t st = streams ? (cudaStream_t)streams[k] : g->streams[(size_t)k];  // an entry of `streams` may be 0 = the default stream
     DeviceScope dev(rdb_chain_device(g->chains[(size_t)k]));
-    group_unpack_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, st>>>(g->packed[(size_t)k], P, G, b, t, accumulate);
-    count_launch();
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail_g(e, "group_unpack_kernel");
+    if (G || b || t)
+    {
+      group_unpack_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, st>>>(g->packed[(size_t)k], P, G, b, t, accumulate);
+      count_launch();
+      const cudaError_t e = cudaGetLastError();
+      if (e != cudaSuccess) return cuda_fail_g(e, "group_unpack_kernel");
+    }
+    const cudaError_t e = cudaEventRecord(g->done[(size_t)k], st);
+    if (e != cudaSuccess) return cuda_fail_g(e, "cudaEventRecord");
   }
   return RDB_OK;
 }

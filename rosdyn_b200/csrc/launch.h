@@ -28,6 +28,10 @@ struct GramWorkspace
   double* ext_dev = nullptr;   // extended model: rigid-body block | cross-tile sums | cross partials | component map
   size_t ext_bytes = 0;
   double* tau_sq_part = nullptr;  // gram.cu: the fused kernels' tau^T tau when measured torques also sit on inputs no chain joint feeds
+  // recorded after the last launch of every Gram call (launch_gram): the next call's stream waits for it before it touches the buffers
+  // above, so the Gram calls of one handle run their device work in call order whatever streams they come on; a buffer is freed only
+  // once it has completed
+  cudaEvent_t done = nullptr;
   // which kernel the last Gram call ran (rdb_chain_gram_kernel_info): 1 run-time specialised (gram_jit.cpp), 0 precompiled, 2 general
   // pipeline (gram.cu), -1 none yet
   int kernel_specialised = -1;
@@ -139,7 +143,8 @@ cudaError_t launch_fill_uniform(double* x, int n_planes, int64_t n, int64_t ld, 
 void fill_uniform_host(double* x, int n_planes, int64_t n, int64_t ld, uint64_t seed, int stream_id);
 
 // gram.cu
-// with_components: the extended model [Phi | Phi_c] (general pipeline); else the rigid-body columns only (fused kernel when it fits)
+// with_components: the extended model [Phi | Phi_c] (general pipeline); else the rigid-body columns only (fused kernel when it fits).
+// Ordered after the previous Gram call of the handle on any stream (ch.gram.done).
 cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                         int accumulate, cudaStream_t st, bool with_components = false);
 // aux.cu: getWrench / getJointTorque with external wrenches, getJacobianLink (two-pass kernels, not the throughput path)
@@ -154,7 +159,8 @@ cudaError_t launch_components_regressor(const ChainHost& ch, const SamplesDev& i
 cudaError_t launch_components_torque(const ChainHost& ch, const SamplesDev& in, const ComponentParams& prm, double* torque, int64_t ld_out,
                                      int accumulate, cudaStream_t st);
 cudaError_t fp64_peak(int kind, int reps, double* tflops);
-// fold.cpp: the chain with its never-moving joints folded away and its revolute axes on +z (ch.gram.fold); rebuilt by every model upload
+// fold.cpp: the chain with its never-moving joints folded away and its revolute axes on +z (ch.gram.fold); rebuilt by every model upload.
+// upload = true rewrites ch.gram.fold_dev: no work that reads it may be queued or running (upload_model synchronises the device first)
 cudaError_t fold_chain(ChainHost& ch, bool upload = true);  // upload = false: the host image ch.gram.fold only
 // every joint of the folded chain is revolute about exactly e_z of its link frame: the fused kernels' REV generators (gram_common.cuh) hold
 // the axis as a compile-time constant; any other chain takes the generic generator
