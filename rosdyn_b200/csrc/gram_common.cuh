@@ -317,12 +317,12 @@ __device__ __forceinline__ T3<X, Y, W> mk3(X x, Y y, W z)
 {
   return T3<X, Y, W>{x, y, z};
 }
-template <class A>
-__device__ __forceinline__ V3 tod3(const A& a)
-{
-  return V3{tv_d(a.x), tv_d(a.y), tv_d(a.z)};
-}
 // the operations of spatial.cuh, in the same order, on typed vectors (V3 or T3)
+template <class A, class B>
+__device__ __forceinline__ auto tsub(const A& a, const B& b)
+{
+  return mk3(tadd(a.x, tneg(b.x)), tadd(a.y, tneg(b.y)), tadd(a.z, tneg(b.z)));
+}
 template <class A, class B>
 __device__ __forceinline__ auto tdot(const A& a, const B& b)
 {
@@ -388,9 +388,9 @@ __device__ __forceinline__ void gram_emit(const ChainDev<NJ>& C, double (&tau)[N
     if (G::stored(J, L, p))  // the exact zeros the layout drops are not stored
       o[G::pos(L, p) * 32 + (lane ^ (4 * (G::pos(L, p) & 3)))] = e[p];
 }
-template <class M, int NJ, int Z, int L, int J, class U, class S>
+template <class M, int NJ, int Z, int L, int J, class U, class S, class Fm, class W, class Al>
 __device__ __forceinline__ void gram_project(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, const U& u, const S& s,
-                                             const V3& fm, const V3& w, const V3& al)
+                                             const Fm& fm, const W& w, const Al& al)
 {
   const auto h = tcross_add(tcross_add(tcross(u, al), w, tcross(w, u)), fm, s);
   const auto rho = tcross(s, w);
@@ -405,64 +405,111 @@ __device__ __forceinline__ void gram_project(const ChainDev<NJ>& C, double (&tau
 // joint type and the axis are then compile-time facts: R = A' Rz(q) mixes two columns of A', the rates gain their e_z terms directly, the
 // first transport of a joint's unit twist [0; e_z] is a row of R, and the projection of a link on its own joint has closed forms with two
 // exact zeros (the mass and m c_z columns).  M: where the model constants come from (RtModel, or a run-time generated model type).
+// With a compile-time model the walk's state stays typed as well (T3 of double / Zr / Un): the base at rest, gravity, the rate terms and the
+// carried unit twists keep the exact zeros and ones they inherit from the model, so their products are not issued either.  The types change
+// from link to link, hence one function instantiation per link (gram_rev_link) that takes the state by value, and the carried twists of the
+// earlier joints as a pack that grows by one per link (RevTwists).  With RtModel every component is a double and the code is the
+// precompiled walk.
+
+// the unit twists (U_j, S_j) of joints 0 .. N-1 moved to the current link: the last joint in front, the earlier ones in `rest`
+struct RevTwistsEnd
+{
+  static constexpr int N = 0;
+};
+template <class U, class S, class Rest>
+struct RevTwists
+{
+  static constexpr int N = Rest::N + 1;
+  U u;
+  S s;
+  Rest rest;
+};
+template <class U, class S, class Rest>
+__device__ __forceinline__ RevTwists<U, S, Rest> mk_twists(const U& u, const S& s, const Rest& rest)
+{
+  return RevTwists<U, S, Rest>{u, s, rest};
+}
+// every twist of the pack moved one link further: U = R^T (U + S x t), S = R^T S
+template <class R, class T, class P>
+__device__ __forceinline__ auto rev_transport(const R& r, const T& t, const P& p)
+{
+  if constexpr (P::N == 0) return p;
+  else
+  {
+    const auto rest = rev_transport(r, t, p.rest);
+    return mk_twists(trotT(r, tcross_add(p.u, p.s, t)), trotT(r, p.s), rest);
+  }
+}
+// the projections of link L on the joints of the pack (joint P::N - 1 in front)
+template <class M, int NJ, int Z, int L, class P, class Fm, class W, class Al>
+__device__ __forceinline__ void rev_project(const ChainDev<NJ>& C, double (&tau)[NJ], double* __restrict__ slot, int lane, const P& p, const Fm& fm,
+                                            const W& w, const Al& al)
+{
+  if constexpr (P::N > 0)
+  {
+    rev_project<M, NJ, Z, L>(C, tau, slot, lane, p.rest, fm, w, al);
+    gram_project<M, NJ, Z, L, P::N - 1>(C, tau, slot, lane, p.u, p.s, fm, w, al);
+  }
+}
+
+// link L of the REV walk: v, w, a, al, g of link L-1 (L == 0: the base at rest and the model's gravity) and the twists of joints 0 .. L-2
+// moved to link L-1
+template <int L, int NJ, class M, int Z, class V, class W, class A, class Al, class G, class P>
+__device__ __forceinline__ void gram_rev_link(const ChainDev<NJ>& C, const GenIn<NJ>& x, double* __restrict__ slot, int lane, double (&tau)[NJ],
+                                              const V& vp, const W& wp, const A& ap, const Al& alp, const G& gp, const P& twists)
+{
+  if constexpr (L < NJ)
+  {
+    const double dql = x.dq[L], ddql = x.ddq[L];
+    const double sl = x.sv[L], cl = x.cv[L];
+    const auto t = mk3(kc<M, MK_T, L, 0>(C), kc<M, MK_T, L, 1>(C), kc<M, MK_T, L, 2>(C));
+    // R = A' Rz(q), row k: (fma(s, A'[k][1], c A'[k][0]), fma(-s, A'[k][0], c A'[k][1]), A'[k][2])
+    auto row = [&](auto kc_) {
+      constexpr int k = decltype(kc_)::value;
+      const auto a0 = kc<M, MK_A, L, 3 * k>(C);
+      const auto a1 = kc<M, MK_A, L, 3 * k + 1>(C);
+      return mk3(tfma(sl, a1, tmul(cl, a0)), tfma(-sl, a0, tmul(cl, a1)), kc<M, MK_A, L, 3 * k + 2>(C));
+    };
+    const auto R = mk3(row(ic<0>{}), row(ic<1>{}), row(ic<2>{}));
+    const auto v = trotT(R, tcross_add(vp, wp, t));
+    const auto wr = trotT(R, wp);
+    const auto ar = trotT(R, tcross_add(ap, alp, t));
+    const auto alr = trotT(R, alp);
+    const auto g = trotT(R, gp);
+    // s = e_z:  w += s Dq,  a += (v x s) Dq,  al += (w x s) Dq + s DDq
+    const auto w = mk3(wr.x, wr.y, tadd(wr.z, dql));
+    const auto a = mk3(tfma(v.y, dql, ar.x), tfma(tneg(v.x), dql, ar.y), ar.z);
+    const auto al = mk3(tfma(w.y, dql, alr.x), tfma(tneg(w.x), dql, alr.y), tadd(alr.z, ddql));
+    // [0; e_z] of joint L-1 moved to link L: S = R^T e_z, U = R^T (e_z x t), in front of the earlier joints' twists moved on
+    const auto moved = [&] {
+      if constexpr (L == 0) return twists;
+      else
+        return mk_twists(mk3(tfma(t.x, R.y.x, tneg(tmul(t.y, R.x.x))), tfma(t.x, R.y.y, tneg(tmul(t.y, R.x.y))),
+                             tfma(t.x, R.y.z, tneg(tmul(t.y, R.x.z)))),
+                         R.z, rev_transport(R, t, twists));
+    }();
+    const auto fm = tcross_add(tsub(a, g), w, v);
+    rev_project<M, NJ, Z, L>(C, tau, slot, lane, moved, fm, w, al);
+    // own joint, unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
+    const auto e7 = tmul(w.x, w.y);
+    gram_emit<M, NJ, Z, L, L, true>(C, tau, slot, lane, Zr{}, fm.y, tneg(fm.x), Zr{}, tneg(e7), tfma(w.x, w.x, tneg(tmul(w.y, w.y))),
+                                    tfma(tneg(w.y), w.z, al.x), e7, tfma(w.x, w.z, al.y), al.z);
+    gram_rev_link<L + 1, NJ, M, Z>(C, x, slot, lane, tau, v, w, a, al, g, moved);
+  }
+}
+
 template <int NJ, class M, int Z>
 __device__ __forceinline__ void gram_walk_rev(const ChainDev<NJ>& C, const GenIn<NJ>& x, double* __restrict__ slot, int lane, double (&tau)[NJ])
 {
   static_assert(REV_AXIS[0] == 0.0 && REV_AXIS[1] == 0.0 && REV_AXIS[2] == 1.0, "the REV walk below is written for the axis s = e_z");
-  V3 U[NJ], S[NJ];
-  V3 v = v3(0, 0, 0), w = v3(0, 0, 0), a = v3(0, 0, 0), al = v3(0, 0, 0), g;
-  static_for<0, NJ>([&](auto lc) {
-    constexpr int l = decltype(lc)::value;
-    const double dql = x.dq[l], ddql = x.ddq[l];
-    const double sl = x.sv[l], cl = x.cv[l];
-    const auto t = mk3(kc<M, MK_T, l, 0>(C), kc<M, MK_T, l, 1>(C), kc<M, MK_T, l, 2>(C));
-    // R = A' Rz(q), row k: (fma(s, A'[k][1], c A'[k][0]), fma(-s, A'[k][0], c A'[k][1]), A'[k][2])
-    auto row = [&](auto kc_) {
-      constexpr int k = decltype(kc_)::value;
-      const auto a0 = kc<M, MK_A, l, 3 * k>(C);
-      const auto a1 = kc<M, MK_A, l, 3 * k + 1>(C);
-      return mk3(tfma(sl, a1, tmul(cl, a0)), tfma(-sl, a0, tmul(cl, a1)), kc<M, MK_A, l, 3 * k + 2>(C));
-    };
-    const auto R = mk3(row(ic<0>{}), row(ic<1>{}), row(ic<2>{}));
-    v = tod3(trotT(R, tcross_add(v, w, t)));
-    w = tod3(trotT(R, w));
-    a = tod3(trotT(R, tcross_add(a, al, t)));
-    al = tod3(trotT(R, al));
-    if constexpr (l == 0) g = tod3(trotT(R, mk3(kc<M, MK_G, 0, 0>(C), kc<M, MK_G, 0, 1>(C), kc<M, MK_G, 0, 2>(C))));
-    else g = tod3(trotT(R, g));
-    // s = e_z:  w += s Dq,  a += (v x s) Dq,  al += (w x s) Dq + s DDq
-    w.z += dql;
-    a.x = fma(v.y, dql, a.x);
-    a.y = fma(-v.x, dql, a.y);
-    al.x = fma(w.y, dql, al.x);
-    al.y = fma(-w.x, dql, al.y);
-    al.z += ddql;
-    static_for<0, (l > 0 ? l - 1 : 0)>([&](auto jc) {
-      constexpr int j = decltype(jc)::value;
-      U[j] = tod3(trotT(R, tcross_add(U[j], S[j], t)));
-      S[j] = tod3(trotT(R, S[j]));
-    });
-    // [0; e_z] of joint l-1 moved to link l: S = R^T e_z, U = R^T (e_z x t) -- typed, for the projection of this link
-    const auto S1 = R.z;
-    const auto U1 = mk3(tfma(t.x, R.y.x, tneg(tmul(t.y, R.x.x))), tfma(t.x, R.y.y, tneg(tmul(t.y, R.x.y))), tfma(t.x, R.y.z, tneg(tmul(t.y, R.x.z))));
-    if constexpr (l > 0)
-    {
-      S[l - 1] = tod3(S1);
-      U[l - 1] = tod3(U1);
-    }
-    const V3 fm = cross_add(a - g, w, v);
-    static_for<0, l + 1>([&](auto jc) {
-      constexpr int j = decltype(jc)::value;
-      if constexpr (j == l)  // unit twist [0; e_z]: u = 0, h = fm x e_z, rho = e_z x w
-      {
-        const double e7 = w.x * w.y;
-        gram_emit<M, NJ, Z, l, j, true>(C, tau, slot, lane, Zr{}, fm.y, -fm.x, Zr{}, -e7, fma(w.x, w.x, -(w.y * w.y)), fma(-w.y, w.z, al.x),
-                                        e7, fma(w.x, w.z, al.y), al.z);
-      }
-      else if constexpr (j == l - 1) gram_project<M, NJ, Z, l, j>(C, tau, slot, lane, U1, S1, fm, w, al);
-      else gram_project<M, NJ, Z, l, j>(C, tau, slot, lane, U[j], S[j], fm, w, al);
-    });
-  });
+  // the base is at rest: v = w = a = al = 0 (with RtModel doubles of +0.0, like every other value there)
+  const auto z = [] {
+    if constexpr (M::RUNTIME) return 0.0;
+    else return Zr{};
+  }();
+  const auto z3 = mk3(z, z, z);
+  gram_rev_link<0, NJ, M, Z>(C, x, slot, lane, tau, z3, z3, z3, z3, mk3(kc<M, MK_G, 0, 0>(C), kc<M, MK_G, 0, 1>(C), kc<M, MK_G, 0, 2>(C)),
+                             RevTwistsEnd{});
 }
 
 // any joint types and axes (the constant-bank model)

@@ -24,7 +24,8 @@
 //   * all-revolute chains whose folded axes are all e_z (fold.cpp puts every revolute link in such a canonical frame) run the REV generator,
 //     which holds the axis as a compile-time constant: 2 019 instead of 2 412 FP64 instructions per sample for 6 joints (2 658 / 3 119 for 7).
 //   * on such chains the launchers run the same kernel compiled at run time against the chain's own constants (gram_jit.cpp, model type M):
-//     the products with exact zeros and ones are not issued, 1 347 FP64 instructions per sample for C6 (1 851 for C7), same results.
+//     the products with the exact zeros and ones of the model, and of the walk's state that inherits them (the base at rest, gravity, the
+//     carried unit twists), are not issued: 1 082 FP64 instructions per sample for C6 (1 522 for C7), same results.
 // Per-CTA partials (tiles, then b and tau^T tau) are summed in a fixed order by gram_fused_reduce_kernel (bit-reproducible for a given n).
 // XC > 0: the extended model [Phi | Phi_c] (friction / spring columns) in ONE pass -- the same slots, the component columns of every joint
 // in a small side buffer next to each slot, the MMA warps keep the rigid-body tiles and the cross tiles in registers.

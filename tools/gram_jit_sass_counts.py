@@ -3,8 +3,9 @@
 
   python tools/gram_jit_sass_counts.py      -> profiles/gram_jit_sass.json
 
-For C6 and C7 (rosdyn_b200.fixtures), rdb_gram_specialised_cubin compiles gram_fused_kernel<K, SLOTS, true, 0> against the chain's folded
-constants for sm_100a, as a Gram call on a B200 does.  The counts are taken as in tools/sass_counts.py (generator = the code in front of the
+For C6 and C7 (rosdyn_b200.fixtures), rdb_gram_specialised_cubin compiles gram_fused_kernel<K, SLOTS, true, XC> against the chain's folded
+constants for sm_100a, as a Gram call on a B200 does: the rigid-body kernel (XC = 0) and the extended model with a two-column component
+(friction) on every joint (XC = 2, tools/bench_ext.py).  The counts are taken as in tools/sass_counts.py (generator = the code in front of the
 first DMMA), next to the precompiled kernel's from profiles/gram_fused_sass.json; registers and spills come from cuobjdump -res-usage."""
 import ctypes
 import json
@@ -23,7 +24,8 @@ from rosdyn_b200 import _lib, fixtures  # noqa: E402
 from rosdyn_b200.descriptor import to_ctypes  # noqa: E402
 
 KPW = 2
-CHAINS = {"c6": "gram_fused_kernel<6, 4, true, 0", "c7": "gram_fused_kernel<7, 3, true, 0"}
+CHAINS = {"c6": "gram_fused_kernel<6, 4, true, 0", "c7": "gram_fused_kernel<7, 3, true, 0", "c6_ext": "gram_fused_kernel<6, 4, true, 2",
+          "c7_ext": "gram_fused_kernel<7, 3, true, 2"}
 
 
 def count(cubin: str):
@@ -47,7 +49,7 @@ def main():
     out = {}
     with tempfile.TemporaryDirectory() as tmp:
         for name, kargs in CHAINS.items():
-            cdesc, keep = to_ctypes(fixtures.by_name(name))
+            cdesc, keep = to_ctypes(fixtures.by_name(name.split("_")[0]))
             path = os.path.join(tmp, name + ".cubin")
             why = ctypes.create_string_buffer(4096)
             t0 = time.perf_counter()
@@ -57,9 +59,10 @@ def main():
             if st != 0:
                 raise SystemExit(f"{name}: {lib.rdb_last_error().decode()}")
             r = count(path)
-            K = int(kargs.split("<")[1].split(",")[0])
+            K, XC = (int(a) for a in kargs.split("<")[1].split(", ")[::3])
             r.update({"kernel": kargs + ", GramJitModel>", "nvrtc_compile_s_cpu": round(dt, 2),
-                      "precompiled_gen_dp_instr_per_sample": pre.get(f"K{K}_rev", {}).get("gen_dp_instr_per_sample")})
+                      # profiles/gram_fused_sass.json counts the rigid-body kernels only
+                      "precompiled_gen_dp_instr_per_sample": pre.get(f"K{K}_rev", {}).get("gen_dp_instr_per_sample") if XC == 0 else None})
             out[name] = r
             print(f"{name}: generator FP64 instr / sample {r['gen_dp_instr_per_sample']} (precompiled {r['precompiled_gen_dp_instr_per_sample']}; "
                   f"DFMA {r['gen_ops']['DFMA']}, DMUL {r['gen_ops']['DMUL']}, DADD {r['gen_ops']['DADD']}), DMMA per 4 samples "
