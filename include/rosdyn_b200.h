@@ -24,8 +24,8 @@
  *     makes that device current for the call and restores the caller's device, so handles of several devices can be driven from one thread;
  *   - entries that take `const rdb_chain*` only read the handle and may run concurrently on one handle (distinct streams); entries that take
  *     `rdb_chain*` use per-handle workspaces and are serialised by a per-handle lock;
- *   - the Gram entries of one handle (rdb_regressor_gram_batch, rdb_regressor_gram_ext_batch, rdb_regressor_gram_batch_host, and
- *     rdb_regressor_gram_sharded on each device) run their device work in call order whatever the streams: each call's stream waits for the
+ *   - the Gram entries of one handle (rdb_regressor_gram_batch, rdb_regressor_gram_segmented_batch, rdb_regressor_gram_ext_batch,
+ *     rdb_regressor_gram_batch_host, and rdb_regressor_gram_sharded on each device) run their device work in call order whatever the streams: each call's stream waits for the
  *     device work of the previous call before it touches the shared workspace (free on the same stream).  They never overlap on one handle;
  *     for concurrent Gram work use one handle per stream;
  *   - a model change (rdb_chain_set_input_joints, and the creation of the handle) synchronises the handle's device before and after it
@@ -236,6 +236,21 @@ rdb_status rdb_forward_dynamics_batch(const rdb_chain* chain, const rdb_samples*
 rdb_status rdb_regressor_gram_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, double* gram, double* rhs,
                                     double* tau_sq, int32_t accumulate, void* stream);
 
+/* Normal equations of each contiguous sample segment [offsets[k], offsets[k+1]) of one batch, k = 0 .. n_segments-1, in one call
+ * (information matrices of many candidate excitation trajectories, one system per recorded experiment, folds, time windows):
+ *   gram[k][P*P], rhs[k][P], tau_sq[k]   (P = 10*n_joints; contiguous, segment stride P*P / P / 1; tau_sq may be NULL)
+ * with the conventions of rdb_regressor_gram_batch (tau_meas [n_inputs][in->ld] or NULL = getJointTorque; accumulate != 0 adds).
+ * offsets: HOST array of n_segments + 1 int64, non-decreasing, 0 <= offsets[0], offsets[n_segments] <= in->n; read before return.
+ * An empty segment gets zeros (or is left unchanged when accumulate != 0).  Device pointers, asynchronous on `stream`.
+ * n_segments == 0 does nothing; n_segments < 0, offsets NULL, decreasing or outside [0, n], gram or rhs NULL: RDB_ERR_INVALID_ARG;
+ * samples without dq / ddq: RDB_ERR_DIM_MISMATCH.
+ * On chains the fused kernel takes (1 to 7 moving joints) every segment is cut into work items of 4 096 samples, one CTA each, and all
+ * segments run in a few launches; a segment's result depends on its own samples only, bit for bit, wherever it sits in the call.  Other
+ * chains (more than 7 moving joints, no moving joint) run the general pipeline once per segment: correct, but slow for short segments. */
+rdb_status rdb_regressor_gram_segmented_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, int64_t n_segments,
+                                              const int64_t* offsets, double* gram, double* rhs, double* tau_sq, int32_t accumulate,
+                                              void* stream);
+
 /* Chain::getWrench / Chain::getJointTorque(q,Dq,DDq,ext_wrenches_in_link_frame) (PI.h:1225-1274).
  * ext_wrenches[nL][6][ld_ext]: wrenches applied TO the links, in link frames, [force; torque] per link (NULL = none).  The reference
  * brings them to the base frame with the TWIST transform spatialTranformation(-ext, T_bl) (PI.h:1255, SA.h:193-197); mirrored
@@ -350,7 +365,9 @@ int32_t rdb_chain_device(const rdb_chain* chain);
  * (NVRTC) against the chain's own constants, 0 for the precompiled fused kernel (chains that are not all-revolute, NVRTC missing or failing,
  * RDB_GRAM_JIT=0), 2 for the general pipeline (materialised regressor and tiled contraction: more than 7 moving joints, no moving joint, or
  * a component set the one-pass kernel refuses), -1 before the first call.  reason (optional, reason_len bytes, NUL-terminated) says why, or
- * how long the compile took; for the general pipeline it starts with "general pipeline:". */
+ * how long the compile took; for the general pipeline it starts with "general pipeline:".  After rdb_regressor_gram_segmented_batch the
+ * reason of a fused run starts with "gram_fused_segmented_kernel, ", and that of a general-pipeline run with
+ * "general pipeline: one pass per segment". */
 rdb_status rdb_chain_gram_kernel_info(const rdb_chain* chain, int32_t* specialised, char* reason, int32_t reason_len);
 /* Host only, no device needed (inspection tools): the cubin of the run-time specialised kernel of an all-revolute chain, written to `path`.
  * kernel_args: the kernel and its template arguments without the model, e.g. "gram_fused_kernel<6, 4, true, 0"; arch e.g. "sm_100a". */

@@ -210,6 +210,15 @@ public:
   {
     check(rdb_regressor_gram_batch(m_h, &in, tau_meas, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
   }
+  // one normal-equation system per segment [offsets[k], offsets[k+1]) (rdb_regressor_gram_segmented_batch): gram[K][P*P], rhs[K][P],
+  // tau_sq[K] (or nullptr) on the device, K = offsets.size() - 1; offsets stay on the host
+  void getRegressorGramSegmented(const rdb_samples& in, const double* tau_meas, const std::vector<int64_t>& offsets, double* gram, double* rhs,
+                                 double* tau_sq, bool accumulate, void* stream = nullptr)
+  {
+    if (offsets.empty()) throw std::invalid_argument("offsets needs K + 1 entries");
+    check(rdb_regressor_gram_segmented_batch(m_h, &in, tau_meas, (int64_t)offsets.size() - 1, offsets.data(), gram, rhs, tau_sq,
+                                             accumulate ? 1 : 0, stream));
+  }
   // Chain::getWrench / getJointTorque(q,Dq,DDq,ext_wrenches_in_link_frame) (primitives_impl.h:1225-1274); ext [nL][6][ld_ext] or nullptr
   void getWrench(const rdb_samples& in, const double* ext_wrenches, int64_t ld_ext, double* torque, double* wrenches, int64_t ld_out, void* stream = nullptr)
   {

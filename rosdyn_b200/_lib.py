@@ -70,6 +70,8 @@ SYMBOLS = {
     "rdb_forward_dynamics_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, i64, ctypes.c_void_p, ctypes.c_void_p]),
     "rdb_forward_dynamics_batch_host": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, i64, ctypes.c_void_p]),
     "rdb_regressor_gram_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32, ctypes.c_void_p]),
+    "rdb_regressor_gram_segmented_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, i64, ctypes.POINTER(i64), _dp, _dp, _dp, i32,
+                                                 ctypes.c_void_p]),
     "rdb_wrench_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, i64, _dp, _dp, i64, ctypes.c_void_p]),
     "rdb_jacobian_link_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), i32, _dp, i64, ctypes.c_void_p]),
     "rdb_local_ik_batch": (i32, [ctypes.c_void_p, i64, i64, _dp, _dp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),

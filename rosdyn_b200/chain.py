@@ -513,6 +513,38 @@ class Chain:
             check(self._lib.rdb_regressor_gram_batch_host(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(G), _ptr(b), _ptr(tt), int(acc)))
         return G, b, tt
 
+    def regressorGramSegmented(self, q, Dq, DDq, offsets, tau_meas=None, out=None):
+        """Normal equations of each contiguous sample segment [offsets[k], offsets[k+1]) in one call: returns (G[K,P,P], b[K,P], tau_sq[K])
+        as torch CUDA tensors, K = len(offsets) - 1, with the conventions of regressorGram.  Device (torch CUDA) arrays only; offsets is a
+        host int sequence, non-decreasing, inside [0, N].  `out=(G,b,tau_sq)` accumulates into existing tensors of those shapes.
+        An empty segment gets zeros (is left unchanged when accumulating)."""
+        if Dq is None or DDq is None:
+            raise ValueError("Input data dimensions mismatch")
+        dev, single, n, arrs = self._prep([q, Dq, DDq, None])
+        if not dev:
+            raise ValueError("regressorGramSegmented takes device (torch CUDA) arrays")
+        tau_arr = None
+        if tau_meas is not None:
+            arrs, tau_arr = self._with_tau(dev, n, arrs, tau_meas)
+        offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+        if offs.size < 1:
+            raise ValueError("offsets needs at least one entry (K + 1 for K segments)")
+        K, P = offs.size - 1, 10 * self.nJ
+        acc = out is not None
+        if acc:
+            G, b, tt = out
+            if tuple(G.shape) != (K, P, P) or tuple(b.shape) != (K, P) or tuple(tt.shape) != (K,):
+                raise ValueError("out: need G[K,P,P], b[K,P], tau_sq[K]")
+        else:
+            dv = arrs[0].device
+            G = torch.empty((K, P, P), dtype=torch.float64, device=dv)
+            b = torch.empty((K, P), dtype=torch.float64, device=dv)
+            tt = torch.empty((K,), dtype=torch.float64, device=dv)
+        s = self._samples(n, arrs)
+        check(self._lib.rdb_regressor_gram_segmented_batch(self._h, ctypes.byref(s), _ptr(tau_arr), K,
+                                                            offs.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), _ptr(G), _ptr(b),
+                                                            _ptr(tt), int(acc), self._stream()))
+        return G, b, tt
 
     # ------------------------------------------------------------------ additive joint components (SURVEY.md 8f N2)
     def setComponents(self, components: Sequence[dict]) -> int:

@@ -258,6 +258,7 @@ void rdb_chain_destroy(rdb_chain* chain)
   if (chain->gram.fold_dev) cudaFree(chain->gram.fold_dev);
   if (chain->gram.ext_dev) cudaFree(chain->gram.ext_dev);
   if (chain->gram.tau_sq_part) cudaFree(chain->gram.tau_sq_part);
+  if (chain->gram.seg_dev) cudaFree(chain->gram.seg_dev);
   if (chain->host_arena.base) cudaFree(chain->host_arena.base);
   if (chain->host_arena.map_h) cudaFreeHost(chain->host_arena.map_h);
   if (chain->host_arena.pin) cudaFreeHost(chain->host_arena.pin);
@@ -439,6 +440,26 @@ rdb_status rdb_regressor_gram_batch(rdb_chain* chain, const rdb_samples* in, con
   if (in->n > 0 && (!in->dq || !in->ddq)) return fail(RDB_ERR_DIM_MISMATCH, "Input data dimensions mismatch");
   if (!gram || !rhs) return fail(RDB_ERR_INVALID_ARG, "gram / rhs must not be null");
   RDB_CUDA(launch_gram(*chain, to_dev(in), tau_meas, gram, rhs, tau_sq, accumulate, (cudaStream_t)stream));
+  return RDB_OK;
+}
+
+rdb_status rdb_regressor_gram_segmented_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, int64_t n_segments,
+                                              const int64_t* offsets, double* gram, double* rhs, double* tau_sq, int32_t accumulate,
+                                              void* stream)
+{
+  rdb_status s = check_samples(chain, in, true);
+  if (s != RDB_OK) return s;
+  if (n_segments < 0) return fail(RDB_ERR_INVALID_ARG, "n_segments must not be negative");
+  if (n_segments == 0) return RDB_OK;
+  if (!offsets) return fail(RDB_ERR_INVALID_ARG, "offsets must not be null");
+  if (offsets[0] < 0 || offsets[n_segments] > in->n) return fail(RDB_ERR_INVALID_ARG, "offsets must lie in [0, n]");
+  for (int64_t k = 0; k < n_segments; k++)
+    if (offsets[k + 1] < offsets[k]) return fail(RDB_ERR_INVALID_ARG, "offsets must not decrease");
+  if (!gram || !rhs) return fail(RDB_ERR_INVALID_ARG, "gram / rhs must not be null");
+  RDB_ENTER(chain);
+  RDB_LOCK(chain);  // as rdb_regressor_gram_batch: one Gram workspace per handle, ordered across streams by launch_gram_segmented
+  if (in->n > 0 && (!in->dq || !in->ddq)) return fail(RDB_ERR_DIM_MISMATCH, "Input data dimensions mismatch");
+  RDB_CUDA(launch_gram_segmented(*chain, to_dev(in), tau_meas, n_segments, offsets, gram, rhs, tau_sq, accumulate, (cudaStream_t)stream));
   return RDB_OK;
 }
 

@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <string>
 #include <vector>
 
 #include "launch.h"
@@ -193,6 +194,86 @@ __global__ void __launch_bounds__(256) gram_unfed_tau_sq_kernel(const double* __
   }
 }
 
+// segmented: one block per segment k (offsets on the device), the same fixed order per segment
+__global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const double* __restrict__ tau, int64_t ld,
+                                                                          const int64_t* __restrict__ offsets, int64_t nseg, UnfedRows u,
+                                                                          const double* __restrict__ part, double* __restrict__ tau_sq,
+                                                                          int accumulate)
+{
+  __shared__ double red[256];
+  for (int64_t k = blockIdx.x; k < nseg; k += gridDim.x)
+  {
+    const int64_t lo = offsets[k], hi = offsets[k + 1];
+    if (accumulate && lo == hi) continue;
+    double s = 0.0;
+    for (int r = 0; r < u.n; r++)
+      for (int64_t i = lo + threadIdx.x; i < hi; i += blockDim.x)
+      {
+        const double t = tau[(int64_t)u.row[r] * ld + i];
+        s = fma(t, t, s);
+      }
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int w = 128; w > 0; w >>= 1)
+    {
+      if ((int)threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
+      __syncthreads();
+    }
+    if (threadIdx.x == 0)
+    {
+      const double v = part[k] + red[0];
+      tau_sq[k] = accumulate ? tau_sq[k] + v : v;
+    }
+    __syncthreads();
+  }
+}
+
+// the inputs no chain joint feeds
+static UnfedRows unfed_rows(const ChainHost& ch)
+{
+  UnfedRows u{};
+  std::vector<char> fed(ch.host.n_in, 0);
+  for (int j = 0; j < ch.host.nj; j++)
+    if (ch.host.joint[j].in >= 0) fed[ch.host.joint[j].in] = 1;
+  for (int i = 0; i < ch.host.n_in; i++)
+    if (!fed[i]) u.row[u.n++] = i;
+  return u;
+}
+
+cudaError_t launch_unfed_tau_sq_segmented(const ChainHost& ch, const double* tau, int64_t ld, const int64_t* offsets, int64_t nseg,
+                                          const double* part, double* tau_sq, int accumulate, cudaStream_t st)
+{
+  if (nseg <= 0) return cudaSuccess;
+  gram_unfed_tau_sq_segmented_kernel<<<(unsigned)std::min<int64_t>(nseg, 65535), 256, 0, st>>>(tau, ld, offsets, nseg, unfed_rows(ch), part,
+                                                                                              tau_sq, accumulate);
+  count_launch();
+  return cudaGetLastError();
+}
+
+// rdb_chain_gram_kernel_info after a call on the general pipeline: why the fused kernels did not take it
+static std::string general_pipeline_why(const ChainHost& ch, bool force_v0, bool with_components)
+{
+  const int K = ch.gram.fold.nj;
+  if (force_v0) return "general pipeline: RDB_GRAM_IMPL=v0";
+  if (K > 7) return "general pipeline: more than 7 moving joints (" + std::to_string(K) + ")";
+  if (K < 1) return "general pipeline: no moving joint";
+  if (with_components)
+    return "general pipeline: a component set the one-pass kernel refuses (a component on an input no chain joint feeds, "
+           "or more than 8 component columns on one joint)";
+  return "general pipeline: the fused kernel does not take this chain";
+}
+
+// Development builds (-DRDB_DEV_SWITCHES, never the shipped library) can force the general pipeline with RDB_GRAM_IMPL=v0
+static bool gram_force_v0()
+{
+#ifdef RDB_DEV_SWITCHES
+  static const bool force_v0 = [] { const char* e = getenv("RDB_GRAM_IMPL"); return e && e[0] == 'v'; }();
+  return force_v0;
+#else
+  return false;
+#endif
+}
+
 static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                                  int accumulate, cudaStream_t st, bool with_components)
 {
@@ -209,13 +290,8 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
     return cudaGetLastError();
   }
   {
-    // fused warp-specialised kernel (gram_fused.cu) whenever the chain fits it.  Development builds (-DRDB_DEV_SWITCHES, never the shipped
-    // library) can force the general pipeline with RDB_GRAM_IMPL=v0
-#ifdef RDB_DEV_SWITCHES
-    static const bool force_v0 = [] { const char* e = getenv("RDB_GRAM_IMPL"); return e && e[0] == 'v'; }();
-#else
-    constexpr bool force_v0 = false;
-#endif
+    // fused warp-specialised kernel (gram_fused.cu) whenever the chain fits it
+    const bool force_v0 = gram_force_v0();
     if (!force_v0)
     {
       cudaError_t e = cudaErrorNotSupported;
@@ -234,28 +310,15 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
         e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
       if (e == cudaSuccess && unfed)
       {
-        UnfedRows u{};
-        std::vector<char> fed(n_in, 0);
-        for (int j = 0; j < ch.host.nj; j++)
-          if (ch.host.joint[j].in >= 0) fed[ch.host.joint[j].in] = 1;
-        for (int i = 0; i < n_in; i++)
-          if (!fed[i]) u.row[u.n++] = i;
-        gram_unfed_tau_sq_kernel<<<1, 256, 0, st>>>(tau_meas, in.ld, in.n, u, ts, tau_sq, accumulate);
+        gram_unfed_tau_sq_kernel<<<1, 256, 0, st>>>(tau_meas, in.ld, in.n, unfed_rows(ch), ts, tau_sq, accumulate);
         count_launch();
         e = cudaGetLastError();
       }
       if (e != cudaErrorNotSupported) return e;
     }
     // rdb_chain_gram_kernel_info describes the last Gram call: say that this one ran the general pipeline, and why
-    const int K = ch.gram.fold.nj;
     ch.gram.kernel_specialised = 2;
-    if (force_v0) ch.gram.kernel_why = "general pipeline: RDB_GRAM_IMPL=v0";
-    else if (K > 7) ch.gram.kernel_why = "general pipeline: more than 7 moving joints (" + std::to_string(K) + ")";
-    else if (K < 1) ch.gram.kernel_why = "general pipeline: no moving joint";
-    else if (P != Pr)
-      ch.gram.kernel_why = "general pipeline: a component set the one-pass kernel refuses (a component on an input no chain joint feeds, "
-                           "or more than 8 component columns on one joint)";
-    else ch.gram.kernel_why = "general pipeline: the fused kernel does not take this chain";
+    ch.gram.kernel_why = general_pipeline_why(ch, force_v0, P != Pr);
   }
   const int nblk = (P + 1 + BLK - 1) / BLK;
   const int npairs = nblk * (nblk + 1) / 2;
@@ -326,6 +389,48 @@ cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_m
   if (e != cudaSuccess) return e;
   e = gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components);
   const cudaError_t r = cudaEventRecord(ch.gram.done, st);  // also after a failed launch: whatever was queued stays ordered
+  return e != cudaSuccess ? e : r;
+}
+
+static cudaError_t gram_segmented_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,
+                                           double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
+{
+  const int64_t P = 10 * ch.host.nj;
+  const bool force_v0 = gram_force_v0();
+  if (!force_v0 && ch.host.n_in > 0 && P > 0)
+  {
+    const bool unfed = tau_meas && tau_sq && !ch.inputs_cover_all;
+    const cudaError_t e = launch_gram_fused_segmented(ch, in, tau_meas, nseg, offsets, gram, rhs, tau_sq, accumulate, unfed, st);
+    if (e != cudaErrorNotSupported) return e;
+  }
+  // the general pipeline, one pass per segment: correct for every chain, slow for many short segments.  ch.gram.done is recorded behind
+  // every segment, so that a workspace which grows for a longer segment is freed only once the segments before it are done with it
+  for (int64_t k = 0; k < nseg; k++)
+  {
+    const int64_t lo = offsets[k], hi = offsets[k + 1];
+    auto at = [&](const double* p) { return p ? p + lo : nullptr; };
+    const SamplesDev v{hi - lo, in.ld, at(in.q), at(in.dq), at(in.ddq), nullptr};
+    cudaError_t e = gram_launches(ch, v, at(tau_meas), gram + k * P * P, rhs + k * P, tau_sq ? tau_sq + k : nullptr, accumulate, st, false);
+    if (e != cudaSuccess) return e;
+    e = cudaEventRecord(ch.gram.done, st);
+    if (e != cudaSuccess) return e;
+  }
+  ch.gram.kernel_specialised = 2;
+  ch.gram.kernel_why = "general pipeline: one pass per segment (slow for short segments); " +
+                       general_pipeline_why(ch, force_v0, false).substr(sizeof("general pipeline: ") - 1);
+  return cudaSuccess;
+}
+
+// ordered like launch_gram
+cudaError_t launch_gram_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets, double* gram,
+                                  double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
+{
+  cudaError_t e = ch.gram.done ? cudaSuccess : cudaEventCreateWithFlags(&ch.gram.done, cudaEventDisableTiming);
+  if (e != cudaSuccess) return e;
+  e = cudaStreamWaitEvent(st, ch.gram.done, 0);
+  if (e != cudaSuccess) return e;
+  e = gram_segmented_launches(ch, in, tau_meas, nseg, offsets, gram, rhs, tau_sq, accumulate, st);
+  const cudaError_t r = cudaEventRecord(ch.gram.done, st);
   return e != cudaSuccess ? e : r;
 }
 

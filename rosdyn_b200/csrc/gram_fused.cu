@@ -18,12 +18,11 @@ namespace rdb
 // column-major), rhs, tau_sq.  One thread per partial entry, and per entry of the P x (P + 1) output: the parameter columns without a position
 // (identically zero columns of Phi, GramGeom::has_pos) get exact zeros in their row, column and rhs.
 template <int NJ, int Z>
-__global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int nparts, int pstride, double* __restrict__ gram,
-                                         double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
+__device__ __forceinline__ void gram_fused_reduce_entry(int e, const double* __restrict__ partial, int nparts, int pstride, double* __restrict__ gram,
+                                                        double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
 {
   using G = GramGeom<NJ, Z>;
   constexpr int P = G::P;
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (!accumulate && e < P * (P + 1))
   {
     const int c = e / (P + 1), r = e % (P + 1);  // r == P: rhs
@@ -80,6 +79,25 @@ __global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int
     *tau_sq = accumulate ? *tau_sq + s : s;
 }
 template <int NJ, int Z>
+__global__ void gram_fused_reduce_kernel(const double* __restrict__ partial, int nparts, int pstride, double* __restrict__ gram,
+                                         double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
+{
+  gram_fused_reduce_entry<NJ, Z>(blockIdx.x * blockDim.x + threadIdx.x, partial, nparts, pstride, gram, rhs, tau_sq, accumulate);
+}
+// segmented: blockIdx.y is row y of the wave's segment table (rows[3 y ..]: first item of the wave, item count, segment), which sums its
+// items' partials in item order.  Output o = the segment (by_segment) or y, at gram + o gstride, rhs + o rstride, tau_sq + o tstride.  A row
+// without items writes zeros (the host lists empty segments only when the call does not accumulate).
+template <int NJ, int Z>
+__global__ void gram_fused_reduce_segmented_kernel(const double* __restrict__ partial, const int64_t* __restrict__ rows, int pstride,
+                                                   double* __restrict__ gram, double* __restrict__ rhs, double* __restrict__ tau_sq,
+                                                   int64_t gstride, int64_t rstride, int64_t tstride, int by_segment, int accumulate)
+{
+  const int64_t* r = rows + 3 * (int64_t)blockIdx.y;
+  const int64_t o = by_segment ? r[2] : (int64_t)blockIdx.y;
+  gram_fused_reduce_entry<NJ, Z>(blockIdx.x * blockDim.x + threadIdx.x, partial + r[0] * pstride, (int)r[1], pstride, gram + o * gstride,
+                                 rhs + o * rstride, tau_sq ? tau_sq + o * tstride : nullptr, accumulate);
+}
+template <int NJ, int Z>
 static void launch_fused_reduce(const double* partial, int nparts, int pstride, double* gram, double* rhs, double* tau_sq, int accumulate,
                                 cudaStream_t st)
 {
@@ -90,12 +108,12 @@ static void launch_fused_reduce(const double* partial, int nparts, int pstride, 
 }
 
 // G = E^T G' E, b = E^T b' (upper triangle computed, mirrored): one thread per entry of the full matrix, 100 products each
-__global__ void gram_fold_expand_kernel(const double* __restrict__ T, const int32_t* __restrict__ kof, const double* __restrict__ Gr,
-                                        const double* __restrict__ br, const double* __restrict__ tsr, int nj, int Pr, double* __restrict__ gram,
-                                        double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
+__device__ __forceinline__ void gram_fold_expand_entry(int e, const double* __restrict__ T, const int32_t* __restrict__ kof,
+                                                       const double* __restrict__ Gr, const double* __restrict__ br, const double* __restrict__ tsr,
+                                                       int nj, int Pr, double* __restrict__ gram, double* __restrict__ rhs,
+                                                       double* __restrict__ tau_sq, int accumulate)
 {
   const int P = 10 * nj;
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= P * (P + 1)) return;
   const int a = e / (P + 1), b = e % (P + 1);  // b == P: right-hand side
   if (e == P && tau_sq) *tau_sq = accumulate ? *tau_sq + *tsr : *tsr;
@@ -120,6 +138,23 @@ __global__ void gram_fold_expand_kernel(const double* __restrict__ T, const int3
   const double v = accumulate ? gram[(size_t)b * P + a] + s : s;
   gram[(size_t)b * P + a] = v;
   if (a != b) gram[(size_t)a * P + b] = v;
+}
+__global__ void gram_fold_expand_kernel(const double* __restrict__ T, const int32_t* __restrict__ kof, const double* __restrict__ Gr,
+                                        const double* __restrict__ br, const double* __restrict__ tsr, int nj, int Pr, double* __restrict__ gram,
+                                        double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
+{
+  gram_fold_expand_entry(blockIdx.x * blockDim.x + threadIdx.x, T, kof, Gr, br, tsr, nj, Pr, gram, rhs, tau_sq, accumulate);
+}
+// segmented: blockIdx.y is row y of the wave's segment table; its reduced equations sit at red + y rstride (G' | b' | tau_sq), its output
+// is segment rows[3 y + 2] of gram / rhs / tau_sq
+__global__ void gram_fold_expand_segmented_kernel(const double* __restrict__ T, const int32_t* __restrict__ kof, const double* __restrict__ red,
+                                                  int64_t rstride, const int64_t* __restrict__ rows, int nj, int Pr, double* __restrict__ gram,
+                                                  double* __restrict__ rhs, double* __restrict__ tau_sq, int accumulate)
+{
+  const int64_t P = 10 * nj, k = rows[3 * (int64_t)blockIdx.y + 2];
+  const double* Gr = red + (int64_t)blockIdx.y * rstride;
+  gram_fold_expand_entry(blockIdx.x * blockDim.x + threadIdx.x, T, kof, Gr, Gr + (size_t)Pr * Pr, Gr + (size_t)Pr * Pr + Pr, nj, Pr,
+                         gram + k * P * P, rhs + k * P, tau_sq ? tau_sq + k : nullptr, accumulate);
 }
 
 // Timing experiments (1: skip the generation, 2: skip the MMA) exist in development builds only (-DRDB_DEV_SWITCHES); the shipped library
@@ -192,18 +227,22 @@ constexpr int gf_slots()
 // gram_fused_kernel on the folded chain, one per-CTA partial (gram_partial_doubles) each into `partials`: *grid CTAs.  On REV chains the
 // kernel is the one specialised at run time to the chain's constants when it can be built (gram_jit.cpp), else the precompiled
 // instantiation; other chains always run the precompiled generic kernel.
-template <int NJ, bool REV, int XC>
+// SEG: gram_fused_segmented_kernel instead, one CTA per work item of items[0 .. 2 *grid) (device table of start, length).
+template <int NJ, bool REV, int XC, bool SEG = false>
 static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const SamplesDev& in, const double* tau_meas, double* partials,
-                                       int* grid, cudaStream_t st)
+                                       int* grid, cudaStream_t st, const int64_t* items = nullptr)
 {
   constexpr int Z = REV ? (XC ? 1 : 2) : 0;  // as in the kernel
   constexpr int SLOTS = gf_slots<NJ, Z, XC>();
   static_assert(SLOTS >= 2, "the fused kernel needs two slots");
-  const void* kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, XC>);
+  const char* name = SEG ? "gram_fused_segmented_kernel" : "gram_fused_kernel";
+  const void* kfn = nullptr;
+  if constexpr (SEG) kfn = reinterpret_cast<const void*>(gram_fused_segmented_kernel<NJ, SLOTS, REV, XC>);
+  else kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, XC>);
   if (REV)
   {
     char args[64];
-    snprintf(args, sizeof args, "gram_fused_kernel<%d, %d, true, %d", NJ, SLOTS, XC);
+    snprintf(args, sizeof args, "%s<%d, %d, true, %d", name, NJ, SLOTS, XC);
     if (const void* jk = gram_jit_kernel(ch, args)) kfn = jk;
   }
   else
@@ -211,20 +250,26 @@ static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const
     ch.gram.kernel_specialised = 0;
     ch.gram.kernel_why = "precompiled kernel: not every folded joint is revolute about e_z (generic generator)";
   }
+  if (SEG) ch.gram.kernel_why = std::string(name) + ", " + ch.gram.kernel_why;  // rdb_chain_gram_kernel_info names the segmented kernel
   const size_t smem = sizeof(double) * (size_t)gram_smem_doubles<NJ, Z, SLOTS, XC>();
   cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  const int64_t ngroups = (in.n + 31) / 32;
-  constexpr int B = gram_group_block<SLOTS, XC>();
-  *grid = (int)std::min<int64_t>(ch.sm_count, (ngroups + B - 1) / B);
+  if (!SEG)
+  {
+    const int64_t ngroups = (in.n + 31) / 32;
+    constexpr int B = gram_group_block<SLOTS, XC>();
+    *grid = (int)std::min<int64_t>(ch.sm_count, (ngroups + B - 1) / B);
+  }
   ChainDev<NJ> C = narrow_g<NJ>(ch.gram.fold);
   GramComps comps = gc;
   SamplesDev ins = in;
   const double* tm = tau_meas;
+  const int64_t* it = items;
   double* part = partials;
   int dbg = gram_dev_switch();
-  void* args[] = {&C, &comps, &ins, &tm, &part, &dbg};
-  e = cudaLaunchKernel(kfn, dim3(*grid), dim3(GF_THREADS), args, smem, st);
+  void* args_whole[] = {&C, &comps, &ins, &tm, &part, &dbg};
+  void* args_seg[] = {&C, &comps, &ins, &tm, &it, &part, &dbg};
+  e = cudaLaunchKernel(kfn, dim3(*grid), dim3(GF_THREADS), SEG ? args_seg : args_whole, smem, st);
   if (e != cudaSuccess) return e;
   count_launch();
   return cudaSuccess;
@@ -268,6 +313,166 @@ cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double*
   case N:                                                                                     \
     return rev ? launch_fused_nj<N, true>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st) \
                : launch_fused_nj<N, false>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
+    X(1) X(2) X(3) X(4) X(5) X(6) X(7)
+#undef X
+  }
+  return cudaErrorNotSupported;
+}
+
+// ---------------------------------------------------------------------------------------------- segmented normal equations
+// Work items: every segment is cut, from its start, into items of `item` samples (the last one short); each item is one CTA of
+// gram_fused_segmented_kernel.  The items run in waves of at most `wave` items and `wave` segment rows, so the workspace of partials is
+// bounded by the wave, not by the number of segments.  A wave holds whole segments; a segment of more than `wave` items runs alone over
+// ceil(items / wave) waves, each one after the first added into its output.  Both cuts depend on the segment's length alone, and every sum runs
+// in item order, so a segment's result depends on its own samples only, bit for bit, wherever it sits in the call.
+// Chosen by measurement on a B200 (tools/bench_gram_segmented.py, profiles/gram_segmented_bench*.json, DESIGN.md 3.3.1): 128 groups (4 096
+// samples) per item, 8 items per SM per wave.  The environment variables RDB_GRAM_SEG_ITEM_GROUPS and RDB_GRAM_SEG_WAVE_PER_SM override
+// them for such measurements; results are reproducible for a given setting.
+constexpr int GF_SEG_ITEM_GROUPS = 128;
+constexpr int GF_SEG_WAVE_PER_SM = 8;
+
+static int64_t seg_knob(const char* env, int64_t dflt, int64_t hi)
+{
+  const char* e = getenv(env);
+  const long long v = e && *e ? atoll(e) : 0;
+  return v >= 1 && v <= hi ? (int64_t)v : dflt;
+}
+
+struct SegPlan
+{
+  struct Wave
+  {
+    int64_t item0, nitems, row0, nrows;
+    int accumulate;
+  };
+  std::vector<Wave> waves;
+  std::vector<int64_t> tab;  // offsets [K + 1] | items (start, length) | rows (first item in the wave, items, segment)
+  int64_t nitems = 0, max_rows = 0, wave = 0;
+};
+
+static SegPlan plan_segments(int64_t nseg, const int64_t* offsets, int64_t item, int64_t wave, int accumulate)
+{
+  SegPlan p;
+  p.wave = wave;
+  std::vector<int64_t> items, rows;
+  SegPlan::Wave cur{0, 0, 0, 0, accumulate};
+  auto flush = [&] {
+    if (cur.nitems || cur.nrows) p.waves.push_back(cur);
+    p.max_rows = std::max(p.max_rows, cur.nrows);
+    cur = SegPlan::Wave{(int64_t)items.size() / 2, 0, (int64_t)rows.size() / 3, 0, accumulate};
+  };
+  auto add_items = [&](int64_t lo, int64_t hi, int64_t i0, int64_t ni) {
+    for (int64_t i = i0; i < i0 + ni; i++)
+    {
+      items.push_back(lo + i * item);
+      items.push_back(std::min(item, hi - lo - i * item));
+    }
+  };
+  for (int64_t k = 0; k < nseg; k++)
+  {
+    const int64_t lo = offsets[k], hi = offsets[k + 1], ni = (hi - lo + item - 1) / item;
+    if (ni > wave)  // alone, over several waves
+    {
+      flush();
+      for (int64_t w0 = 0; w0 < ni; w0 += wave)
+      {
+        const int64_t nw = std::min(wave, ni - w0);
+        rows.insert(rows.end(), {0, nw, k});
+        add_items(lo, hi, w0, nw);
+        cur.nitems = nw;
+        cur.nrows = 1;
+        cur.accumulate = w0 ? 1 : accumulate;
+        flush();
+      }
+      continue;
+    }
+    if (ni == 0 && accumulate) continue;  // an empty segment is left as it is
+    if (cur.nitems + ni > wave || cur.nrows == wave) flush();
+    rows.insert(rows.end(), {cur.nitems, ni, k});  // an empty segment: a row without items, which writes zeros
+    add_items(lo, hi, 0, ni);
+    cur.nitems += ni;
+    cur.nrows++;
+  }
+  flush();
+  p.nitems = (int64_t)items.size() / 2;
+  p.tab.assign(offsets, offsets + nseg + 1);
+  p.tab.insert(p.tab.end(), items.begin(), items.end());
+  p.tab.insert(p.tab.end(), rows.begin(), rows.end());
+  return p;
+}
+
+template <int NJ, bool REV>
+static cudaError_t launch_fused_segmented_nj(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const SegPlan& plan,
+                                             double* gram, double* rhs, double* tau_sq, int accumulate, bool unfed, cudaStream_t st)
+{
+  constexpr int Z = REV ? 2 : 0;  // as in the kernel
+  using G = GramGeom<NJ, Z>;
+  const int nj = ch.host.nj, Pr = G::P, P = 10 * nj;
+  const bool fold = !ch.gram.fold_identity;
+  // workspace: per-item partials of one wave | (folded chain) reduced equations G' | b' | tau_sq of each row of a wave | (unfed) the fused
+  // tau^T tau of every segment | the plan's table
+  const int64_t RS = (int64_t)Pr * Pr + Pr + 1;
+  const size_t n_part = (size_t)plan.wave * G::PARTIAL, n_red = fold ? (size_t)plan.max_rows * RS : 0, n_ts = unfed ? (size_t)nseg : 0;
+  cudaError_t e = grow(ch.gram.seg_dev, ch.gram.seg_bytes, sizeof(double) * (n_part + n_red + n_ts) + sizeof(int64_t) * plan.tab.size(),
+                       ch.gram.done);
+  if (e != cudaSuccess) return e;
+  double* part = ch.gram.seg_dev;
+  double* red = part + n_part;
+  double* ts = red + n_red;
+  int64_t* tab = reinterpret_cast<int64_t*>(ts + n_ts);
+  e = cudaMemcpyAsync(tab, plan.tab.data(), sizeof(int64_t) * plan.tab.size(), cudaMemcpyHostToDevice, st);  // pageable: staged before return
+  if (e != cudaSuccess) return e;
+  const int64_t* items = tab + nseg + 1;
+  const int64_t* rows = items + 2 * plan.nitems;
+  if (unfed) cudaMemsetAsync(ts, 0, sizeof(double) * nseg, st);
+  double* tso = unfed ? ts : tau_sq;
+  const double* Tm = ch.gram.fold_dev;
+  const int32_t* kof = reinterpret_cast<const int32_t*>(ch.gram.fold_dev + (size_t)nj * 100 + (size_t)(Pr + 1) * (Pr + 1));
+  const int nred = std::max(G::PARTIAL, Pr * (Pr + 1));
+  for (const SegPlan::Wave& w : plan.waves)
+  {
+    if (w.nitems)
+    {
+      int grid = (int)w.nitems;
+      e = launch_fused_kernel<NJ, REV, 0, true>(ch, GramComps{}, in, tau_meas, part, &grid, st, items + 2 * w.item0);
+      if (e != cudaSuccess) return e;
+    }
+    const int64_t* wr = rows + 3 * w.row0;
+    const dim3 rg((nred + 255) / 256, (unsigned)w.nrows);
+    if (!fold)
+      gram_fused_reduce_segmented_kernel<NJ, Z><<<rg, 256, 0, st>>>(part, wr, G::PARTIAL, gram, rhs, tso, (int64_t)P * P, P, 1, 1, w.accumulate);
+    else
+    {
+      gram_fused_reduce_segmented_kernel<NJ, Z><<<rg, 256, 0, st>>>(part, wr, G::PARTIAL, red, red + (size_t)Pr * Pr, red + (size_t)Pr * Pr + Pr,
+                                                                    RS, RS, RS, 0, 0);
+      count_launch();
+      gram_fold_expand_segmented_kernel<<<dim3((P * (P + 1) + 127) / 128, (unsigned)w.nrows), 128, 0, st>>>(Tm, kof, red, RS, wr, nj, Pr, gram, rhs,
+                                                                                                             tso, w.accumulate);
+    }
+    count_launch();
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+  }
+  if (unfed) return launch_unfed_tau_sq_segmented(ch, tau_meas, in.ld, tab, nseg, ts, tau_sq, accumulate, st);
+  return cudaSuccess;
+}
+
+// returns cudaErrorNotSupported when the chain does not fit the fused kernel (caller runs the general pipeline per segment).  unfed: measured
+// torques also sit on inputs no chain joint feeds (their squares join tau_sq per segment, launch_unfed_tau_sq_segmented)
+cudaError_t launch_gram_fused_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,
+                                        double* gram, double* rhs, double* tau_sq, int accumulate, bool unfed, cudaStream_t st)
+{
+  if (ch.gram.fold_version != ch.model_version || ch.gram.fold.nj < 1 || ch.gram.fold.nj > 7) return cudaErrorNotSupported;
+  const int64_t item = 32 * seg_knob("RDB_GRAM_SEG_ITEM_GROUPS", GF_SEG_ITEM_GROUPS, 1 << 20);
+  const int64_t wave = ch.sm_count * seg_knob("RDB_GRAM_SEG_WAVE_PER_SM", GF_SEG_WAVE_PER_SM, 65535 / std::max(ch.sm_count, 1));
+  const SegPlan plan = plan_segments(nseg, offsets, item, wave, accumulate);
+  const bool rev = fold_rev_canonical(ch.gram.fold);
+  switch (ch.gram.fold.nj)
+  {
+#define X(N)                                                                                                            \
+  case N:                                                                                                               \
+    return rev ? launch_fused_segmented_nj<N, true>(ch, in, tau_meas, nseg, plan, gram, rhs, tau_sq, accumulate, unfed, st) \
+               : launch_fused_segmented_nj<N, false>(ch, in, tau_meas, nseg, plan, gram, rhs, tau_sq, accumulate, unfed, st);
     X(1) X(2) X(3) X(4) X(5) X(6) X(7)
 #undef X
   }

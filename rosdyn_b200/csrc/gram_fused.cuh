@@ -123,6 +123,20 @@ __device__ __forceinline__ int64_t gram_cta_groups(int64_t ngroups)
   const int64_t q = (nb - 1 - blockIdx.x) / gridDim.x;  // the last block of this CTA
   return q * B + min((int64_t)B, ngroups - (q * gridDim.x + blockIdx.x) * B);
 }
+// Which groups a CTA takes, chosen at compile time by the kernel: WIN = false, the CTA-strided walk above over the whole batch
+// (gram_fused_kernel); WIN = true, every group of `in` in order (gram_fused_segmented_kernel hands each CTA its own window as `in`)
+template <int B, bool WIN>
+__device__ __forceinline__ int64_t gram_role_groups(int64_t ngroups)
+{
+  if constexpr (WIN) return ngroups;
+  else return gram_cta_groups<B>(ngroups);
+}
+template <int B, bool WIN>
+__device__ __forceinline__ int64_t gram_role_group(int64_t k)
+{
+  if constexpr (WIN) return k;
+  else return gram_group<B>(k);
+}
 
 // ---------------------------------------------------------------------------------------------- extended model [Phi | Phi_c]
 // The component columns of a joint -- element-wise functions of that joint's q, Dq (friction_polynomial1.h:45-52, friction_polynomial2.h:42-58,
@@ -210,19 +224,19 @@ __host__ __device__ constexpr int gram_smem_doubles()
 }
 
 // ---------------------------------------------------------------------------------------------- generator side
-template <int NJ, int SLOTS, bool REV, int Z, int XC, class M>
+template <int NJ, int SLOTS, bool REV, int Z, int XC, class M, bool WIN = false>
 __device__ __forceinline__ void gram_gen_role(const ChainDev<NJ>& C, const GramComps& comps, const SamplesDev& in, const double* __restrict__ tau_meas,
                                               double* smem, double* side0, GramBars* bars, int w, int lane, int dbg)
 {
   using G = GramGeom<NJ, Z>;
   constexpr int B = gram_group_block<SLOTS, XC>();
-  const int64_t nk = gram_cta_groups<B>((in.n + 31) / 32);
+  const int64_t nk = gram_role_groups<B, WIN>((in.n + 31) / 32);
   for (int64_t k = w; k < nk; k += GF_GENS)
   {
     const int s = (int)(k % SLOTS);
     const uint32_t u = (uint32_t)(k / SLOTS);
     // the inputs are requested BEFORE waiting for the slot: the DRAM latency hides behind the consumers' work on the previous group
-    const int64_t i = gram_group<B>(k) * 32 + lane;
+    const int64_t i = gram_role_group<B, WIN>(k) * 32 + lane;
     GenIn<NJ> cur;
     gen_load<NJ>(C, in, min(i, in.n - 1), cur);
     trig_all<NJ>(cur.q, cur.sv, cur.cv);
@@ -446,7 +460,7 @@ __device__ __forceinline__ void gram_cross_reduce_smem(double (&xacc)[NX][2], do
   }
 }
 
-template <int NJ, int SLOTS, int PAR, int Z, int XC>
+template <int NJ, int SLOTS, int PAR, int Z, int XC, bool WIN = false>
 __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem, const double* side0, GramBars* bars, int ks, int lane, int dbg)
 {
   using G = GramGeom<NJ, Z>;
@@ -459,7 +473,7 @@ __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem
   for (int k = 0; k < NB; k++) bacc[k] = 0.0;
 #pragma unroll
   for (int k = 0; k < NX; k++) xacc[k][0] = xacc[k][1] = 0.0;
-  const int64_t nk = gram_cta_groups<B>((in.n + 31) / 32);
+  const int64_t nk = gram_role_groups<B, WIN>((in.n + 31) / 32);
 #pragma unroll 1
   for (int64_t k = 0; k < nk; k++)
   {
@@ -533,6 +547,63 @@ __global__ void __launch_bounds__(GF_THREADS, 1)
   const int mma_id = warp, ks = mma_id % GF_KSPLIT;
   if (mma_id < GF_KSPLIT) gram_mma_role<NJ, SLOTS, 0, Z, XC>(in, smem, side0, &bars, ks, lane, dbg);
   else gram_mma_role<NJ, SLOTS, 1, Z, XC>(in, smem, side0, &bars, ks, lane, dbg);
+  double* out = partial + (size_t)blockIdx.x * NOUT;
+  for (int k = mma_id * 32 + lane; k < NOUT; k += 32 * GF_MMA_WARPS) out[k] = smem[k];
+}
+
+// Segmented normal equations (rdb_regressor_gram_segmented_batch): CTA b owns work item b, the window [items[2 b], + items[2 b + 1]) of the
+// batch, which lies inside one segment.  The roles see that window as their batch (plane pointers and tau_meas offset to its start, n = its
+// length: ld_in loads by plane stride, so nothing else moves), take its groups in order (WIN), and clamp and zero lanes at its end.  The
+// partial of item b goes to partial + b NOUT, in the layout of gram_fused_kernel; gram_fused.cu sums the items of a segment in item order.
+// Otherwise this is gram_fused_kernel line for line.  The two do not share a device function for the body: with one more inline level
+// ptxas derived other known bits of the lane index and the extended instantiations of gram_fused_kernel compiled to different instructions.
+template <int NJ, int SLOTS, bool REV, int XC = 0, class M = RtModel>
+__global__ void __launch_bounds__(GF_THREADS, 1)
+    gram_fused_segmented_kernel(const __grid_constant__ ChainDev<NJ> C, const __grid_constant__ GramComps comps, const SamplesDev in,
+                                const double* __restrict__ tau_meas, const int64_t* __restrict__ items, double* __restrict__ partial,
+                                const int dbg)
+{
+  constexpr int Z = REV ? (XC ? 1 : 2) : 0;
+  constexpr int NOUT = gram_partial_doubles<NJ, Z, XC>();
+  extern __shared__ __align__(16) double smem[];
+  __shared__ GramBars bars;
+  // the window lives in shared memory, not in registers: the roles reread it where the unsegmented kernel rereads its parameters
+  __shared__ SamplesDev win;
+  __shared__ const double* tm;
+  double* const side0 = smem + gram_side_offset<NJ, Z, SLOTS, XC>();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 32)
+  {
+    const int64_t s0 = items[2 * (int64_t)blockIdx.x];
+    win = SamplesDev{items[2 * (int64_t)blockIdx.x + 1], in.ld, in.q + s0, in.dq + s0, in.ddq + s0, nullptr};
+    tm = tau_meas ? tau_meas + s0 : nullptr;
+  }
+  if constexpr (gram_group_block<SLOTS, XC>() == SLOTS)
+  {
+    if (threadIdx.x == 0)
+    {
+      for (int s = 0; s < SLOTS; s++)
+      {
+        mbarrier_init(&bars.full[s], 1);
+        mbarrier_init(&bars.empty[s], GF_MMA_WARPS);
+      }
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+  }
+  else if (threadIdx.x < SLOTS)
+  {
+    bars.filled[threadIdx.x] = 0;
+    bars.drained[threadIdx.x] = 0;
+  }
+  __syncthreads();
+  if (warp >= GF_MMA_WARPS)
+  {
+    gram_gen_role<NJ, SLOTS, REV, Z, XC, M, true>(C, comps, win, tm, smem, side0, &bars, warp - GF_MMA_WARPS, lane, dbg);
+    return;
+  }
+  const int mma_id = warp, ks = mma_id % GF_KSPLIT;
+  if (mma_id < GF_KSPLIT) gram_mma_role<NJ, SLOTS, 0, Z, XC, true>(win, smem, side0, &bars, ks, lane, dbg);
+  else gram_mma_role<NJ, SLOTS, 1, Z, XC, true>(win, smem, side0, &bars, ks, lane, dbg);
   double* out = partial + (size_t)blockIdx.x * NOUT;
   for (int k = mma_id * 32 + lane; k < NOUT; k += 32 * GF_MMA_WARPS) out[k] = smem[k];
 }

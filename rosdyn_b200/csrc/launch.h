@@ -28,6 +28,8 @@ struct GramWorkspace
   double* ext_dev = nullptr;   // extended model: rigid-body block | cross-tile sums | cross partials | component map
   size_t ext_bytes = 0;
   double* tau_sq_part = nullptr;  // gram.cu: the fused kernels' tau^T tau when measured torques also sit on inputs no chain joint feeds
+  double* seg_dev = nullptr;  // gram_fused.cu, segmented calls: item partials of a wave | reduced rows | per-segment tau^T tau | item table
+  size_t seg_bytes = 0;
   // recorded after the last launch of every Gram call (launch_gram): the next call's stream waits for it before it touches the buffers
   // above, so the Gram calls of one handle run their device work in call order whatever streams they come on; a buffer is freed only
   // once it has completed
@@ -180,6 +182,18 @@ bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, 
 // gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
                               int accumulate, cudaStream_t st);
+// gram.cu: the normal equations of every segment [offsets[k], offsets[k + 1]) of the batch (host offsets, k < nseg), segment k at gram + k P P,
+// rhs + k P, tau_sq + k; fused segmented kernel when the chain fits it, else the general pipeline once per segment.  Ordered like launch_gram.
+cudaError_t launch_gram_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets, double* gram,
+                                  double* rhs, double* tau_sq, int accumulate, cudaStream_t st);
+// gram_fused.cu: the fused part of the above; cudaErrorNotSupported when the chain does not fit the fused kernel.  unfed: tau_sq gets the
+// measured torques of the inputs no chain joint feeds too (launch_unfed_tau_sq_segmented)
+cudaError_t launch_gram_fused_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,
+                                        double* gram, double* rhs, double* tau_sq, int accumulate, bool unfed, cudaStream_t st);
+// gram.cu: tau_sq[k] = (accumulate ? tau_sq[k] : 0) + part[k] + the squares of the measured torques of the inputs no chain joint feeds over
+// segment k (device offsets [nseg + 1]); an empty segment is left as it is when accumulating
+cudaError_t launch_unfed_tau_sq_segmented(const ChainHost& ch, const double* tau, int64_t ld, const int64_t* offsets, int64_t nseg,
+                                          const double* part, double* tau_sq, int accumulate, cudaStream_t st);
 // gram_fused.cu: G = E^T G' E, b = E^T b' from the reduced (folded-chain) normal equations kept in ch.gram.fold_dev
 cudaError_t launch_fold_expand(ChainHost& ch, double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st);
 // same for the extended model [Phi | Phi_c] (gram is Pt x Pt, Pt = 10 nJ + component columns)
