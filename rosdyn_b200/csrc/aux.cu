@@ -156,21 +156,6 @@ __global__ void __launch_bounds__(64) aux_kernel_generic(const ChainDev<RDB_MAX_
   aux_body<RDB_MAX_JOINTS>(*C, in, o, i);
 }
 
-template <int NJ>
-static ChainDev<NJ> narrow_a(const ChainDev<RDB_MAX_JOINTS>& h)
-{
-  ChainDev<NJ> c;
-  c.nj = h.nj;
-  c.n_in = h.n_in;
-  for (int k = 0; k < 3; k++) c.g[k] = h.g[k];
-  for (int j = 0; j < NJ; j++)
-  {
-    c.joint[j] = h.joint[j];
-    c.link[j] = h.link[j];
-  }
-  return c;
-}
-
 cudaError_t launch_aux(const ChainHost& ch, const SamplesDev& in, const double* ext, int64_t ld_ext, double* torque, double* wrenches,
                        double* jac_link, int link, int64_t ld_out, cudaStream_t st)
 {
@@ -180,9 +165,9 @@ cudaError_t launch_aux(const ChainHost& ch, const SamplesDev& in, const double* 
     for (int j = 0; j < link && j < ch.host.nj; j++)
       if (ch.host.joint[j].in >= 0) o.k_before++;
   if (ch.host.nj <= 8)
-    aux_kernel<8><<<(unsigned)((in.n + 127) / 128), 128, 0, st>>>(narrow_a<8>(ch.host), in, o);
+    aux_kernel<8><<<(unsigned)((in.n + 127) / 128), 128, 0, st>>>(narrow<8>(ch.host), in, o);
   else
-    aux_kernel_generic<<<(unsigned)((in.n + 63) / 64), 64, 0, st>>>(ch.dev, in, o);
+    aux_kernel_generic<<<(unsigned)((in.n + 63) / 64), 64, 0, st>>>(ch.dev.get(), in, o);
   count_launch();
   return cudaGetLastError();
 }

@@ -135,8 +135,8 @@ static rdb_status build_model(const rdb_chain_desc* d, ChainHost* ch)
 static rdb_status upload_model(ChainHost* ch)
 {
   RDB_CUDA(cudaDeviceSynchronize());
-  if (!ch->dev) RDB_CUDA(cudaMalloc(&ch->dev, sizeof(ch->host)));
-  RDB_CUDA(cudaMemcpy(ch->dev, &ch->host, sizeof(ch->host), cudaMemcpyHostToDevice));
+  RDB_CUDA(ch->dev.grow(sizeof(ch->host), nullptr));
+  RDB_CUDA(cudaMemcpy(ch->dev.get(), &ch->host, sizeof(ch->host), cudaMemcpyHostToDevice));
   cudaDeviceGetAttribute(&ch->sm_count, cudaDevAttrMultiProcessorCount, ch->device);
   ch->model_version++;
   RDB_CUDA(fold_chain(*ch));
@@ -238,7 +238,6 @@ rdb_status rdb_chain_create(const rdb_chain_desc* desc, rdb_chain** out)
   }
   if (s != RDB_OK)
   {
-    if (ch->dev) cudaFree(ch->dev);
     delete ch;
     return s;
   }
@@ -250,32 +249,7 @@ void rdb_chain_destroy(rdb_chain* chain)
 {
   if (!chain) return;
   DeviceScope dev__(chain->device);
-  cudaDeviceSynchronize();  // work queued on the caller's streams may still read the model and the workspaces freed below
-  if (chain->gram.done) cudaEventDestroy(chain->gram.done);
-  if (chain->dev) cudaFree(chain->dev);
-  if (chain->gram.partials) cudaFree(chain->gram.partials);
-  if (chain->gram.fused_partials) cudaFree(chain->gram.fused_partials);
-  if (chain->gram.fold_dev) cudaFree(chain->gram.fold_dev);
-  if (chain->gram.ext_dev) cudaFree(chain->gram.ext_dev);
-  if (chain->gram.tau_sq_part) cudaFree(chain->gram.tau_sq_part);
-  if (chain->gram.seg_dev) cudaFree(chain->gram.seg_dev);
-  if (chain->host_arena.base) cudaFree(chain->host_arena.base);
-  if (chain->host_arena.map_h) cudaFreeHost(chain->host_arena.map_h);
-  if (chain->host_arena.pin) cudaFreeHost(chain->host_arena.pin);
-  for (int k = 0; k < GramHostPipe::NSLOT; k++)
-    if (chain->gram_host.pin[k]) cudaFreeHost(chain->gram_host.pin[k]);
-  for (int k = 0; k < 2; k++)
-    if (chain->host_arena.st[k]) cudaStreamDestroy(chain->host_arena.st[k]);
-  GramHostPipe& hp = chain->gram_host;
-  for (int k = 0; k < GramHostPipe::NSLOT; k++)
-  {
-    if (hp.stage[k]) cudaFree(hp.stage[k]);
-    if (hp.copied[k]) cudaEventDestroy(hp.copied[k]);
-    if (hp.freed[k]) cudaEventDestroy(hp.freed[k]);
-  }
-  if (hp.d_out) cudaFree(hp.d_out);
-  if (hp.copy) cudaStreamDestroy(hp.copy);
-  if (hp.comp) cudaStreamDestroy(hp.comp);
+  cudaDeviceSynchronize();  // work queued on the caller's streams may still read the model and the workspaces the handle frees
   delete chain;
 }
 
@@ -808,7 +782,7 @@ struct HostPipe
     const int slots = n > chunk ? 2 : 1;
     for (int k = 0; k < 2; k++)
     {
-      if (!ar.st[k]) RDB_CUDA(cudaStreamCreateWithFlags(&ar.st[k], cudaStreamNonBlocking));
+      RDB_CUDA(ar.st[k].ensure());
       st[k] = ar.st[k];
     }
     size_t need = 0;
@@ -816,19 +790,19 @@ struct HostPipe
       if ((p->h_in || p->h_out) && p->planes > 0) need += sizeof(double) * (size_t)p->planes * chunk * slots;
     if (slots == 1 && need <= RDB_HOST_MAPPED_BYTES)
     {
-      if (!ar.map_h && !ar.map_failed)
+      if (!ar.map_h.get() && !ar.map_failed)
       {
         // no mapped pinned memory on this host (locked-memory limit, ...): remembered, the copy path below serves small calls as well
-        if (cudaHostAlloc(&ar.map_h, RDB_HOST_MAPPED_BYTES, cudaHostAllocMapped) != cudaSuccess ||
-            cudaHostGetDevicePointer(&ar.map_d, ar.map_h, 0) != cudaSuccess)
+        if (ar.map_h.grow(RDB_HOST_MAPPED_BYTES, nullptr) != cudaSuccess ||
+            cudaHostGetDevicePointer(&ar.map_d, ar.map_h.get(), 0) != cudaSuccess)
         {
           cudaGetLastError();
-          if (ar.map_h) cudaFreeHost(ar.map_h);
-          ar.map_h = ar.map_d = nullptr;
+          ar.map_h.reset();
+          ar.map_d = nullptr;
           ar.map_failed = true;
         }
       }
-      if (ar.map_h)
+      if (ar.map_h.get())
       {
         mapped = true;
         size_t o = 0;
@@ -836,36 +810,21 @@ struct HostPipe
           if ((p->h_in || p->h_out) && p->planes > 0)
           {
             p->d[0] = ar.map_d + o;
-            p->hm = ar.map_h + o;
+            p->hm = ar.map_h.get() + o;
             o += (size_t)p->planes * chunk;
           }
         return RDB_OK;
       }
     }
-    if (ar.bytes < need)
+    RDB_CUDA(ar.base.grow(need, nullptr));
+    if (bounce && ar.pin.grow(need, nullptr) != cudaSuccess)
     {
-      if (ar.base) cudaFree(ar.base);
-      ar.base = nullptr;
-      ar.bytes = 0;
-      RDB_CUDA(cudaMalloc(&ar.base, need));
-      ar.bytes = need;
+      cudaGetLastError();
+      ar.pin_failed = true;  // no pinned memory to spare: the driver's staging serves
+      bounce = false;
     }
-    if (bounce && ar.pin_bytes < need)
-    {
-      if (ar.pin) cudaFreeHost(ar.pin);
-      ar.pin = nullptr;
-      ar.pin_bytes = 0;
-      if (cudaHostAlloc(&ar.pin, need, cudaHostAllocDefault) == cudaSuccess) ar.pin_bytes = need;
-      else
-      {
-        cudaGetLastError();
-        ar.pin = nullptr;
-        ar.pin_failed = true;  // no pinned memory to spare: the driver's staging serves
-        bounce = false;
-      }
-    }
-    double* cur = ar.base;
-    double* hcur = ar.pin;
+    double* cur = ar.base.get();
+    double* hcur = ar.pin.get();
     for (Plane* p : all)
       if ((p->h_in || p->h_out) && p->planes > 0)
         for (int k = 0; k < slots; k++)
@@ -1175,38 +1134,17 @@ rdb_status rdb_regressor_gram_batch_host(rdb_chain* chain, const rdb_samples* in
     return std::min<int64_t>(std::max<int64_t>(v, 1 << 10), 1 << 24);
   }();
   const size_t n_out = (size_t)P * P + P + 1;
-  if (!hp.copy)
+  const size_t slot_doubles = 4 * (size_t)std::max(n_in, 1) * chunk;
+  RDB_CUDA(hp.copy.ensure());
+  RDB_CUDA(hp.comp.ensure());
+  for (int k = 0; k < GramHostPipe::NSLOT; k++)
   {
-    RDB_CUDA(cudaStreamCreateWithFlags(&hp.copy, cudaStreamNonBlocking));
-    RDB_CUDA(cudaStreamCreateWithFlags(&hp.comp, cudaStreamNonBlocking));
-    for (int k = 0; k < GramHostPipe::NSLOT; k++)
-    {
-      RDB_CUDA(cudaEventCreateWithFlags(&hp.copied[k], cudaEventDisableTiming));
-      RDB_CUDA(cudaEventCreateWithFlags(&hp.freed[k], cudaEventDisableTiming));
-    }
+    RDB_CUDA(hp.copied[k].ensure());
+    RDB_CUDA(hp.freed[k].ensure());
+    RDB_CUDA(hp.stage[k].grow(sizeof(double) * slot_doubles, nullptr));
   }
-  if (hp.planes != n_in || !hp.stage[0])
-  {
-    for (int k = 0; k < GramHostPipe::NSLOT; k++)
-    {
-      if (hp.stage[k]) cudaFree(hp.stage[k]);
-      hp.stage[k] = nullptr;
-      RDB_CUDA(cudaMalloc(&hp.stage[k], sizeof(double) * 4 * (size_t)std::max(n_in, 1) * chunk));
-    }
-    if (hp.d_out) cudaFree(hp.d_out);
-    hp.d_out = nullptr;
-    RDB_CUDA(cudaMalloc(&hp.d_out, sizeof(double) * n_out));
-    hp.planes = n_in;
-    hp.n_out = n_out;
-  }
-  else if (hp.n_out < n_out)
-  {
-    cudaFree(hp.d_out);
-    hp.d_out = nullptr;
-    RDB_CUDA(cudaMalloc(&hp.d_out, sizeof(double) * n_out));
-    hp.n_out = n_out;
-  }
-  double* dG = hp.d_out;
+  RDB_CUDA(hp.d_out.grow(sizeof(double) * n_out, nullptr));
+  double* dG = hp.d_out.get();
   double* db = dG + (size_t)P * P;
   double* dt = db + P;
   if (accumulate)
@@ -1220,63 +1158,32 @@ rdb_status rdb_regressor_gram_batch_host(rdb_chain* chain, const rdb_samples* in
     RDB_CUDA(cudaMemsetAsync(dG, 0, sizeof(double) * n_out, hp.comp));
   // Pageable inputs: gather each chunk into a pinned bounce buffer with a few host threads (one plane slice per task), then ONE contiguous
   // asynchronous copy -- the driver would otherwise stage every cudaMemcpy2DAsync synchronously through its own buffer on one thread.
-  bool bounce = false;
-  if (in->n >= (1 << 14) && n_in > 0 && !hp.pin_failed)
-  {
-    cudaPointerAttributes at{};
-    if (cudaPointerGetAttributes(&at, in->q) == cudaSuccess && at.type == cudaMemoryTypeUnregistered) bounce = true;
-    else cudaGetLastError();
-  }
-  const size_t slot_doubles = 4 * (size_t)std::max(n_in, 1) * chunk;
-  if (bounce && hp.pin_doubles < slot_doubles)
-  {
-    for (int s = 0; s < GramHostPipe::NSLOT; s++)
-    {
-      if (hp.pin[s]) cudaFreeHost(hp.pin[s]);
-      hp.pin[s] = nullptr;
-    }
-    hp.pin_doubles = 0;
-    bool ok = true;
-    for (int s = 0; s < GramHostPipe::NSLOT && ok; s++) ok = cudaHostAlloc(&hp.pin[s], sizeof(double) * slot_doubles, cudaHostAllocDefault) == cudaSuccess;
-    if (ok) hp.pin_doubles = slot_doubles;
-    else
+  bool bounce = in->n >= (1 << 14) && n_in > 0 && !hp.pin_failed && is_pageable(in->q);
+  for (int s = 0; s < GramHostPipe::NSLOT && bounce; s++)
+    if (hp.pin[s].grow(sizeof(double) * slot_doubles, nullptr) != cudaSuccess)
     {
       cudaGetLastError();
-      for (int s = 0; s < GramHostPipe::NSLOT; s++)
-      {
-        if (hp.pin[s]) cudaFreeHost(hp.pin[s]);
-        hp.pin[s] = nullptr;
-      }
+      for (PinnedBuffer<>& p : hp.pin) p.reset();
       hp.pin_failed = true;  // no pinned memory to spare: the driver's staging serves
       bounce = false;
     }
-  }
-  const int n_workers = bounce ? rdb::host_threads() : 0;
   int64_t k = 0;
   for (int64_t off = 0; off < in->n; off += chunk, k++)
   {
     const int slot = (int)(k % GramHostPipe::NSLOT);
     const int64_t len = std::min<int64_t>(chunk, in->n - off);
     if (k >= GramHostPipe::NSLOT) RDB_CUDA(cudaStreamWaitEvent(hp.copy, hp.freed[slot], 0));
-    double* base = hp.stage[slot];
+    double* base = hp.stage[slot].get();
     const double* src[4] = {in->q, in->dq, in->ddq, tau_meas};
     if (bounce)
     {
       if (k >= GramHostPipe::NSLOT) RDB_CUDA(cudaEventSynchronize(hp.copied[slot]));  // the previous copy out of this bounce buffer is done
-      double* pb = hp.pin[slot];
-      const int n_arr = tau_meas ? 4 : 3, n_tasks = n_arr * n_in;
-      std::atomic<int> next{0};
-      auto work = [&] {
-        for (int t = next.fetch_add(1); t < n_tasks; t = next.fetch_add(1))
-        {
-          const int a = t / n_in, r = t % n_in;
-          memcpy(pb + ((size_t)a * n_in + r) * chunk, src[a] + (size_t)r * in->ld + off, sizeof(double) * (size_t)len);
-        }
-      };
-      std::vector<std::thread> pool;
-      for (int w = 1; w < n_workers; w++) pool.emplace_back(work);
-      work();
-      for (std::thread& th : pool) th.join();
+      double* pb = hp.pin[slot].get();
+      const int n_arr = tau_meas ? 4 : 3;
+      host_parallel((int64_t)n_arr * n_in, [&](int64_t t) {
+        const int64_t a = t / n_in, r = t % n_in;
+        memcpy(pb + ((size_t)a * n_in + r) * chunk, src[a] + (size_t)r * in->ld + off, sizeof(double) * (size_t)len);
+      });
       RDB_CUDA(cudaMemcpyAsync(base, pb, sizeof(double) * (size_t)n_arr * n_in * chunk, cudaMemcpyHostToDevice, hp.copy));
     }
     else

@@ -210,21 +210,13 @@ cudaError_t fold_chain(ChainHost& ch, bool upload)
   w.fold_identity = (K == H.nj) && !rotated;
   if (upload && !w.fold_identity && K > 0)
   {
-    // the caller (upload_model) has synchronised the device: no kernel still reads fold_dev, so it may be freed and rewritten here
-    const size_t need = sizeof(double) * ((size_t)H.nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1)) + sizeof(int32_t) * H.nj;
-    if (w.fold_bytes < need)
-    {
-      if (w.fold_dev) cudaFree(w.fold_dev);
-      w.fold_dev = nullptr;
-      w.fold_bytes = 0;
-      cudaError_t e = cudaMalloc(&w.fold_dev, need);
-      if (e != cudaSuccess) return e;
-      w.fold_bytes = need;
-    }
-    // layout: T (nj x 100) | reduced normal equations G' (P' x P'), b' (P'), tau_sq | link -> reduced link (nj ints)
-    cudaError_t e = cudaMemcpy(w.fold_dev, T.data(), sizeof(double) * T.size(), cudaMemcpyHostToDevice);
+    // the caller (upload_model) has synchronised the device: no kernel still reads the fold maps, so they may be freed and rewritten here
+    cudaError_t e = w.fold_dev.grow(sizeof(double) * T.size() + sizeof(int32_t) * kof.size(), nullptr);
     if (e != cudaSuccess) return e;
-    e = cudaMemcpy(w.fold_dev + (size_t)H.nj * 100 + (size_t)(10 * K + 1) * (10 * K + 1), kof.data(), sizeof(int32_t) * H.nj, cudaMemcpyHostToDevice);
+    const FoldMaps fm = fold_maps(ch);
+    e = cudaMemcpy(fm.T, T.data(), sizeof(double) * T.size(), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) return e;
+    e = cudaMemcpy(fm.kof, kof.data(), sizeof(int32_t) * kof.size(), cudaMemcpyHostToDevice);
     if (e != cudaSuccess) return e;
   }
   if (upload) w.fold_version = ch.model_version;

@@ -162,40 +162,15 @@ __global__ void gram_reduce_kernel(const double* __restrict__ partial, int npart
   }
 }
 
-// tau_sq = (accumulate ? tau_sq : 0) + (part + the measured torques of the inputs no chain joint feeds, squared and summed).  The fused
-// kernels walk the folded chain, whose rows are the fed inputs only; such an input has a zero regressor row (nothing to add to G or b) but
-// its torque is part of the residual |tau - Phi pi|^2.  part: the fused kernels' tau^T tau of this call.  One block, fixed order: reproducible.
+// tau_sq[k] = (accumulate ? tau_sq[k] : 0) + (part[k] + the measured torques of the inputs no chain joint feeds over segment k, squared and
+// summed).  The fused kernels walk the folded chain, whose rows are the fed inputs only; such an input has a zero regressor row (nothing to
+// add to G or b) but its torque is part of the residual |tau - Phi pi|^2.  part: the fused kernels' tau^T tau of this call.  One block per
+// segment [offsets[k], offsets[k + 1]) (device offsets; nullptr: the one segment [0, n)), fixed order: reproducible.
 struct UnfedRows
 {
   int32_t n, row[RDB_MAX_JOINTS];
 };
-__global__ void __launch_bounds__(256) gram_unfed_tau_sq_kernel(const double* __restrict__ tau, int64_t ld, int64_t n, UnfedRows u,
-                                                                const double* __restrict__ part, double* __restrict__ tau_sq, int accumulate)
-{
-  __shared__ double red[256];
-  double s = 0.0;
-  for (int r = 0; r < u.n; r++)
-    for (int64_t i = threadIdx.x; i < n; i += blockDim.x)
-    {
-      const double t = tau[(int64_t)u.row[r] * ld + i];
-      s = fma(t, t, s);
-    }
-  red[threadIdx.x] = s;
-  __syncthreads();
-  for (int w = 128; w > 0; w >>= 1)
-  {
-    if ((int)threadIdx.x < w) red[threadIdx.x] += red[threadIdx.x + w];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0)
-  {
-    const double v = *part + red[0];
-    *tau_sq = accumulate ? *tau_sq + v : v;
-  }
-}
-
-// segmented: one block per segment k (offsets on the device), the same fixed order per segment
-__global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const double* __restrict__ tau, int64_t ld,
+__global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const double* __restrict__ tau, int64_t ld, int64_t n,
                                                                           const int64_t* __restrict__ offsets, int64_t nseg, UnfedRows u,
                                                                           const double* __restrict__ part, double* __restrict__ tau_sq,
                                                                           int accumulate)
@@ -203,7 +178,7 @@ __global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const 
   __shared__ double red[256];
   for (int64_t k = blockIdx.x; k < nseg; k += gridDim.x)
   {
-    const int64_t lo = offsets[k], hi = offsets[k + 1];
+    const int64_t lo = offsets ? offsets[k] : 0, hi = offsets ? offsets[k + 1] : n;
     if (accumulate && lo == hi) continue;
     double s = 0.0;
     for (int r = 0; r < u.n; r++)
@@ -240,11 +215,11 @@ static UnfedRows unfed_rows(const ChainHost& ch)
   return u;
 }
 
-cudaError_t launch_unfed_tau_sq_segmented(const ChainHost& ch, const double* tau, int64_t ld, const int64_t* offsets, int64_t nseg,
-                                          const double* part, double* tau_sq, int accumulate, cudaStream_t st)
+cudaError_t launch_unfed_tau_sq(const ChainHost& ch, const double* tau, int64_t ld, int64_t n, const int64_t* offsets, int64_t nseg,
+                                const double* part, double* tau_sq, int accumulate, cudaStream_t st)
 {
   if (nseg <= 0) return cudaSuccess;
-  gram_unfed_tau_sq_segmented_kernel<<<(unsigned)std::min<int64_t>(nseg, 65535), 256, 0, st>>>(tau, ld, offsets, nseg, unfed_rows(ch), part,
+  gram_unfed_tau_sq_segmented_kernel<<<(unsigned)std::min<int64_t>(nseg, 65535), 256, 0, st>>>(tau, ld, n, offsets, nseg, unfed_rows(ch), part,
                                                                                               tau_sq, accumulate);
   count_launch();
   return cudaGetLastError();
@@ -297,23 +272,18 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
       cudaError_t e = cudaErrorNotSupported;
       // measured torques on inputs no chain joint feeds: the fused kernels' tau^T tau goes to a zeroed scratch word first
       const bool unfed = tau_meas && tau_sq && !ch.inputs_cover_all;
-      if (unfed && !ch.gram.tau_sq_part)
+      if (unfed)
       {
-        e = cudaMalloc(&ch.gram.tau_sq_part, sizeof(double));
+        e = ch.gram.tau_sq_part.grow(sizeof(double), ch.gram.done);
         if (e != cudaSuccess) return e;
+        cudaMemsetAsync(ch.gram.tau_sq_part.get(), 0, sizeof(double), st);
       }
-      if (unfed) cudaMemsetAsync(ch.gram.tau_sq_part, 0, sizeof(double), st);
-      double* ts = unfed ? ch.gram.tau_sq_part : tau_sq;
+      double* ts = unfed ? ch.gram.tau_sq_part.get() : tau_sq;
       if (P == Pr)
         e = launch_gram_fused(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
       else
         e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
-      if (e == cudaSuccess && unfed)
-      {
-        gram_unfed_tau_sq_kernel<<<1, 256, 0, st>>>(tau_meas, in.ld, in.n, unfed_rows(ch), ts, tau_sq, accumulate);
-        count_launch();
-        e = cudaGetLastError();
-      }
+      if (e == cudaSuccess && unfed) e = launch_unfed_tau_sq(ch, tau_meas, in.ld, in.n, nullptr, 1, ts, tau_sq, accumulate, st);
       if (e != cudaErrorNotSupported) return e;
     }
     // rdb_chain_gram_kernel_info describes the last Gram call: say that this one ran the general pipeline, and why
@@ -328,21 +298,9 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
   chunk = std::min<int64_t>((chunk / 128) * 128, std::max<int64_t>(in.n, 128));
   const int gx = std::max(1, std::min<int>(ch.sm_count * 2 / std::max(1, npairs) + 1, (int)((chunk + 15) / 16)));
   const size_t need = sizeof(double) * ((size_t)chunk * (P * n_in + n_in) + (size_t)gx * npairs * TILE_ELEMS);
-  if (ch.gram.bytes < need)
-  {
-    if (ch.gram.partials)
-    {
-      cudaError_t e = cudaEventSynchronize(ch.gram.done);  // the previous Gram call may still read the old buffer
-      if (e != cudaSuccess) return e;
-      cudaFree(ch.gram.partials);
-    }
-    ch.gram.partials = nullptr;
-    ch.gram.bytes = 0;
-    cudaError_t e = cudaMalloc(&ch.gram.partials, need);
-    if (e != cudaSuccess) return e;
-    ch.gram.bytes = need;
-  }
-  double* w_phi = ch.gram.partials;
+  cudaError_t e = ch.gram.partials.grow(need, ch.gram.done);
+  if (e != cudaSuccess) return e;
+  double* w_phi = ch.gram.partials.get();
   double* w_tau = w_phi + (size_t)chunk * P * n_in;
   double* w_part = w_tau + (size_t)chunk * n_in;
   for (int64_t off = 0; off < in.n; off += chunk)
@@ -351,7 +309,7 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
     SamplesDev v{len, in.ld, in.q + off, in.dq + off, in.ddq + off, nullptr};
     const bool own_tau = (tau_meas == nullptr);
     if (!ch.inputs_cover_all) cudaMemsetAsync(w_phi, 0, sizeof(double) * (size_t)chunk * (P * n_in + n_in), st);
-    cudaError_t e = launch_dyn(ch, own_tau ? (DYN_REGRESSOR_ | DYN_TORQUE_) : DYN_REGRESSOR_, v, w_phi, own_tau ? w_tau : nullptr, nullptr, chunk, st);
+    e = launch_dyn(ch, own_tau ? (DYN_REGRESSOR_ | DYN_TORQUE_) : DYN_REGRESSOR_, v, w_phi, own_tau ? w_tau : nullptr, nullptr, chunk, st);
     if (e != cudaSuccess) return e;
     if (P > Pr)  // component planes follow the rigid-body planes (plane index = col * n_in + row)
     {
@@ -377,19 +335,25 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
   return cudaSuccess;
 }
 
-// Every Gram call of a handle (device entries, the host entry's chunks, the group's shards) goes through here.  The workspace of
-// ch.gram is shared by all of them, and callers may pass any stream: each call's stream first waits for the device work of the previous
+// Every Gram call of a handle (device entries, the host entry's chunks, the group's shards) runs its launches through here.  The workspace
+// of ch.gram is shared by all of them, and callers may pass any stream: each call's stream first waits for the device work of the previous
 // call (free on the same stream), and the call's own work is recorded for the next one.
-cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
-                        cudaStream_t st, bool with_components)
+template <class F>
+static cudaError_t ordered_gram_call(ChainHost& ch, cudaStream_t st, F&& launches)
 {
-  cudaError_t e = ch.gram.done ? cudaSuccess : cudaEventCreateWithFlags(&ch.gram.done, cudaEventDisableTiming);
+  cudaError_t e = ch.gram.done.ensure();
   if (e != cudaSuccess) return e;
   e = cudaStreamWaitEvent(st, ch.gram.done, 0);
   if (e != cudaSuccess) return e;
-  e = gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components);
+  e = launches();
   const cudaError_t r = cudaEventRecord(ch.gram.done, st);  // also after a failed launch: whatever was queued stays ordered
   return e != cudaSuccess ? e : r;
+}
+
+cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
+                        cudaStream_t st, bool with_components)
+{
+  return ordered_gram_call(ch, st, [&] { return gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components); });
 }
 
 static cudaError_t gram_segmented_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,
@@ -421,17 +385,10 @@ static cudaError_t gram_segmented_launches(ChainHost& ch, const SamplesDev& in, 
   return cudaSuccess;
 }
 
-// ordered like launch_gram
 cudaError_t launch_gram_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets, double* gram,
                                   double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
 {
-  cudaError_t e = ch.gram.done ? cudaSuccess : cudaEventCreateWithFlags(&ch.gram.done, cudaEventDisableTiming);
-  if (e != cudaSuccess) return e;
-  e = cudaStreamWaitEvent(st, ch.gram.done, 0);
-  if (e != cudaSuccess) return e;
-  e = gram_segmented_launches(ch, in, tau_meas, nseg, offsets, gram, rhs, tau_sq, accumulate, st);
-  const cudaError_t r = cudaEventRecord(ch.gram.done, st);
-  return e != cudaSuccess ? e : r;
+  return ordered_gram_call(ch, st, [&] { return gram_segmented_launches(ch, in, tau_meas, nseg, offsets, gram, rhs, tau_sq, accumulate, st); });
 }
 
 // ---------------------------------------------------------------------------------------------------------

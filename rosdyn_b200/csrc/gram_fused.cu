@@ -169,51 +169,22 @@ static int gram_dev_switch()
 #endif
 }
 
-// the reduced normal equations G' | b' | tau_sq of the folded chain (ch.gram.fold_dev, written by the reduce kernels) -> the reference's full
-// parameter vector
+// the reduced normal equations G' | b' | tau_sq of the folded chain (reduced_row(ch, 0), written by the reduce kernels) -> the reference's
+// full parameter vector
 cudaError_t launch_fold_expand(ChainHost& ch, double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
 {
   const int nj = ch.host.nj, Pr = 10 * ch.gram.fold.nj, P = 10 * nj;
-  double* Tm = ch.gram.fold_dev;
-  double* Gr = Tm + (size_t)nj * 100;
-  double* br = Gr + (size_t)Pr * Pr;
-  double* tsr = br + Pr;
-  const int32_t* kof = reinterpret_cast<const int32_t*>(Gr + (size_t)(Pr + 1) * (Pr + 1));
-  gram_fold_expand_kernel<<<(P * (P + 1) + 127) / 128, 128, 0, st>>>(Tm, kof, Gr, br, tsr, nj, Pr, gram, rhs, tau_sq, accumulate);
+  const FoldMaps fm = fold_maps(ch);
+  const ReducedRow r = reduced_row(ch, 0);
+  gram_fold_expand_kernel<<<(P * (P + 1) + 127) / 128, 128, 0, st>>>(fm.T, fm.kof, r.G, r.b, r.tau_sq, nj, Pr, gram, rhs, tau_sq, accumulate);
   count_launch();
   return cudaGetLastError();
 }
 
-template <int NJ>
-static ChainDev<NJ> narrow_g(const ChainDev<RDB_MAX_JOINTS>& h)
+// the reduced normal equations of `rows` systems of the folded chain (ch.gram.reduced)
+static cudaError_t grow_reduced(ChainHost& ch, int64_t rows)
 {
-  ChainDev<NJ> c;
-  c.nj = h.nj;
-  c.n_in = h.n_in;
-  for (int k = 0; k < 3; k++) c.g[k] = h.g[k];
-  for (int j = 0; j < NJ; j++)
-  {
-    c.joint[j] = h.joint[j];
-    c.link[j] = h.link[j];
-  }
-  return c;
-}
-
-// done: the handle's Gram event (launch_gram); the previous Gram call, possibly on another stream, may still use the old buffer
-static cudaError_t grow(double*& p, size_t& have, size_t need, cudaEvent_t done)
-{
-  if (have >= need) return cudaSuccess;
-  if (p)
-  {
-    const cudaError_t e = cudaEventSynchronize(done);
-    if (e != cudaSuccess) return e;
-    cudaFree(p);
-  }
-  p = nullptr;
-  have = 0;
-  cudaError_t e = cudaMalloc(&p, need);
-  if (e == cudaSuccess) have = need;
-  return e;
+  return ch.gram.reduced.grow(sizeof(double) * rows * ReducedRow::doubles(10 * ch.gram.fold.nj), ch.gram.done);
 }
 
 // slots that fit the shared memory of an SM (227 KB minus 1 KB of barriers / static data): the rows, and XC component columns per joint
@@ -260,7 +231,7 @@ static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const
     constexpr int B = gram_group_block<SLOTS, XC>();
     *grid = (int)std::min<int64_t>(ch.sm_count, (ngroups + B - 1) / B);
   }
-  ChainDev<NJ> C = narrow_g<NJ>(ch.gram.fold);
+  ChainDev<NJ> C = narrow<NJ>(ch.gram.fold);
   GramComps comps = gc;
   SamplesDev ins = in;
   const double* tm = tau_meas;
@@ -281,23 +252,21 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
 {
   constexpr int Z = REV ? 2 : 0;  // as in the kernel
   using G = GramGeom<NJ, Z>;
-  cudaError_t e = grow(ch.gram.fused_partials, ch.gram.fused_bytes, sizeof(double) * (size_t)ch.sm_count * G::PARTIAL, ch.gram.done);
+  cudaError_t e = ch.gram.fused_partials.grow(sizeof(double) * (size_t)ch.sm_count * G::PARTIAL, ch.gram.done);
+  if (e == cudaSuccess && !ch.gram.fold_identity) e = grow_reduced(ch, 1);
   if (e != cudaSuccess) return e;
+  double* part = ch.gram.fused_partials.get();
   int grid = 0;
-  e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, ch.gram.fused_partials, &grid, st);
+  e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, part, &grid, st);
   if (e != cudaSuccess) return e;
   if (ch.gram.fold_identity)
   {
-    launch_fused_reduce<NJ, Z>(ch.gram.fused_partials, grid, G::PARTIAL, gram, rhs, tau_sq, accumulate, st);
+    launch_fused_reduce<NJ, Z>(part, grid, G::PARTIAL, gram, rhs, tau_sq, accumulate, st);
     return cudaGetLastError();
   }
   // folded chain: reduce into G', b', then expand to the reference's full parameter vector
-  const int nj = ch.host.nj, Pr = G::P;
-  double* Tm = ch.gram.fold_dev;
-  double* Gr = Tm + (size_t)nj * 100;
-  double* br = Gr + (size_t)Pr * Pr;
-  double* tsr = br + Pr;
-  launch_fused_reduce<NJ, Z>(ch.gram.fused_partials, grid, G::PARTIAL, Gr, br, tsr, 0, st);
+  const ReducedRow r = reduced_row(ch, 0);
+  launch_fused_reduce<NJ, Z>(part, grid, G::PARTIAL, r.G, r.b, r.tau_sq, 0, st);
   return launch_fold_expand(ch, gram, rhs, tau_sq, accumulate, st);
 }
 
@@ -409,16 +378,14 @@ static cudaError_t launch_fused_segmented_nj(ChainHost& ch, const SamplesDev& in
   using G = GramGeom<NJ, Z>;
   const int nj = ch.host.nj, Pr = G::P, P = 10 * nj;
   const bool fold = !ch.gram.fold_identity;
-  // workspace: per-item partials of one wave | (folded chain) reduced equations G' | b' | tau_sq of each row of a wave | (unfed) the fused
-  // tau^T tau of every segment | the plan's table
-  const int64_t RS = (int64_t)Pr * Pr + Pr + 1;
-  const size_t n_part = (size_t)plan.wave * G::PARTIAL, n_red = fold ? (size_t)plan.max_rows * RS : 0, n_ts = unfed ? (size_t)nseg : 0;
-  cudaError_t e = grow(ch.gram.seg_dev, ch.gram.seg_bytes, sizeof(double) * (n_part + n_red + n_ts) + sizeof(int64_t) * plan.tab.size(),
-                       ch.gram.done);
+  // workspace: per-item partials of one wave | (unfed) the fused tau^T tau of every segment | the plan's table; (folded chain) the reduced
+  // equations of each row of a wave
+  const size_t n_part = (size_t)plan.wave * G::PARTIAL, n_ts = unfed ? (size_t)nseg : 0;
+  cudaError_t e = ch.gram.seg_dev.grow(sizeof(double) * (n_part + n_ts) + sizeof(int64_t) * plan.tab.size(), ch.gram.done);
+  if (e == cudaSuccess && fold) e = grow_reduced(ch, plan.max_rows);
   if (e != cudaSuccess) return e;
-  double* part = ch.gram.seg_dev;
-  double* red = part + n_part;
-  double* ts = red + n_red;
+  double* part = ch.gram.seg_dev.get();
+  double* ts = part + n_part;
   int64_t* tab = reinterpret_cast<int64_t*>(ts + n_ts);
   e = cudaMemcpyAsync(tab, plan.tab.data(), sizeof(int64_t) * plan.tab.size(), cudaMemcpyHostToDevice, st);  // pageable: staged before return
   if (e != cudaSuccess) return e;
@@ -426,8 +393,6 @@ static cudaError_t launch_fused_segmented_nj(ChainHost& ch, const SamplesDev& in
   const int64_t* rows = items + 2 * plan.nitems;
   if (unfed) cudaMemsetAsync(ts, 0, sizeof(double) * nseg, st);
   double* tso = unfed ? ts : tau_sq;
-  const double* Tm = ch.gram.fold_dev;
-  const int32_t* kof = reinterpret_cast<const int32_t*>(ch.gram.fold_dev + (size_t)nj * 100 + (size_t)(Pr + 1) * (Pr + 1));
   const int nred = std::max(G::PARTIAL, Pr * (Pr + 1));
   for (const SegPlan::Wave& w : plan.waves)
   {
@@ -443,17 +408,19 @@ static cudaError_t launch_fused_segmented_nj(ChainHost& ch, const SamplesDev& in
       gram_fused_reduce_segmented_kernel<NJ, Z><<<rg, 256, 0, st>>>(part, wr, G::PARTIAL, gram, rhs, tso, (int64_t)P * P, P, 1, 1, w.accumulate);
     else
     {
-      gram_fused_reduce_segmented_kernel<NJ, Z><<<rg, 256, 0, st>>>(part, wr, G::PARTIAL, red, red + (size_t)Pr * Pr, red + (size_t)Pr * Pr + Pr,
-                                                                    RS, RS, RS, 0, 0);
+      const FoldMaps fm = fold_maps(ch);
+      const ReducedRow r = reduced_row(ch, 0);
+      const int64_t RS = ReducedRow::doubles(Pr);
+      gram_fused_reduce_segmented_kernel<NJ, Z><<<rg, 256, 0, st>>>(part, wr, G::PARTIAL, r.G, r.b, r.tau_sq, RS, RS, RS, 0, 0);
       count_launch();
-      gram_fold_expand_segmented_kernel<<<dim3((P * (P + 1) + 127) / 128, (unsigned)w.nrows), 128, 0, st>>>(Tm, kof, red, RS, wr, nj, Pr, gram, rhs,
-                                                                                                             tso, w.accumulate);
+      gram_fold_expand_segmented_kernel<<<dim3((P * (P + 1) + 127) / 128, (unsigned)w.nrows), 128, 0, st>>>(fm.T, fm.kof, r.G, RS, wr, nj, Pr, gram,
+                                                                                                             rhs, tso, w.accumulate);
     }
     count_launch();
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
   }
-  if (unfed) return launch_unfed_tau_sq_segmented(ch, tau_meas, in.ld, tab, nseg, ts, tau_sq, accumulate, st);
+  if (unfed) return launch_unfed_tau_sq(ch, tau_meas, in.ld, in.n, tab, nseg, ts, tau_sq, accumulate, st);
   return cudaSuccess;
 }
 
@@ -571,10 +538,10 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   const int nj = ch.host.nj, P = 10 * nj, Pc = ch.comps.cols, Pt = P + Pc;
   // workspace: rigid block (P*P + P + 1) | cross sums (NXT*64) | per-CTA partials (sm_count*PSTRIDE) | component map (2 Pc ints)
   const size_t n_rigid = (size_t)P * P + P + 1, n_sum = (size_t)G::NXT * 64, n_part = (size_t)ch.sm_count * PSTRIDE;
-  cudaError_t e = grow(ch.gram.ext_dev, ch.gram.ext_bytes, sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc,
-                       ch.gram.done);
+  cudaError_t e = ch.gram.ext_dev.grow(sizeof(double) * (n_rigid + n_sum + n_part) + sizeof(int32_t) * 2 * (size_t)Pc, ch.gram.done);
+  if (e == cudaSuccess && !ch.gram.fold_identity) e = grow_reduced(ch, 1);
   if (e != cudaSuccess) return e;
-  double* Gt = ch.gram.ext_dev;
+  double* Gt = ch.gram.ext_dev.get();
   double* bt = Gt + (size_t)P * P;
   double* tst = bt + P;
   double* xsum = tst + 1;
@@ -588,9 +555,8 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   if (ch.gram.fold_identity) launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gt, bt, tst, 0, st);
   else
   {
-    double* Gr = ch.gram.fold_dev + (size_t)nj * 100;
-    double* br = Gr + (size_t)G::P * G::P;
-    launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gr, br, br + G::P, 0, st);
+    const ReducedRow r = reduced_row(ch, 0);
+    launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, r.G, r.b, r.tau_sq, 0, st);
     e = launch_fold_expand(ch, Gt, bt, tst, 0, st);
     if (e != cudaSuccess) return e;
   }
@@ -598,10 +564,8 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   count_launch();
   gram_ext_scatter_kernel<<<(P * (P + 1) + 255) / 256, 256, 0, st>>>(Gt, bt, tst, P, Pt, gram, rhs, tau_sq, accumulate);
   count_launch();
-  const double* Tm1 = ch.gram.fold_identity ? nullptr : ch.gram.fold_dev;
-  const int32_t* kof1 =
-      ch.gram.fold_identity ? nullptr : reinterpret_cast<const int32_t*>(ch.gram.fold_dev + (size_t)nj * 100 + (size_t)(G::P + 1) * (G::P + 1));
-  gram_cross_finish_kernel<NJ, Z><<<((P + 1 + Pc) * Pc + 127) / 128, 128, 0, st>>>(xsum, Tm1, kof1, dmap, dmap + Pc, nj, Pc, gram, rhs, accumulate);
+  const FoldMaps fm = ch.gram.fold_identity ? FoldMaps{nullptr, nullptr} : fold_maps(ch);
+  gram_cross_finish_kernel<NJ, Z><<<((P + 1 + Pc) * Pc + 127) / 128, 128, 0, st>>>(xsum, fm.T, fm.kof, dmap, dmap + Pc, nj, Pc, gram, rhs, accumulate);
   count_launch();
   return cudaGetLastError();
 }

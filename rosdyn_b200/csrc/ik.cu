@@ -313,7 +313,7 @@ cudaError_t launch_ik(const ChainHost& ch, int64_t n, int64_t ld, const double* 
   for (int k = 0; k < 6; k++) prm.weight[k] = weight ? weight[k] : 1.0;
   prm.tol = tol;
   prm.max_iter = max_iter;
-  ik_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(ch.dev, prm, n, ld, target, seed, sol, status, iters, err);
+  ik_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(ch.dev.get(), prm, n, ld, target, seed, sol, status, iters, err);
   count_launch();
   return cudaGetLastError();
 }

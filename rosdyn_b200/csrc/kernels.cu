@@ -890,21 +890,6 @@ void fill_uniform_host(double* x, int n_planes, int64_t n, int64_t ld, uint64_t 
 // =============================================================================================================
 // launchers
 // =============================================================================================================
-template <int NJ>
-static ChainDev<NJ> narrow(const ChainDev<RDB_MAX_JOINTS>& h)
-{
-  ChainDev<NJ> c;
-  c.nj = h.nj;
-  c.n_in = h.n_in;
-  for (int k = 0; k < 3; k++) c.g[k] = h.g[k];
-  for (int j = 0; j < NJ; j++)
-  {
-    c.joint[j] = h.joint[j];
-    c.link[j] = h.link[j];
-  }
-  return c;
-}
-
 static inline unsigned grid_for(int64_t n) { return (unsigned)((n + RDB_BLOCK - 1) / RDB_BLOCK); }
 
 #define RDB_FAST_NJ(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8)
@@ -953,7 +938,7 @@ static cudaError_t launch_dyn_mode(const ChainHost& ch, const SamplesDev& in, co
     RDB_FAST_NJ(X)
 #undef X
     default:
-      dyn_kernel_generic<MODE><<<grid, RDB_BLOCK, 0, st>>>(ch.dev, in, out);
+      dyn_kernel_generic<MODE><<<grid, RDB_BLOCK, 0, st>>>(ch.dev.get(), in, out);
   }
   count_launch();
   return cudaGetLastError();
@@ -994,7 +979,7 @@ static cudaError_t launch_kin_mask(const ChainHost& ch, const SamplesDev& in, co
     RDB_FAST_NJ(X)
 #undef X
     default:
-      kin_kernel_generic<MASK><<<grid, RDB_BLOCK, 0, st>>>(ch.dev, in, o);
+      kin_kernel_generic<MASK><<<grid, RDB_BLOCK, 0, st>>>(ch.dev.get(), in, o);
   }
   count_launch();
   return cudaGetLastError();
