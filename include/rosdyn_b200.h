@@ -251,6 +251,30 @@ rdb_status rdb_regressor_gram_segmented_batch(rdb_chain* chain, const rdb_sample
                                               const int64_t* offsets, double* gram, double* rhs, double* tau_sq, int32_t accumulate,
                                               void* stream);
 
+/* Diagonal weights of the normal equations: the weight of input joint r (input order) in sample i is
+ *   w[r * joint_stride + i * sample_stride]          (DEVICE memory; strides in doubles, >= 0)
+ * (1, 0): one weight per joint (WLS);  (0, 1): one per sample (masks, IRLS);  (ld_w, 1): planes [n_inputs][ld_w];  (0, 0): one scalar.
+ * Weights must be finite and >= 0; they are device data and are not checked: other values give unspecified outputs. */
+typedef struct rdb_gram_weights
+{
+  const double* w;
+  int64_t joint_stride;
+  int64_t sample_stride;
+} rdb_gram_weights;
+
+/* Weighted normal equations (weighted least squares: per-joint noise weights, sample masks, IRLS re-weights), W_s = diag(w[., s]):
+ *   gram   (+)= sum_s Phi_s^T W_s Phi_s
+ *   rhs    (+)= sum_s Phi_s^T W_s tau_s
+ *   tau_sq (+)= sum_s tau_s^T W_s tau_s
+ * with every other convention of rdb_regressor_gram_batch (tau_meas NULL = getJointTorque, accumulate, ordering with the handle's other
+ * Gram calls on any stream).  Inputs no chain joint feeds have a zero regressor row; with tau_meas their w tau^2 joins tau_sq.
+ * weights NULL, weights->w NULL or a negative stride: RDB_ERR_INVALID_ARG; otherwise the errors of rdb_regressor_gram_batch.
+ * w == 1 gives the results of rdb_regressor_gram_batch bit for bit.  rdb_normal_equations_solve takes the outputs as they are; its
+ * residual_sq is then sum_s ||W_s^(1/2) (Phi_s pi - tau_s)||^2.  One-hot per-joint weights (1 for input r, 0 elsewhere) give G_r, b_r and
+ * tau_r^T tau_r, from which ||tau_r - Phi_r pi||^2 = tau_r^T tau_r - 2 pi^T b_r + pi^T G_r pi: the per-joint residuals of a fit. */
+rdb_status rdb_regressor_gram_weighted_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, const rdb_gram_weights* weights,
+                                             double* gram, double* rhs, double* tau_sq, int32_t accumulate, void* stream);
+
 /* Chain::getWrench / Chain::getJointTorque(q,Dq,DDq,ext_wrenches_in_link_frame) (PI.h:1225-1274).
  * ext_wrenches[nL][6][ld_ext]: wrenches applied TO the links, in link frames, [force; torque] per link (NULL = none).  The reference
  * brings them to the base frame with the TWIST transform spatialTranformation(-ext, T_bl) (PI.h:1255, SA.h:193-197); mirrored
@@ -319,6 +343,9 @@ rdb_status rdb_components_torque_batch(const rdb_chain* chain, const rdb_samples
  * same conventions as rdb_regressor_gram_batch.  tau_s = tau_meas when given, else the rigid-body getJointTorque. */
 rdb_status rdb_regressor_gram_ext_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, double* gram, double* rhs,
                                         double* tau_sq, int32_t accumulate, void* stream);
+/* The same with diagonal weights (rdb_regressor_gram_weighted_batch): the component columns of input joint r are weighted with row r. */
+rdb_status rdb_regressor_gram_ext_weighted_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, const rdb_gram_weights* weights,
+                                                 double* gram, double* rhs, double* tau_sq, int32_t accumulate, void* stream);
 
 /* Chain::getMultiplicity (PI.h:1470-1517), HOST arrays: every joint vector q + 2 pi k that stays inside [q_min, q_max], revolute input
  * joints only (joint_type_of_input[i] = RDB_JOINT_* of the chain joint fed by input i), in the reference's order (q first; per joint
@@ -349,7 +376,8 @@ rdb_status rdb_gram_row_layout(int32_t nj, int32_t* pos, int32_t* rowlen, int32_
  * Minimum-norm least-squares solution of gram * parameters = rhs through a symmetric eigen-decomposition: the regressor is rank
  * deficient in the standard parameters, so eigenvalues <= rel_tol * lambda_max (rel_tol <= 0: 1e-10) are discarded.
  * gram[P*P] column-major (as rdb_regressor_gram_batch returns it, copied to the host), rhs[P]; outputs parameters[P],
- * optional eigenvalues[P] (descending), rank, residual_sq = tau_sq - 2 pi^T rhs + pi^T gram pi = sum ||Phi pi - tau||^2. */
+ * optional eigenvalues[P] (descending), rank, residual_sq = tau_sq - 2 pi^T rhs + pi^T gram pi = sum ||Phi pi - tau||^2
+ * (sum ||W^(1/2) (Phi pi - tau)||^2 for the outputs of rdb_regressor_gram_weighted_batch: a weighted least-squares solution). */
 rdb_status rdb_normal_equations_solve(int32_t P, const double* gram, const double* rhs, double tau_sq, double rel_tol, double* parameters,
                                       double* eigenvalues, int32_t* rank, double* residual_sq);
 
@@ -367,7 +395,8 @@ int32_t rdb_chain_device(const rdb_chain* chain);
  * a component set the one-pass kernel refuses), -1 before the first call.  reason (optional, reason_len bytes, NUL-terminated) says why, or
  * how long the compile took; for the general pipeline it starts with "general pipeline:".  After rdb_regressor_gram_segmented_batch the
  * reason of a fused run starts with "gram_fused_segmented_kernel, ", and that of a general-pipeline run with
- * "general pipeline: one pass per segment". */
+ * "general pipeline: one pass per segment".  After a weighted call (rdb_regressor_gram_weighted_batch, rdb_regressor_gram_ext_weighted_batch)
+ * the reason of a fused run starts with "gram_fused_weighted_kernel, ". */
 rdb_status rdb_chain_gram_kernel_info(const rdb_chain* chain, int32_t* specialised, char* reason, int32_t reason_len);
 /* Host only, no device needed (inspection tools): the cubin of the run-time specialised kernel of an all-revolute chain, written to `path`.
  * kernel_args: the kernel and its template arguments without the model, e.g. "gram_fused_kernel<6, 4, true, 0"; arch e.g. "sm_100a". */

@@ -210,6 +210,12 @@ public:
   {
     check(rdb_regressor_gram_batch(m_h, &in, tau_meas, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
   }
+  // weighted normal equations (rdb_regressor_gram_weighted_batch): sum Phi^T W Phi, Phi^T W tau, tau^T W tau with the device weights w
+  void getRegressorGram(const rdb_samples& in, const double* tau_meas, const rdb_gram_weights& w, double* gram, double* rhs, double* tau_sq,
+                        bool accumulate, void* stream = nullptr)
+  {
+    check(rdb_regressor_gram_weighted_batch(m_h, &in, tau_meas, &w, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
+  }
   // one normal-equation system per segment [offsets[k], offsets[k+1]) (rdb_regressor_gram_segmented_batch): gram[K][P*P], rhs[K][P],
   // tau_sq[K] (or nullptr) on the device, K = offsets.size() - 1; offsets stay on the host
   void getRegressorGramSegmented(const rdb_samples& in, const double* tau_meas, const std::vector<int64_t>& offsets, double* gram, double* rhs,
@@ -283,6 +289,12 @@ public:
   void getRegressorGramExt(const rdb_samples& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, bool accumulate, void* stream = nullptr)
   {
     check(rdb_regressor_gram_ext_batch(m_h, &in, tau_meas, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
+  }
+  // the same with diagonal weights (rdb_regressor_gram_ext_weighted_batch)
+  void getRegressorGramExt(const rdb_samples& in, const double* tau_meas, const rdb_gram_weights& w, double* gram, double* rhs, double* tau_sq,
+                           bool accumulate, void* stream = nullptr)
+  {
+    check(rdb_regressor_gram_ext_weighted_batch(m_h, &in, tau_meas, &w, gram, rhs, tau_sq, accumulate ? 1 : 0, stream));
   }
   // minimum-norm solution of the normal equations (host arrays); returns the rank
   static int solveNormalEquations(const VectorXd& gram, const VectorXd& rhs, double tau_sq, VectorXd& parameters, double* residual_sq = nullptr,

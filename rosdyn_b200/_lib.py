@@ -39,6 +39,10 @@ class CUrdfChain(ctypes.Structure):
                 ("ddq_max", ctypes.POINTER(ctypes.c_double)), ("tau_max", ctypes.POINTER(ctypes.c_double))]
 
 
+class CGramWeights(ctypes.Structure):
+    _fields_ = [("w", _dp), ("joint_stride", i64), ("sample_stride", i64)]
+
+
 class CComponentDesc(ctypes.Structure):
     _fields_ = [("type", i32), ("input_index", i32), ("min_velocity", ctypes.c_double), ("max_velocity", ctypes.c_double)]
 
@@ -72,6 +76,8 @@ SYMBOLS = {
     "rdb_regressor_gram_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32, ctypes.c_void_p]),
     "rdb_regressor_gram_segmented_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, i64, ctypes.POINTER(i64), _dp, _dp, _dp, i32,
                                                  ctypes.c_void_p]),
+    "rdb_regressor_gram_weighted_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, ctypes.POINTER(CGramWeights), _dp, _dp, _dp, i32,
+                                                ctypes.c_void_p]),
     "rdb_wrench_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, i64, _dp, _dp, i64, ctypes.c_void_p]),
     "rdb_jacobian_link_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), i32, _dp, i64, ctypes.c_void_p]),
     "rdb_local_ik_batch": (i32, [ctypes.c_void_p, i64, i64, _dp, _dp, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double),
@@ -83,6 +89,8 @@ SYMBOLS = {
     "rdb_components_regressor_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, i64, ctypes.c_void_p]),
     "rdb_components_torque_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), ctypes.POINTER(ctypes.c_double), _dp, i64, i32, ctypes.c_void_p]),
     "rdb_regressor_gram_ext_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, _dp, _dp, _dp, i32, ctypes.c_void_p]),
+    "rdb_regressor_gram_ext_weighted_batch": (i32, [ctypes.c_void_p, ctypes.POINTER(CSamples), _dp, ctypes.POINTER(CGramWeights), _dp, _dp, _dp,
+                                                    i32, ctypes.c_void_p]),
     "rdb_fold_parameter_map": (i32, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
     "rdb_fold_canonical_frame": (i32, [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
     "rdb_gram_row_layout": (i32, [i32, ctypes.POINTER(i32), ctypes.POINTER(i32), ctypes.POINTER(i32)]),

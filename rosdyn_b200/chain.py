@@ -486,16 +486,42 @@ class Chain:
         check(self._lib.rdb_chain_gram_kernel_info(self._h, ctypes.byref(flag), buf, len(buf)))
         return flag.value, buf.value.decode(errors="replace")
 
-    def regressorGram(self, q, Dq, DDq, tau_meas=None, out=None):
+    def _weights(self, dev, n, weights):
+        """The rdb_gram_weights of a torch CUDA float64 tensor broadcastable to (n_inputs, N): shape (n_inputs,) (one weight per joint, also
+        when N == n_inputs), (N,) or (1, N) (one per sample), (n_inputs, N), a 0-d scalar, or any expanded view of these.  Its two element
+        strides are passed as they are (an expanded dimension has stride 0).  Returns the struct and the view it points into."""
+        from ._lib import CGramWeights
+        if not dev or not _is_torch(weights) or not weights.is_cuda:
+            raise ValueError("weights take device (torch CUDA) arrays, with device samples")
+        if weights.dtype != torch.float64:
+            raise ValueError("weights must be float64")
+        w = weights
+        if w.ndim == 1 and w.shape[0] == self.n_in:
+            w = w.reshape(-1, 1)  # one weight per joint
+        try:
+            w = w.expand(self.n_in, n)
+        except RuntimeError:
+            raise ValueError(f"weights: shape {tuple(weights.shape)} does not broadcast to (n_inputs, N) = ({self.n_in}, {n})") from None
+        js, ss = w.stride()
+        if min(js, ss) < 0:
+            raise ValueError("weights: negative strides")
+        return CGramWeights(ctypes.c_void_p(w.data_ptr()), js if self.n_in > 1 else 0, ss if n > 1 else 0), w
+
+    def regressorGram(self, q, Dq, DDq, tau_meas=None, out=None, weights=None):
         """Fused getRegressor -> normal equations: returns (G[P,P], b[P], tau_sq[1]) with
         G = sum Phi^T Phi, b = sum Phi^T tau, tau_sq = sum tau^T tau; tau = tau_meas or getJointTorque.
-        `out=(G,b,tau_sq)` accumulates into existing arrays (chunked / multi-pass use)."""
+        `out=(G,b,tau_sq)` accumulates into existing arrays (chunked / multi-pass use).
+        `weights`: diagonal weights W (weighted least squares, rdb_regressor_gram_weighted_batch): G = sum Phi^T W Phi, b = sum Phi^T W tau,
+        tau_sq = sum tau^T W tau.  A torch CUDA float64 tensor broadcastable to (n_inputs, N): (n_inputs,) one weight per joint, (N,) one per
+        sample, (n_inputs, N) one per row and sample, or expanded views; device samples only (ValueError for host arrays)."""
         if Dq is None or DDq is None:
             raise ValueError("Input data dimensions mismatch")
         dev, single, n, arrs = self._prep([q, Dq, DDq, None])
         tau_arr = None
         if tau_meas is not None:
             arrs, tau_arr = self._with_tau(dev, n, arrs, tau_meas)
+        if weights is not None:
+            cw, _keep = self._weights(dev, n, weights)
         P = 10 * self.nJ
         acc = out is not None
         if acc:
@@ -507,7 +533,10 @@ class Chain:
         else:
             G, b, tt = np.empty((P, P)), np.empty((P,)), np.empty((1,))
         s = self._samples(n, arrs)
-        if dev:
+        if weights is not None:
+            check(self._lib.rdb_regressor_gram_weighted_batch(self._h, ctypes.byref(s), _ptr(tau_arr), ctypes.byref(cw), _ptr(G), _ptr(b), _ptr(tt),
+                                                              int(acc), self._stream()))
+        elif dev:
             check(self._lib.rdb_regressor_gram_batch(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(G), _ptr(b), _ptr(tt), int(acc), self._stream()))
         else:
             check(self._lib.rdb_regressor_gram_batch_host(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(G), _ptr(b), _ptr(tt), int(acc)))
@@ -598,14 +627,17 @@ class Chain:
                                                     _ld(tau), int(out is not None), self._stream()))
         return tau[:, 0] if (single and out is None) else tau
 
-    def regressorGramExt(self, q, Dq, DDq, tau_meas=None, out=None):
-        """Normal equations of the extended model [Phi | Phi_components]: (G[Pt,Pt], b[Pt], tau_sq[1]), Pt = 10*nJ + Pc."""
+    def regressorGramExt(self, q, Dq, DDq, tau_meas=None, out=None, weights=None):
+        """Normal equations of the extended model [Phi | Phi_components]: (G[Pt,Pt], b[Pt], tau_sq[1]), Pt = 10*nJ + Pc.
+        `weights`: as in regressorGram; the component columns of joint r are weighted with row r."""
         dev, single, n, arrs = self._prep([q, Dq, DDq, None])
         if not dev:
             raise ValueError("component entry points take device (torch CUDA) arrays")
         tau_arr = None
         if tau_meas is not None:
             arrs, tau_arr = self._with_tau(dev, n, arrs, tau_meas)
+        if weights is not None:
+            cw, _keep = self._weights(dev, n, weights)
         Pt = 10 * self.nJ + self.getComponentColumns()
         acc = out is not None
         if acc:
@@ -615,7 +647,12 @@ class Chain:
             b = torch.empty((Pt,), dtype=torch.float64, device=arrs[0].device)
             tt = torch.empty((1,), dtype=torch.float64, device=arrs[0].device)
         s = self._samples(n, arrs)
-        check(self._lib.rdb_regressor_gram_ext_batch(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(G), _ptr(b), _ptr(tt), int(acc), self._stream()))
+        if weights is not None:
+            check(self._lib.rdb_regressor_gram_ext_weighted_batch(self._h, ctypes.byref(s), _ptr(tau_arr), ctypes.byref(cw), _ptr(G), _ptr(b),
+                                                                  _ptr(tt), int(acc), self._stream()))
+        else:
+            check(self._lib.rdb_regressor_gram_ext_batch(self._h, ctypes.byref(s), _ptr(tau_arr), _ptr(G), _ptr(b), _ptr(tt), int(acc),
+                                                         self._stream()))
         return G, b, tt
 
 

@@ -567,6 +567,34 @@ rdb_status rdb_regressor_gram_ext_batch(rdb_chain* chain, const rdb_samples* in,
   return RDB_OK;
 }
 
+// rdb_regressor_gram_weighted_batch / rdb_regressor_gram_ext_weighted_batch: the weights, then the checks of the unweighted entries
+static rdb_status gram_weighted(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, const rdb_gram_weights* weights, double* gram,
+                                double* rhs, double* tau_sq, int32_t accumulate, void* stream, bool with_components)
+{
+  if (!weights || !weights->w) return fail(RDB_ERR_INVALID_ARG, "weights / weights->w must not be null");
+  if (weights->joint_stride < 0 || weights->sample_stride < 0) return fail(RDB_ERR_INVALID_ARG, "weight strides must not be negative");
+  rdb_status s = check_samples(chain, in, true);
+  if (s != RDB_OK) return s;
+  RDB_ENTER(chain);
+  RDB_LOCK(chain);
+  if (in->n > 0 && (!in->dq || !in->ddq)) return fail(RDB_ERR_DIM_MISMATCH, "Input data dimensions mismatch");
+  if (!gram || !rhs) return fail(RDB_ERR_INVALID_ARG, "gram / rhs must not be null");
+  RDB_CUDA(launch_gram(*chain, to_dev(in), tau_meas, gram, rhs, tau_sq, accumulate, (cudaStream_t)stream, with_components, weights));
+  return RDB_OK;
+}
+
+rdb_status rdb_regressor_gram_weighted_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, const rdb_gram_weights* weights,
+                                             double* gram, double* rhs, double* tau_sq, int32_t accumulate, void* stream)
+{
+  return gram_weighted(chain, in, tau_meas, weights, gram, rhs, tau_sq, accumulate, stream, false);
+}
+
+rdb_status rdb_regressor_gram_ext_weighted_batch(rdb_chain* chain, const rdb_samples* in, const double* tau_meas, const rdb_gram_weights* weights,
+                                                 double* gram, double* rhs, double* tau_sq, int32_t accumulate, void* stream)
+{
+  return gram_weighted(chain, in, tau_meas, weights, gram, rhs, tau_sq, accumulate, stream, true);
+}
+
 rdb_status rdb_fill_uniform(double* x, int32_t n_planes, int64_t n, int64_t ld, uint64_t seed, int32_t stream_id, void* stream)
 {
   if (!x || n_planes < 0 || n_planes > 64 || n < 0 || ld < n || stream_id < 0 || stream_id > 3)

@@ -170,10 +170,11 @@ struct UnfedRows
 {
   int32_t n, row[RDB_MAX_JOINTS];
 };
-__global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const double* __restrict__ tau, int64_t ld, int64_t n,
-                                                                          const int64_t* __restrict__ offsets, int64_t nseg, UnfedRows u,
-                                                                          const double* __restrict__ part, double* __restrict__ tau_sq,
-                                                                          int accumulate)
+// W: the weighted sum of squares w t t (gram_unfed_tau_sq_weighted_kernel), in the same order
+template <bool W>
+__device__ __forceinline__ void gram_unfed_tau_sq_body(const double* __restrict__ tau, int64_t ld, int64_t n, const int64_t* __restrict__ offsets,
+                                                       int64_t nseg, const UnfedRows& u, const double* __restrict__ part, double* __restrict__ tau_sq,
+                                                       int accumulate, const rdb_gram_weights& wt)
 {
   __shared__ double red[256];
   for (int64_t k = blockIdx.x; k < nseg; k += gridDim.x)
@@ -185,7 +186,8 @@ __global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const 
       for (int64_t i = lo + threadIdx.x; i < hi; i += blockDim.x)
       {
         const double t = tau[(int64_t)u.row[r] * ld + i];
-        s = fma(t, t, s);
+        if constexpr (W) s = fma(__dmul_rn(wt.w[u.row[r] * wt.joint_stride + i * wt.sample_stride], t), t, s);
+        else s = fma(t, t, s);
       }
     red[threadIdx.x] = s;
     __syncthreads();
@@ -202,6 +204,20 @@ __global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const 
     __syncthreads();
   }
 }
+__global__ void __launch_bounds__(256) gram_unfed_tau_sq_segmented_kernel(const double* __restrict__ tau, int64_t ld, int64_t n,
+                                                                          const int64_t* __restrict__ offsets, int64_t nseg, UnfedRows u,
+                                                                          const double* __restrict__ part, double* __restrict__ tau_sq,
+                                                                          int accumulate)
+{
+  gram_unfed_tau_sq_body<false>(tau, ld, n, offsets, nseg, u, part, tau_sq, accumulate, rdb_gram_weights{});
+}
+__global__ void __launch_bounds__(256) gram_unfed_tau_sq_weighted_kernel(const double* __restrict__ tau, int64_t ld, int64_t n,
+                                                                         const int64_t* __restrict__ offsets, int64_t nseg, UnfedRows u,
+                                                                         const double* __restrict__ part, double* __restrict__ tau_sq,
+                                                                         int accumulate, const rdb_gram_weights wt)
+{
+  gram_unfed_tau_sq_body<true>(tau, ld, n, offsets, nseg, u, part, tau_sq, accumulate, wt);
+}
 
 // the inputs no chain joint feeds
 static UnfedRows unfed_rows(const ChainHost& ch)
@@ -216,13 +232,27 @@ static UnfedRows unfed_rows(const ChainHost& ch)
 }
 
 cudaError_t launch_unfed_tau_sq(const ChainHost& ch, const double* tau, int64_t ld, int64_t n, const int64_t* offsets, int64_t nseg,
-                                const double* part, double* tau_sq, int accumulate, cudaStream_t st)
+                                const double* part, double* tau_sq, int accumulate, cudaStream_t st, const rdb_gram_weights* wt)
 {
   if (nseg <= 0) return cudaSuccess;
-  gram_unfed_tau_sq_segmented_kernel<<<(unsigned)std::min<int64_t>(nseg, 65535), 256, 0, st>>>(tau, ld, n, offsets, nseg, unfed_rows(ch), part,
-                                                                                              tau_sq, accumulate);
+  const unsigned grid = (unsigned)std::min<int64_t>(nseg, 65535);
+  if (wt) gram_unfed_tau_sq_weighted_kernel<<<grid, 256, 0, st>>>(tau, ld, n, offsets, nseg, unfed_rows(ch), part, tau_sq, accumulate, *wt);
+  else gram_unfed_tau_sq_segmented_kernel<<<grid, 256, 0, st>>>(tau, ld, n, offsets, nseg, unfed_rows(ch), part, tau_sq, accumulate);
   count_launch();
   return cudaGetLastError();
+}
+
+// General pipeline, weighted: row r of every Phi plane of a chunk (plane c n_in + r, c < P) and of the staged tau, times sqrt(w) of that row
+// and sample, so that the SYRK's sums of products carry w once.  Sample s of the chunk is sample off + s of the call.
+__global__ void gram_weight_rows_kernel(double* __restrict__ phi, double* __restrict__ tau, int64_t ld, int64_t len, int n_in, int P,
+                                        const rdb_gram_weights wt, int64_t off)
+{
+  const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+  const int r = blockIdx.y;
+  if (s >= len) return;
+  const double sw = sqrt(wt.w[r * wt.joint_stride + (off + s) * wt.sample_stride]);
+  for (int c = 0; c < P; c++) phi[((int64_t)c * n_in + r) * ld + s] *= sw;
+  tau[(int64_t)r * ld + s] *= sw;
 }
 
 // rdb_chain_gram_kernel_info after a call on the general pipeline: why the fused kernels did not take it
@@ -250,7 +280,7 @@ static bool gram_force_v0()
 }
 
 static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                                 int accumulate, cudaStream_t st, bool with_components)
+                                 int accumulate, cudaStream_t st, bool with_components, const rdb_gram_weights* wt = nullptr)
 {
   const int n_in = ch.host.n_in, Pr = 10 * ch.host.nj;     // rigid-body columns
   const int P = Pr + (with_components ? ch.comps.cols : 0);  // + component columns (extended model)
@@ -280,10 +310,10 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
       }
       double* ts = unfed ? ch.gram.tau_sq_part.get() : tau_sq;
       if (P == Pr)
-        e = launch_gram_fused(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
+        e = launch_gram_fused(ch, in, tau_meas, gram, rhs, ts, accumulate, st, wt);
       else
-        e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, ts, accumulate, st);
-      if (e == cudaSuccess && unfed) e = launch_unfed_tau_sq(ch, tau_meas, in.ld, in.n, nullptr, 1, ts, tau_sq, accumulate, st);
+        e = launch_gram_fused_ext(ch, in, tau_meas, gram, rhs, ts, accumulate, st, wt);
+      if (e == cudaSuccess && unfed) e = launch_unfed_tau_sq(ch, tau_meas, in.ld, in.n, nullptr, 1, ts, tau_sq, accumulate, st, wt);
       if (e != cudaErrorNotSupported) return e;
     }
     // rdb_chain_gram_kernel_info describes the last Gram call: say that this one ran the general pipeline, and why
@@ -318,12 +348,17 @@ static cudaError_t gram_launches(ChainHost& ch, const SamplesDev& in, const doub
     }
     const double* tau = own_tau ? w_tau : tau_meas + off;
     const int64_t tau_ld = own_tau ? chunk : in.ld;
-    // the SYRK kernel takes one ld for both; when tau comes from the caller with another stride, stage it
-    if (!own_tau && tau_ld != chunk)
+    // the SYRK kernel takes one ld for both; when tau comes from the caller with another stride, stage it (weighted: always, it is scaled)
+    if (!own_tau && (tau_ld != chunk || wt))
     {
       e = cudaMemcpy2DAsync(w_tau, chunk * sizeof(double), tau, tau_ld * sizeof(double), len * sizeof(double), n_in, cudaMemcpyDeviceToDevice, st);
       if (e != cudaSuccess) return e;
       tau = w_tau;
+    }
+    if (wt)
+    {
+      gram_weight_rows_kernel<<<dim3((unsigned)((len + 255) / 256), n_in), 256, 0, st>>>(w_phi, w_tau, chunk, len, n_in, P, *wt, off);
+      count_launch();
     }
     syrk_dmma_kernel<<<dim3(gx, npairs), SY_THREADS, 0, st>>>(w_phi, tau, chunk, len, n_in, P, nblk, w_part);
     count_launch();
@@ -351,9 +386,9 @@ static cudaError_t ordered_gram_call(ChainHost& ch, cudaStream_t st, F&& launche
 }
 
 cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq, int accumulate,
-                        cudaStream_t st, bool with_components)
+                        cudaStream_t st, bool with_components, const rdb_gram_weights* wt)
 {
-  return ordered_gram_call(ch, st, [&] { return gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components); });
+  return ordered_gram_call(ch, st, [&] { return gram_launches(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, with_components, wt); });
 }
 
 static cudaError_t gram_segmented_launches(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,

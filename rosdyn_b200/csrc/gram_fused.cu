@@ -187,28 +187,33 @@ static cudaError_t grow_reduced(ChainHost& ch, int64_t rows)
   return ch.gram.reduced.grow(sizeof(double) * rows * ReducedRow::doubles(10 * ch.gram.fold.nj), ch.gram.done);
 }
 
-// slots that fit the shared memory of an SM (227 KB minus 1 KB of barriers / static data): the rows, and XC component columns per joint
-template <int NJ, int Z, int XC>
+// slots that fit the shared memory of an SM (227 KB minus 1 KB of barriers / static data): the rows, XC component columns per joint and (WT)
+// the weight of every row
+template <int NJ, int Z, int XC, bool WT = false>
 constexpr int gf_slots()
 {
-  return std::min<int>(GF_MAX_SLOTS,
-                       (int)((227 * 1024 - 1024) / (sizeof(double) * (GramGeom<NJ, Z>::SLOT_DOUBLES + gram_ext_side_doubles<NJ, XC>()))));
+  return std::min<int>(GF_MAX_SLOTS, (int)((227 * 1024 - 1024) / (sizeof(double) * (GramGeom<NJ, Z>::SLOT_DOUBLES + gram_ext_side_doubles<NJ, XC>() +
+                                                                                     (WT ? 32 * NJ : 0)))));
 }
 
 // gram_fused_kernel on the folded chain, one per-CTA partial (gram_partial_doubles) each into `partials`: *grid CTAs.  On REV chains the
 // kernel is the one specialised at run time to the chain's constants when it can be built (gram_jit.cpp), else the precompiled
 // instantiation; other chains always run the precompiled generic kernel.
 // SEG: gram_fused_segmented_kernel instead, one CTA per work item of items[0 .. 2 *grid) (device table of start, length).
-template <int NJ, bool REV, int XC, bool SEG = false>
+// WT: gram_fused_weighted_kernel instead, with the weights wt (same grid).
+template <int NJ, bool REV, int XC, bool SEG = false, bool WT = false>
 static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const SamplesDev& in, const double* tau_meas, double* partials,
-                                       int* grid, cudaStream_t st, const int64_t* items = nullptr)
+                                       int* grid, cudaStream_t st, const int64_t* items = nullptr, const rdb_gram_weights& wt = {})
 {
+  static_assert(!(SEG && WT), "no weighted segmented kernel");
   constexpr int Z = REV ? (XC ? 1 : 2) : 0;  // as in the kernel
-  constexpr int SLOTS = gf_slots<NJ, Z, XC>();
+  constexpr int SLOTS = gf_slots<NJ, Z, XC, WT>();
   static_assert(SLOTS >= 2, "the fused kernel needs two slots");
-  const char* name = SEG ? "gram_fused_segmented_kernel" : "gram_fused_kernel";
+  static_assert(!WT || XC > 0 || SLOTS == gf_slots<NJ, Z, XC>(), "the weighted rigid-body kernel keeps the slots, hence the groups, of gram_fused_kernel");
+  const char* name = SEG ? "gram_fused_segmented_kernel" : (WT ? "gram_fused_weighted_kernel" : "gram_fused_kernel");
   const void* kfn = nullptr;
   if constexpr (SEG) kfn = reinterpret_cast<const void*>(gram_fused_segmented_kernel<NJ, SLOTS, REV, XC>);
+  else if constexpr (WT) kfn = reinterpret_cast<const void*>(gram_fused_weighted_kernel<NJ, SLOTS, REV, XC>);
   else kfn = reinterpret_cast<const void*>(gram_fused_kernel<NJ, SLOTS, REV, XC>);
   if (REV)
   {
@@ -221,8 +226,9 @@ static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const
     ch.gram.kernel_specialised = 0;
     ch.gram.kernel_why = "precompiled kernel: not every folded joint is revolute about e_z (generic generator)";
   }
-  if (SEG) ch.gram.kernel_why = std::string(name) + ", " + ch.gram.kernel_why;  // rdb_chain_gram_kernel_info names the segmented kernel
-  const size_t smem = sizeof(double) * (size_t)gram_smem_doubles<NJ, Z, SLOTS, XC>();
+  // rdb_chain_gram_kernel_info names the segmented and the weighted kernel
+  if (SEG || WT) ch.gram.kernel_why = std::string(name) + ", " + ch.gram.kernel_why;
+  const size_t smem = sizeof(double) * (size_t)gram_smem_doubles_w<NJ, Z, SLOTS, XC, WT>();
   cudaError_t e = cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   if (!SEG)
@@ -236,19 +242,29 @@ static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const
   SamplesDev ins = in;
   const double* tm = tau_meas;
   const int64_t* it = items;
+  rdb_gram_weights w = wt;
   double* part = partials;
   int dbg = gram_dev_switch();
   void* args_whole[] = {&C, &comps, &ins, &tm, &part, &dbg};
   void* args_seg[] = {&C, &comps, &ins, &tm, &it, &part, &dbg};
-  e = cudaLaunchKernel(kfn, dim3(*grid), dim3(GF_THREADS), SEG ? args_seg : args_whole, smem, st);
+  void* args_w[] = {&C, &comps, &ins, &tm, &w, &part, &dbg};
+  e = cudaLaunchKernel(kfn, dim3(*grid), dim3(GF_THREADS), SEG ? args_seg : (WT ? args_w : args_whole), smem, st);
   if (e != cudaSuccess) return e;
   count_launch();
   return cudaSuccess;
 }
+// the same, weighted when wt is given
+template <int NJ, bool REV, int XC>
+static cudaError_t launch_fused_kernel(ChainHost& ch, const GramComps& gc, const SamplesDev& in, const double* tau_meas, double* partials,
+                                       int* grid, cudaStream_t st, const rdb_gram_weights* wt)
+{
+  return wt ? launch_fused_kernel<NJ, REV, XC, false, true>(ch, gc, in, tau_meas, partials, grid, st, nullptr, *wt)
+            : launch_fused_kernel<NJ, REV, XC>(ch, gc, in, tau_meas, partials, grid, st);
+}
 
 template <int NJ, bool REV>
 static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                                   int accumulate, cudaStream_t st)
+                                   int accumulate, cudaStream_t st, const rdb_gram_weights* wt)
 {
   constexpr int Z = REV ? 2 : 0;  // as in the kernel
   using G = GramGeom<NJ, Z>;
@@ -257,7 +273,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
   if (e != cudaSuccess) return e;
   double* part = ch.gram.fused_partials.get();
   int grid = 0;
-  e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, part, &grid, st);
+  e = launch_fused_kernel<NJ, REV, 0>(ch, GramComps{}, in, tau_meas, part, &grid, st, wt);
   if (e != cudaSuccess) return e;
   if (ch.gram.fold_identity)
   {
@@ -272,7 +288,7 @@ static cudaError_t launch_fused_nj(ChainHost& ch, const SamplesDev& in, const do
 
 // returns cudaErrorNotSupported when the chain does not fit the fused kernel (caller falls back to the general pipeline)
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                              int accumulate, cudaStream_t st)
+                              int accumulate, cudaStream_t st, const rdb_gram_weights* wt)
 {
   if (in.n <= 0 || ch.gram.fold_version != ch.model_version) return cudaErrorNotSupported;
   const bool rev = fold_rev_canonical(ch.gram.fold);  // all moving joints revolute about e_z: the specialised generator
@@ -280,8 +296,8 @@ cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double*
   {
 #define X(N)                                                                                  \
   case N:                                                                                     \
-    return rev ? launch_fused_nj<N, true>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st) \
-               : launch_fused_nj<N, false>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st);
+    return rev ? launch_fused_nj<N, true>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, wt) \
+               : launch_fused_nj<N, false>(ch, in, tau_meas, gram, rhs, tau_sq, accumulate, st, wt);
     X(1) X(2) X(3) X(4) X(5) X(6) X(7)
 #undef X
   }
@@ -526,11 +542,24 @@ __global__ void gram_cross_finish_kernel(const double* __restrict__ X, const dou
   }
 }
 
+// weighted extended model: the (component, component) tiles are sums of (w x_m) x_n, whose two halves round differently; gram_cross_finish_kernel
+// writes both.  Keep the upper one (row < column), as the reduction does for the diagonal tiles of the rigid-body block: one thread per pair
+// (c2 > cc) of component columns on the same joint.  With w == 1 both halves are equal and nothing changes.
+__global__ void gram_ext_mirror_kernel(const int32_t* __restrict__ xj, int P, int Pc, double* __restrict__ gram)
+{
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= Pc * Pc) return;
+  const int c2 = e / Pc, cc = e % Pc;
+  if (c2 <= cc || xj[c2] != xj[cc]) return;
+  const int64_t Pt = P + Pc;
+  gram[(int64_t)(P + cc) * Pt + P + c2] = gram[(int64_t)(P + c2) * Pt + P + cc];
+}
+
 // one pass of gram_fused_kernel<.., XC> over the samples: rigid-body tiles -> Gt | bt | tst (full parameter vector) -> the rigid block of the
 // extended normal equations; cross tiles -> xsum -> the cross blocks.  xmap: reduced joint, then slot, of every component column.
 template <int NJ, bool REV, int XC>
 static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::vector<int32_t>& xmap, const SamplesDev& in, const double* tau_meas,
-                                 double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st)
+                                 double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st, const rdb_gram_weights* wt)
 {
   constexpr int Z = REV ? 1 : 0;  // as in the kernel
   using G = GramGeom<NJ, Z>;
@@ -550,7 +579,7 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   e = cudaMemcpyAsync(dmap, xmap.data(), sizeof(int32_t) * xmap.size(), cudaMemcpyHostToDevice, st);  // pageable source: staged before return
   if (e != cudaSuccess) return e;
   int grid = 0;
-  e = launch_fused_kernel<NJ, REV, XC>(ch, gc, in, tau_meas, xpart, &grid, st);
+  e = launch_fused_kernel<NJ, REV, XC>(ch, gc, in, tau_meas, xpart, &grid, st, wt);
   if (e != cudaSuccess) return e;
   if (ch.gram.fold_identity) launch_fused_reduce<NJ, Z>(xpart, grid, PSTRIDE, Gt, bt, tst, 0, st);
   else
@@ -567,6 +596,11 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
   const FoldMaps fm = ch.gram.fold_identity ? FoldMaps{nullptr, nullptr} : fold_maps(ch);
   gram_cross_finish_kernel<NJ, Z><<<((P + 1 + Pc) * Pc + 127) / 128, 128, 0, st>>>(xsum, fm.T, fm.kof, dmap, dmap + Pc, nj, Pc, gram, rhs, accumulate);
   count_launch();
+  if (wt)
+  {
+    gram_ext_mirror_kernel<<<(Pc * Pc + 127) / 128, 128, 0, st>>>(dmap, P, Pc, gram);
+    count_launch();
+  }
   return cudaGetLastError();
 }
 
@@ -574,7 +608,7 @@ static cudaError_t launch_ext_nj(ChainHost& ch, const GramComps& gc, const std::
 // cudaErrorNotSupported: more than 7 moving joints, a component on an input no chain joint feeds, or more than GX_COLS component columns
 // on one joint (caller falls back to the general pipeline).
 cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                                  int accumulate, cudaStream_t st)
+                                  int accumulate, cudaStream_t st, const rdb_gram_weights* wt)
 {
   if (in.n <= 0 || ch.gram.fold_version != ch.model_version) return cudaErrorNotSupported;
   const ChainDev<RDB_MAX_JOINTS>& F = ch.gram.fold;
@@ -608,9 +642,9 @@ cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const dou
   switch (K)
   {
 #define XL(N, R)                                                                                                  \
-  (xcmax <= 2 ? launch_ext_nj<N, R, 2>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st)               \
-              : (xcmax <= 4 ? launch_ext_nj<N, R, 4>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st) \
-                            : launch_ext_nj<N, R, 8>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st)))
+  (xcmax <= 2 ? launch_ext_nj<N, R, 2>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st, wt)               \
+              : (xcmax <= 4 ? launch_ext_nj<N, R, 4>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st, wt) \
+                            : launch_ext_nj<N, R, 8>(ch, gc, xmap, in, tau_meas, gram, rhs, tau_sq, accumulate, st, wt)))
 #define X(N) \
   case N:    \
     return rev ? XL(N, true) : XL(N, false);

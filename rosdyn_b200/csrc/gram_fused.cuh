@@ -222,11 +222,20 @@ __host__ __device__ constexpr int gram_smem_doubles()
 {
   return gram_side_offset<NJ, Z, SLOTS, XC>() + SLOTS * gram_ext_side_doubles<NJ, XC>();
 }
+// weighted kernels: behind the side buffers, the weight of every (joint row, sample) of each slot, [joint][sample]
+template <int NJ, int Z, int SLOTS, int XC, bool W>
+__host__ __device__ constexpr int gram_smem_doubles_w()
+{
+  return gram_smem_doubles<NJ, Z, SLOTS, XC>() + (W ? SLOTS * 32 * NJ : 0);
+}
 
 // ---------------------------------------------------------------------------------------------- generator side
-template <int NJ, int SLOTS, bool REV, int Z, int XC, class M, bool WIN = false>
+// W: weighted normal equations; the generator also stores the weight of each row of its sample (*wt, input order) behind the side buffers,
+// [slot][joint][sample] (gram_smem_doubles_w)
+template <int NJ, int SLOTS, bool REV, int Z, int XC, class M, bool WIN = false, bool W = false>
 __device__ __forceinline__ void gram_gen_role(const ChainDev<NJ>& C, const GramComps& comps, const SamplesDev& in, const double* __restrict__ tau_meas,
-                                              double* smem, double* side0, GramBars* bars, int w, int lane, int dbg)
+                                              double* smem, double* side0, GramBars* bars, int w, int lane, int dbg,
+                                              const rdb_gram_weights* wt = nullptr)
 {
   using G = GramGeom<NJ, Z>;
   constexpr int B = gram_group_block<SLOTS, XC>();
@@ -239,12 +248,25 @@ __device__ __forceinline__ void gram_gen_role(const ChainDev<NJ>& C, const GramC
     const int64_t i = gram_role_group<B, WIN>(k) * 32 + lane;
     GenIn<NJ> cur;
     gen_load<NJ>(C, in, min(i, in.n - 1), cur);
+    double wv[W ? NJ : 1];
+    if constexpr (W)
+    {
+      const int64_t iw = min(i, in.n - 1);
+#pragma unroll
+      for (int j = 0; j < NJ; j++) wv[j] = __ldg(wt->w + C.joint[j].in * wt->joint_stride + iw * wt->sample_stride);
+    }
     trig_all<NJ>(cur.q, cur.sv, cur.cv);
     // every MMA warp is done with the previous use of the slot (mbarrier: the first wait, on parity 1, returns at once)
     if constexpr (B == SLOTS) mbarrier_wait(&bars->empty[s], (u & 1) ^ 1);
     else wait_counter_ge(&bars->drained[s], GF_MMA_WARPS * u);
     double* slot = smem + (size_t)s * G::SLOT_DOUBLES;
     double* side = side0 + (size_t)s * gram_ext_side_doubles<NJ, XC>();
+    if constexpr (W)
+    {
+      double* wrow = side0 + (size_t)SLOTS * gram_ext_side_doubles<NJ, XC>() + (size_t)s * 32 * NJ;
+#pragma unroll
+      for (int j = 0; j < NJ; j++) wrow[32 * j + lane] = wv[j];
+    }
     if (XC > 0 || !(dbg & 1))
     {
       if constexpr (XC > 0) gram_component_park<NJ, XC>(cur, side, lane);
@@ -292,8 +314,11 @@ __device__ __forceinline__ double gram_load_xside(const double* __restrict__ sid
   const int g = lane >> 2, t = lane & 3;
   return g < XC ? side[(J * XC + g) * 32 + 4 * kk + t] : 0.0;
 }
+// a: the A operands of the step -- the fragments b themselves, or in the weighted kernels b scaled by the weight of the lane's sample, so that
+// every product of the step carries the weight once: G += A^T B = sum_s w_s Phi_s^T Phi_s (diagonal tiles keep their upper half)
 template <int NJ, int PAR, int J, int Z>
-__device__ __forceinline__ void gram_mma_step(const double (&b)[GramGeom<NJ, Z>::NF], double (&acc)[GramGeom<NJ, Z>::ntiles(PAR)][2])
+__device__ __forceinline__ void gram_mma_step(const double (&a)[GramGeom<NJ, Z>::NF], const double (&b)[GramGeom<NJ, Z>::NF],
+                                              double (&acc)[GramGeom<NJ, Z>::ntiles(PAR)][2])
 {
   using G = GramGeom<NJ, Z>;
   constexpr int T = G::T, TJ = G::tj(J);
@@ -303,23 +328,24 @@ __device__ __forceinline__ void gram_mma_step(const double (&b)[GramGeom<NJ, Z>:
     if (I >= TJ || !G::owns(I, PAR)) continue;
 #pragma unroll
     for (int K = I; K < T; K++)
-      if (K < TJ) dmma884f(acc[G::local(I, K, PAR)][0], acc[G::local(I, K, PAR)][1], b[I], b[K]);
+      if (K < TJ) dmma884f(acc[G::local(I, K, PAR)][0], acc[G::local(I, K, PAR)][1], a[I], b[K]);
   }
 }
 // TC == 0: Phi^T tau on the tile rows this warp owns and (par 0) tau^T tau, by DFMA on the fragments of the step's DMMAs
 template <int NJ, int PAR, int J, int Z>
-__device__ __forceinline__ void gram_tau_step(const double (&b)[GramGeom<NJ, Z>::NF], double (&bacc)[GramGeom<NJ, Z>::nbacc(PAR)])
+__device__ __forceinline__ void gram_tau_step(const double (&a)[GramGeom<NJ, Z>::NF], const double (&b)[GramGeom<NJ, Z>::NF],
+                                              double (&bacc)[GramGeom<NJ, Z>::nbacc(PAR)])
 {
   using G = GramGeom<NJ, Z>;
   static_for<0, G::tj(J)>([&](auto Ic) {
     constexpr int I = decltype(Ic)::value;
-    if constexpr (G::owns(I, PAR)) bacc[G::bown(I, PAR)] = fma(b[I], b[G::T], bacc[G::bown(I, PAR)]);
+    if constexpr (G::owns(I, PAR)) bacc[G::bown(I, PAR)] = fma(a[I], b[G::T], bacc[G::bown(I, PAR)]);
   });
-  if constexpr (PAR == 0) bacc[G::nbacc(PAR) - 1] = fma(b[G::T], b[G::T], bacc[G::nbacc(PAR) - 1]);
+  if constexpr (PAR == 0) bacc[G::nbacc(PAR) - 1] = fma(a[G::T], b[G::T], bacc[G::nbacc(PAR) - 1]);
 }
-// XC: the cross tiles of joint row J, (regular tile I, component tile) and (component, component)
+// XC: the cross tiles of joint row J, (regular tile I, component tile) and (component, component); ax: the component fragment as A operand
 template <int NJ, int PAR, int J, int Z, int NX>
-__device__ __forceinline__ void gram_cross_step(const double (&b)[GramGeom<NJ, Z>::NF], double bx, double (&xacc)[NX][2])
+__device__ __forceinline__ void gram_cross_step(const double (&a)[GramGeom<NJ, Z>::NF], double ax, double bx, double (&xacc)[NX][2])
 {
   using G = GramGeom<NJ, Z>;
   static_for<0, G::tj(J) + 1>([&](auto Ic) {
@@ -327,33 +353,48 @@ __device__ __forceinline__ void gram_cross_step(const double (&b)[GramGeom<NJ, Z
     if constexpr (G::xowns(J, I, PAR))
     {
       constexpr int k = G::xlocal(J, I, PAR);
-      if constexpr (I < G::tj(J)) dmma884f(xacc[k][0], xacc[k][1], b[I], bx);
-      else dmma884f(xacc[k][0], xacc[k][1], bx, bx);  // (component, component) tile of joint J
+      if constexpr (I < G::tj(J)) dmma884f(xacc[k][0], xacc[k][1], a[I], bx);
+      else dmma884f(xacc[k][0], xacc[k][1], ax, bx);  // (component, component) tile of joint J
     }
   });
 }
 // k-steps STEP.. of this warp in one slot; step = (joint row, k-step of the warp); the fragments of the next step are in flight while the
-// DMMAs of the current one issue
-template <int NJ, int PAR, int STEP, int Z, int XC, int NX>
+// DMMAs of the current one issue.  W: wrow holds the weights of the slot [joint][sample], wcur the weight of the lane's sample in this step
+template <int NJ, int PAR, int STEP, int Z, int XC, int NX, bool W = false>
 __device__ __forceinline__ void gram_consume_steps(const double* __restrict__ slot, const double* __restrict__ side, int ks, int lane,
                                                    const double (&bcur)[GramGeom<NJ, Z>::NF], double bxcur,
                                                    double (&acc)[GramGeom<NJ, Z>::ntiles(PAR)][2], double (&bacc)[GramGeom<NJ, Z>::nbacc(PAR)],
-                                                   double (&xacc)[NX][2])
+                                                   double (&xacc)[NX][2], const double* __restrict__ wrow = nullptr, double wcur = 1.0)
 {
   using G = GramGeom<NJ, Z>;
   constexpr int J = STEP / G::KPW;
-  double bnext[G::NF], bxnext = 0.0;
+  double bnext[G::NF], bxnext = 0.0, wnext = 1.0;
   if constexpr (STEP + 1 < G::NSTEPS)
   {
     constexpr int JN = (STEP + 1) / G::KPW;
     const int kn = ks * G::KPW + (STEP + 1) % G::KPW;
     gram_load_frags<NJ, JN, Z>(slot, kn, lane, bnext);
     if constexpr (XC > 0) bxnext = gram_load_xside<JN, XC>(side, kn, lane);
+    if constexpr (W) wnext = wrow[32 * JN + 4 * kn + (lane & 3)];
   }
-  gram_mma_step<NJ, PAR, J, Z>(bcur, acc);
-  if constexpr (!G::TC) gram_tau_step<NJ, PAR, J, Z>(bcur, bacc);
-  if constexpr (XC > 0) gram_cross_step<NJ, PAR, J, Z>(bcur, bxcur, xacc);
-  if constexpr (STEP + 1 < G::NSTEPS) gram_consume_steps<NJ, PAR, STEP + 1, Z, XC>(slot, side, ks, lane, bnext, bxnext, acc, bacc, xacc);
+  if constexpr (W)
+  {
+    // the A operands carry the weight: one DMUL per fragment this warp uses as A (the others are dead and not issued)
+    double a[G::NF];
+#pragma unroll
+    for (int I = 0; I < G::NF; I++) a[I] = __dmul_rn(bcur[I], wcur);
+    gram_mma_step<NJ, PAR, J, Z>(a, bcur, acc);
+    if constexpr (!G::TC) gram_tau_step<NJ, PAR, J, Z>(a, bcur, bacc);
+    if constexpr (XC > 0) gram_cross_step<NJ, PAR, J, Z>(a, __dmul_rn(bxcur, wcur), bxcur, xacc);
+  }
+  else
+  {
+    gram_mma_step<NJ, PAR, J, Z>(bcur, bcur, acc);
+    if constexpr (!G::TC) gram_tau_step<NJ, PAR, J, Z>(bcur, bcur, bacc);
+    if constexpr (XC > 0) gram_cross_step<NJ, PAR, J, Z>(bcur, bxcur, bxcur, xacc);
+  }
+  if constexpr (STEP + 1 < G::NSTEPS)
+    gram_consume_steps<NJ, PAR, STEP + 1, Z, XC, NX, W>(slot, side, ks, lane, bnext, bxnext, acc, bacc, xacc, wrow, wnext);
 }
 
 // fixed-order reduction over the k-split warps that own the same tiles, into shared memory (the slots are dead by now)
@@ -460,8 +501,9 @@ __device__ __forceinline__ void gram_cross_reduce_smem(double (&xacc)[NX][2], do
   }
 }
 
-template <int NJ, int SLOTS, int PAR, int Z, int XC, bool WIN = false>
-__device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem, const double* side0, GramBars* bars, int ks, int lane, int dbg)
+template <int NJ, int SLOTS, int PAR, int Z, int XC, bool WIN = false, bool W = false>
+__device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem, const double* side0, GramBars* bars, int ks, int lane, int dbg,
+                                              const double* wrow0 = nullptr)
 {
   using G = GramGeom<NJ, Z>;
   constexpr int B = gram_group_block<SLOTS, XC>();
@@ -488,7 +530,13 @@ __device__ __forceinline__ void gram_mma_role(const SamplesDev& in, double* smem
       double b0[G::NF], bx0 = 0.0;
       gram_load_frags<NJ, 0, Z>(slot, ks * G::KPW, lane, b0);
       if constexpr (XC > 0) bx0 = gram_load_xside<0, XC>(side, ks * G::KPW, lane);
-      gram_consume_steps<NJ, PAR, 0, Z, XC>(slot, side, ks, lane, b0, bx0, acc, bacc, xacc);
+      if constexpr (W)
+      {
+        const double* wrow = wrow0 + (size_t)s * 32 * NJ;
+        gram_consume_steps<NJ, PAR, 0, Z, XC, NX, true>(slot, side, ks, lane, b0, bx0, acc, bacc, xacc, wrow,
+                                                        wrow[4 * ks * G::KPW + (lane & 3)]);
+      }
+      else gram_consume_steps<NJ, PAR, 0, Z, XC>(slot, side, ks, lane, b0, bx0, acc, bacc, xacc);
     }
     __syncwarp();
     if (lane == 0)
@@ -547,6 +595,58 @@ __global__ void __launch_bounds__(GF_THREADS, 1)
   const int mma_id = warp, ks = mma_id % GF_KSPLIT;
   if (mma_id < GF_KSPLIT) gram_mma_role<NJ, SLOTS, 0, Z, XC>(in, smem, side0, &bars, ks, lane, dbg);
   else gram_mma_role<NJ, SLOTS, 1, Z, XC>(in, smem, side0, &bars, ks, lane, dbg);
+  double* out = partial + (size_t)blockIdx.x * NOUT;
+  for (int k = mma_id * 32 + lane; k < NOUT; k += 32 * GF_MMA_WARPS) out[k] = smem[k];
+}
+
+// Weighted normal equations (rdb_regressor_gram_weighted_batch, rdb_regressor_gram_ext_weighted_batch):
+//   G (+)= sum_s Phi_s^T W_s Phi_s ,  b (+)= sum_s Phi_s^T W_s tau_s ,  tau_sq (+)= sum_s tau_s^T W_s tau_s ,  W_s = diag(w of the rows of s)
+// The weight of the row of folded joint j in sample i is wt.w[C.joint[j].in * wt.joint_stride + i * wt.sample_stride].  The generator loads
+// it with the sample's inputs and stores it beside the slot; the MMA warps scale the A operands of every k-step by it (gram_consume_steps):
+// per k-step and warp one shared load and one DMUL per tile row it owns, and nothing more in the generator warp, which bounds the kernel.
+// Grid, groups, slots of the rigid-body kernel and every summation order are those of gram_fused_kernel, so w == 1 gives its results bit
+// for bit, and a power-of-two weight scales them exactly.  The extended model may keep fewer slots than gram_fused_kernel (the weights take
+// shared memory); its CTAs take one group at a time either way, so the order of the sums does not depend on the slots.
+// Otherwise this is gram_fused_kernel line for line (kept apart for the reason given at gram_fused_segmented_kernel).
+template <int NJ, int SLOTS, bool REV, int XC, class M = RtModel>
+__global__ void __launch_bounds__(GF_THREADS, 1)
+    gram_fused_weighted_kernel(const __grid_constant__ ChainDev<NJ> C, const __grid_constant__ GramComps comps, const SamplesDev in,
+                               const double* __restrict__ tau_meas, const __grid_constant__ rdb_gram_weights wt, double* __restrict__ partial,
+                               const int dbg)
+{
+  constexpr int Z = REV ? (XC ? 1 : 2) : 0;
+  constexpr int NOUT = gram_partial_doubles<NJ, Z, XC>();
+  extern __shared__ __align__(16) double smem[];
+  __shared__ GramBars bars;
+  double* const side0 = smem + gram_side_offset<NJ, Z, SLOTS, XC>();
+  double* const wrow0 = smem + gram_smem_doubles<NJ, Z, SLOTS, XC>();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if constexpr (gram_group_block<SLOTS, XC>() == SLOTS)
+  {
+    if (threadIdx.x == 0)
+    {
+      for (int s = 0; s < SLOTS; s++)
+      {
+        mbarrier_init(&bars.full[s], 1);
+        mbarrier_init(&bars.empty[s], GF_MMA_WARPS);
+      }
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+  }
+  else if (threadIdx.x < SLOTS)
+  {
+    bars.filled[threadIdx.x] = 0;
+    bars.drained[threadIdx.x] = 0;
+  }
+  __syncthreads();
+  if (warp >= GF_MMA_WARPS)
+  {
+    gram_gen_role<NJ, SLOTS, REV, Z, XC, M, false, true>(C, comps, in, tau_meas, smem, side0, &bars, warp - GF_MMA_WARPS, lane, dbg, &wt);
+    return;
+  }
+  const int mma_id = warp, ks = mma_id % GF_KSPLIT;
+  if (mma_id < GF_KSPLIT) gram_mma_role<NJ, SLOTS, 0, Z, XC, false, true>(in, smem, side0, &bars, ks, lane, dbg, wrow0);
+  else gram_mma_role<NJ, SLOTS, 1, Z, XC, false, true>(in, smem, side0, &bars, ks, lane, dbg, wrow0);
   double* out = partial + (size_t)blockIdx.x * NOUT;
   for (int k = mma_id * 32 + lane; k < NOUT; k += 32 * GF_MMA_WARPS) out[k] = smem[k];
 }

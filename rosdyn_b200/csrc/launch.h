@@ -263,9 +263,10 @@ void fill_uniform_host(double* x, int n_planes, int64_t n, int64_t ld, uint64_t 
 
 // gram.cu
 // with_components: the extended model [Phi | Phi_c] (general pipeline); else the rigid-body columns only (fused kernel when it fits).
+// wt: the weighted normal equations (rdb_regressor_gram_weighted_batch), nullptr: unweighted.
 // Ordered after the previous Gram call of the handle on any stream (ch.gram.done).
 cudaError_t launch_gram(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                        int accumulate, cudaStream_t st, bool with_components = false);
+                        int accumulate, cudaStream_t st, bool with_components = false, const rdb_gram_weights* wt = nullptr);
 // aux.cu: getWrench / getJointTorque with external wrenches, getJacobianLink (two-pass kernels, not the throughput path)
 cudaError_t launch_aux(const ChainHost& ch, const SamplesDev& in, const double* ext, int64_t ld_ext, double* torque, double* wrenches,
                        double* jac_link, int link, int64_t ld_out, cudaStream_t st);
@@ -297,9 +298,9 @@ inline bool fold_rev_canonical(const ChainDev<RDB_MAX_JOINTS>& F)
 const void* gram_jit_kernel(ChainHost& ch, const char* kernel_args);
 // gram_jit.cpp: the same kernel's cubin for `arch` (e.g. "sm_100a") without a device (rdb_gram_specialised_cubin)
 bool gram_jit_cubin(const ChainDev<RDB_MAX_JOINTS>& F, const char* kernel_args, const char* arch, std::vector<char>& cubin, std::string& why);
-// gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel
+// gram_fused.cu: cudaErrorNotSupported when the chain does not fit the fused kernel; wt: weighted (gram_fused_weighted_kernel)
 cudaError_t launch_gram_fused(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                              int accumulate, cudaStream_t st);
+                              int accumulate, cudaStream_t st, const rdb_gram_weights* wt = nullptr);
 // gram.cu: the normal equations of every segment [offsets[k], offsets[k + 1]) of the batch (host offsets, k < nseg), segment k at gram + k P P,
 // rhs + k P, tau_sq + k; fused segmented kernel when the chain fits it, else the general pipeline once per segment.  Ordered like launch_gram.
 cudaError_t launch_gram_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets, double* gram,
@@ -309,14 +310,15 @@ cudaError_t launch_gram_segmented(ChainHost& ch, const SamplesDev& in, const dou
 cudaError_t launch_gram_fused_segmented(ChainHost& ch, const SamplesDev& in, const double* tau_meas, int64_t nseg, const int64_t* offsets,
                                         double* gram, double* rhs, double* tau_sq, int accumulate, bool unfed, cudaStream_t st);
 // gram.cu: tau_sq[k] = (accumulate ? tau_sq[k] : 0) + part[k] + the squares of the measured torques of the inputs no chain joint feeds over
-// segment k (device offsets [nseg + 1]; nullptr: the one segment [0, n)); an empty segment is left as it is when accumulating
+// segment k (device offsets [nseg + 1]; nullptr: the one segment [0, n)); an empty segment is left as it is when accumulating.
+// wt: each square times its weight (one segment only)
 cudaError_t launch_unfed_tau_sq(const ChainHost& ch, const double* tau, int64_t ld, int64_t n, const int64_t* offsets, int64_t nseg,
-                                const double* part, double* tau_sq, int accumulate, cudaStream_t st);
+                                const double* part, double* tau_sq, int accumulate, cudaStream_t st, const rdb_gram_weights* wt = nullptr);
 // gram_fused.cu: G = E^T G' E, b = E^T b' from the reduced (folded-chain) normal equations of reduced_row(ch, 0)
 cudaError_t launch_fold_expand(ChainHost& ch, double* gram, double* rhs, double* tau_sq, int accumulate, cudaStream_t st);
 // same for the extended model [Phi | Phi_c] (gram is Pt x Pt, Pt = 10 nJ + component columns)
 cudaError_t launch_gram_fused_ext(ChainHost& ch, const SamplesDev& in, const double* tau_meas, double* gram, double* rhs, double* tau_sq,
-                                  int accumulate, cudaStream_t st);
+                                  int accumulate, cudaStream_t st, const rdb_gram_weights* wt = nullptr);
 
 enum : int
 {
